@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- rollout trajectories/sec (value + adjoint gradient) of the CUDA path, with the CPU restatement beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C3] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE evaluation of the Monte-Carlo rollout estimator (rollout.jl:279-340): all M trajectories of the
@@ -42,7 +42,9 @@ TRAFFIC_NCU = {"C3": (120366848, "profiles/r3_dram_c3_fullM.csv")}  # algorithmi
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps: of the device-resident and the e2e arm, or of --impl reference (the CPU baseline legs beside the "
+                         "b200 arm run once; C4's full loop follows --sga-iters)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="C3")
     ap.add_argument("--M", type=int, default=None, help="override the number of trajectories")
@@ -52,7 +54,32 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=None, help="trajectories in the CPU baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sga-iters", type=int, default=100, help="C4: Adam iterations of the full stochastic-gradient-ascent loop")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (per-trajectory results and the merged estimate) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, per_traj, estimate):
+    """Writes the arrays to out_dir/<name>.npy as float64. per_traj: name -> array whose LAST axis is the sample index (all M of
+    them). If these exceed DUMP_LIMIT_BYTES, a fixed seeded subset of the sample indices is kept, listed in sample_index.npy;
+    all files together, npy headers included, stay within DUMP_LIMIT_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    M = next(iter(per_traj.values())).shape[-1]
+    per_sample = 8 * sum(a.size // M for a in per_traj.values())
+    budget = DUMP_LIMIT_BYTES - 8 * sum(np.size(a) for a in estimate.values()) - 4096 * (len(per_traj) + len(estimate) + 1)
+    if per_sample * M > budget:
+        # each kept sample also costs its 8-byte entry in sample_index
+        keep = np.sort(np.random.default_rng(0).choice(M, budget // (per_sample + 8), replace=False))
+        per_traj = {k: a[..., keep] for k, a in per_traj.items()}
+        per_traj["sample_index"] = keep
+    for name, a in list(per_traj.items()) + list(estimate.items()):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def workload_config(wl, normals, n_gpus):
@@ -158,9 +185,15 @@ def run_reference(args):
     rn_full, dd_full = workload_inputs(pkg, None, wl_full, args.normals, wl_full.M)
     times = []
     for i in range(args.warmup + args.steps):
-        tput, dt, _ = cpu_leg(args.workload, wl_full.M, sample, cores, args.normals, rn_full, dd_full)
+        tput, dt, r = cpu_leg(args.workload, wl_full.M, sample, cores, args.normals, rn_full, dd_full)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:  # the last timed step: the first `sample` trajectories of the workload
+        keys = ("values", "status") + (("grad_x", "grad_theta") if wl_full.with_grad else ())
+        estimate = {"mean": np.array([r["values"].mean()]), "std": np.array([r["values"].std(ddof=1)])}
+        if wl_full.with_grad:
+            estimate.update(grad_x_mean=r["grad_x"].mean(axis=1), grad_x_std=r["grad_x"].std(axis=1, ddof=1))
+        dump_outputs(args.dump_outputs, {k: r[k] for k in keys}, estimate)
     ms = 1e3 * float(np.mean(times))
     value = sample / (ms * 1e-3)
     s1 = max(2, min(sample, sample // cores))
@@ -280,6 +313,26 @@ def main():
         sampler.start()
     total_ms = timed(device_step, args.steps, max(args.warmup, 3))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # what a caller of the timed path receives from its last step: the per-trajectory containers of this rank's shard
+        # (rbo_get_results) and the estimate merged from the all-reduced partial sums; the later arms overwrite both
+        res = {"values": np.zeros(m_count), "status": np.zeros(m_count, np.int32)}
+        if want_grad:
+            res.update(grad_x=np.zeros((d, m_count), order="F"), grad_theta=np.zeros((len(wl.theta), m_count), order="F"))
+        eng.handle.check(eng.lib.rbo_get_results(eng.handle.h, pkg._lib.dptr(res["values"]), pkg._lib.dptr(res.get("grad_x")),
+                                                 pkg._lib.dptr(res.get("grad_theta")), None, None, pkg._lib.iptr(res["status"])))
+        shards = [res]
+        if world > 1:
+            shards = [None] * world
+            dist.all_gather_object(shards, res)
+        if rank == 0:
+            est_mean, est_std, est_gm, est_gs = finalize(sums.cpu().numpy())
+            estimate = {"mean": np.array([est_mean]), "std": np.array([est_std])}
+            if want_grad:
+                estimate.update(grad_x_mean=est_gm, grad_x_std=est_gs)
+            if sga:
+                estimate["x"] = x_cur.copy()  # the iterate the last Adam step produced
+            dump_outputs(args.dump_outputs, {k: np.concatenate([s[k] for s in shards], axis=-1) for k in res}, estimate)
     ms_per_step = total_ms / args.steps
     value = M / (ms_per_step * 1e-3)
 
@@ -341,7 +394,7 @@ def main():
             eng.handle.check(eng.lib.rbo_partial_sums_device(eng.handle.h, ctypes.c_void_p(sums.data_ptr()), nsum))
             dist.all_reduce(sums)
 
-    e2e_steps = max(2, min(args.steps, 3))
+    e2e_steps = args.steps
     e2e_ms = timed(e2e_step, e2e_steps, 1) / e2e_steps
     e2e_value = M / (e2e_ms * 1e-3)
     ok_e2e = int(st_pin.max()) == 0

@@ -899,3 +899,23 @@ def test_trust_region_step_matches_the_oracle_step(pkg, orc):
         assert nbad <= 2, (n, nbad)
     assert worst < 1e-9, worst  # observed 2e-12
     eng.close()
+
+
+def test_bench_dump_outputs_is_reproducible(pkg, tmp_path):
+    """bench.py --dump-outputs writes the last timed step's results; the inputs are fixed by the arguments, so two runs (with a
+    different number of timed steps) dump the same arrays, and the dumped estimate is the mean of the dumped trajectories."""
+    import os, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for steps in (1, 2):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", "1", "--M", "512",
+                              "--no-cpu-baseline", "--dump-outputs", str(tmp_path / f"s{steps}")], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-2000:]
+    names = sorted(p.name for p in (tmp_path / "s1").iterdir())
+    assert names == ["grad_theta.npy", "grad_x.npy", "grad_x_mean.npy", "grad_x_std.npy", "mean.npy", "status.npy", "std.npy", "values.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "s1" / n), np.load(tmp_path / "s2" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, b), n
+    v, gx = np.load(tmp_path / "s1" / "values.npy"), np.load(tmp_path / "s1" / "grad_x.npy")
+    assert v.shape == (512,) and gx.shape == (10, 512) and np.all(np.load(tmp_path / "s1" / "status.npy") == 0)
+    assert np.isclose(np.load(tmp_path / "s1" / "mean.npy")[0], v.mean(), rtol=1e-12)
+    assert np.allclose(np.load(tmp_path / "s1" / "grad_x_mean.npy"), gx.mean(axis=1), rtol=1e-10, atol=1e-14)

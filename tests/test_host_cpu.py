@@ -106,15 +106,50 @@ def test_finalize_sums_merges_shards(pkg):
         assert lib.rbo_finalize_sums(p(bad), d, nth, C.byref(m), C.byref(s), p(gm), p(gs), p(tm), p(ts)) == -5
 
 
-def test_bench_reference_arm_runs_on_cpu():
-    """`bench.py --impl reference` (the CPU restatement on host cores) needs no GPU and prints the contract's JSON line."""
+def test_bench_reference_arm_runs_on_cpu(pkg, orc, tmp_path):
+    """`bench.py --impl reference` (the CPU restatement on host cores) needs no GPU and prints the contract's JSON line; its
+    --dump-outputs holds the first 16 trajectories of the C3 workload, re-run here through the oracle from the workload's inputs."""
     import json, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0", "--cpu-sample", "16"],
-                         capture_output=True, text=True, timeout=300, cwd=root)
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0", "--cpu-sample", "16",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
     assert line["impl"] == "reference" and line["unit"] == "trajectories/s" and line["value"] > 0
     for key in ("metric", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert key in line
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+    v, gx = np.load(tmp_path / "values.npy"), np.load(tmp_path / "grad_x.npy")
+    assert v.shape == (16,) and gx.shape == (10, 16) and np.all(np.load(tmp_path / "status.npy") == 0)
+    from conftest import oracle_problem, relerr
+    wl = pkg.problems.make_workload("C3")
+    rn = np.asfortranarray(orc.gen_low_discrepancy_sequence(wl.M, wl.d, wl.h + 1)[:16])
+    dd = np.asfortranarray(np.random.default_rng(7).random((wl.d, wl.h, wl.M))[:, :, :16])
+    ref = oracle_problem(orc, wl, wl.surrogate(), rn, orc.generate_initial_guesses(wl.S, wl.lbs, wl.ubs), 1, dual_dirs=dd).rollout(tape=False)
+    assert relerr(v, ref["values"]) < 1e-12 and relerr(gx, ref["grad_x"], floor=np.abs(ref["grad_x"]).max()) < 1e-12
+    assert np.isclose(np.load(tmp_path / "mean.npy")[0], ref["values"].mean(), rtol=1e-12)
+    assert np.allclose(np.load(tmp_path / "grad_x_mean.npy"), ref["grad_x"].mean(axis=1), rtol=1e-12, atol=1e-14)
+
+
+def test_bench_dump_outputs_stays_under_its_size_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 .npy files; above the size limit a fixed seeded subset of the sample indices is kept."""
+    import bench
+    rng = np.random.default_rng(0)
+    M, d = 5000, 1  # one gradient row: sample_index is a third of what a kept sample costs, well above the header slack
+    per_traj = {"values": rng.random(M), "grad_x": rng.random((d, M)), "status": np.zeros(M, np.int32)}
+    estimate = {"mean": np.array([per_traj["values"].mean()])}
+    bench.dump_outputs(str(tmp_path / "all"), per_traj, estimate)
+    assert np.array_equal(np.load(tmp_path / "all" / "grad_x.npy"), per_traj["grad_x"])
+    assert not (tmp_path / "all" / "sample_index.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 100_000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), per_traj, estimate)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grad_x.npy", "mean.npy", "sample_index.npy", "status.npy", "values.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 100_000
+    keep = np.load(tmp_path / "a" / "sample_index.npy").astype(np.int64)
+    assert len(keep) > M // 4 and np.all(np.diff(keep) > 0)
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "grad_x.npy"), per_traj["grad_x"][:, keep])

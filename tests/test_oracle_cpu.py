@@ -294,13 +294,15 @@ def test_oracle_reproduces_golden(orc, name):
 # mixed partials g_mu_theta, g_sigma_theta, g_mu_sigma that only the adjoint / the solver's true Hessian consume.
 # ---------------------------------------------------------------------------------------------------
 def _device_scalars_lib():
-    import ctypes as C, os, subprocess
+    import ctypes as C, os, shutil, subprocess
     here = os.path.dirname(os.path.abspath(__file__))
     src = os.path.join(here, "helpers", "device_scalars.cu")
     so = os.path.join(here, "helpers", "libdevice_scalars.so")
     hdr = os.path.join(os.path.dirname(here), "rollout-bayesian-optimization_b200", "csrc", "rbo_device.cuh")
     if not os.path.exists(so) or max(os.path.getmtime(src), os.path.getmtime(hdr)) > os.path.getmtime(so):
-        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-Xcompiler", "-fPIC", "-shared", "-o", so, src])
+        # $NVCC, else nvcc on PATH, else the toolkit location csrc/Makefile builds with: the build needs no PATH entry, nor does this
+        nvcc = os.environ.get("NVCC") or shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
+        subprocess.check_call([nvcc, "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-Xcompiler", "-fPIC", "-shared", "-o", so, src])
     lib = C.CDLL(so)
     dp = C.POINTER(C.c_double)
     lib.dev_rule_partials.argtypes = [C.c_int, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, dp]
