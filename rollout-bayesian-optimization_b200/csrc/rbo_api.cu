@@ -8,7 +8,9 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "rbo_kernel.cuh"
@@ -41,6 +43,42 @@ using namespace rbo;
 
 static thread_local std::string g_create_error;
 
+// A move-only owned device allocation of `cap` elements of T that only grows: cudaFree / cudaMalloc synchronise the device and
+// cost ~0.1 s on a busy context, so a long-lived handle keeps its largest buffers. Converts to T* for kernel arguments and copies.
+template <class T>
+struct DevBuf {
+  T* p = nullptr;
+  size_t cap = 0;
+
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept { swap(o); }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    swap(o);
+    return *this;
+  }
+  ~DevBuf() { reset(); }
+  void swap(DevBuf& o) noexcept {
+    std::swap(p, o.p);
+    std::swap(cap, o.cap);
+  }
+
+  // Holds at least n elements afterwards; the contents do not survive a reallocation. Empty after a failure.
+  cudaError_t reserve(size_t n) {
+    if (n <= cap) return cudaSuccess;
+    reset();
+    cudaError_t e = cudaMalloc((void**)&p, n * sizeof(T));
+    if (e == cudaSuccess) cap = n;
+    else p = nullptr;
+    return e;
+  }
+  void reset() {
+    if (p) cudaFree(p);
+    p = nullptr;
+    cap = 0;
+  }
+  operator T*() const { return p; }
+};
+
 struct rbo_handle {
   int device = 0;
   cudaStream_t own_stream = nullptr, stream = nullptr;
@@ -54,49 +92,46 @@ struct rbo_handle {
   KernelSpec kern;
   int rule_id = 0;
   double sigma_tol = 1e-8, sigma_n2 = 1e-6, k0 = 1, d2k0 = 0, ymin_base = 0;
-  double *Xb = nullptr, *yb = nullptr, *c0 = nullptr, *u0 = nullptr, *Lf = nullptr, *Lb = nullptr, *Lbf = nullptr, *x0_batch = nullptr;
+  DevBuf<double> Xb, yb, c0, u0, Lf, Lb, Lbf, x0_batch;
   // normals / starts
   int M = 0, hp1 = 0;
-  double* rn = nullptr;
+  DevBuf<double> rn;
   int S = 0;
-  double* starts = nullptr;
-  unsigned* sobol_dirs = nullptr;
-  // outputs
+  DevBuf<double> starts;
+  DevBuf<unsigned> sobol_dirs;
+  // outputs, and the shape of the last launch they hold (what the read-back calls and RBO_FLAG_REPLAY_TAPE go by)
   int outM = 0, outh = -1, outS = 0, outd = 0, outnth = 0;
-  double *values = nullptr, *grad_x = nullptr, *grad_theta = nullptr, *xs = nullptr, *ys = nullptr, *gys = nullptr, *alphas = nullptr;
-  int *best_index = nullptr, *grad_case = nullptr, *status = nullptr, *n_evals = nullptr, *start_status = nullptr, *start_iters = nullptr;
-  int* work_counter = nullptr;
-  double* sums = nullptr;
+  DevBuf<double> values, grad_x, grad_theta, xs, ys, gys, alphas;
+  DevBuf<int> best_index, grad_case, status, n_evals, start_status, start_iters;
+  DevBuf<int> work_counter;
+  DevBuf<double> sums;
   int sums_len = 0;
-  double *dual_dirs = nullptr, *x_forced = nullptr, *cs_tape = nullptr, *gh_nodes = nullptr, *gh_weights = nullptr;
-  size_t cap_ghn = 0, cap_ghw = 0;
+  DevBuf<double> dual_dirs, x_forced, cs_tape, gh_nodes, gh_weights;
   int gh_depth = 0, gh_M = 0;
-  size_t dual_cap = 0, forced_cap = 0, tape_cap = 0;
-  size_t cap_Xb = 0, cap_yb = 0, cap_c0 = 0, cap_u0 = 0, cap_Lf = 0, cap_Lb = 0, cap_Lbf = 0, cap_x0b = 0, cap_rn = 0, cap_starts = 0;
-  // last call
-  int last_h = 0, last_mode = 0, last_nth = 1;
-  bool tape_enabled = true;
+  int last_mode = 0;
   double htol = 1e-4;
   int rs_cap = 0;           // development knob: cap on the row splits of the Gram reductions (0 = default)
   int vglob_wmax = 0;       // development knob: cap on the start slots of the large-n variant (0 = default)
   int force_vglob = 0;      // development / test knob: use the large-n variant even when shared memory would do
-  double* Vscratch = nullptr, *Bscratch = nullptr;
-  double *t_mu = nullptr, *t_sigma = nullptr, *t_dmu = nullptr, *t_dsigma = nullptr, *t_Halpha = nullptr;
-  size_t cap_tex = 0;  // trajectories x steps the extended tape holds
+  DevBuf<double> Vscratch, Bscratch;
+  DevBuf<double> t_mu, t_sigma, t_dmu, t_dsigma, t_Halpha;
   bool tex_valid = false;
-  bool xs_valid = false;
-  int* order = nullptr;     // longest-first order of the trajectories of the last launch (scheduling hint for the next one)
-  size_t cap_order = 0;
+  bool xs_valid = false;    // the x-path of the last rollout is on the device (RBO_FLAG_REPLAY_TAPE)
+  DevBuf<int> order;        // longest-first order of the trajectories of the last launch (scheduling hint for the next one)
   int order_M = 0;          // 0: no valid order
   int lpt = 1;              // RBO_TUNE_LPT
-  unsigned long long* cta_done = nullptr;  // the x-path of the last rollout is on the device (RBO_FLAG_REPLAY_TAPE)
+  DevBuf<unsigned long long> cta_done;  // per-CTA finish time of the last launch (device %globaltimer)
   // resident surrogate in its canonical device form (rbo_set_surrogate / rbo_condition): L0^-1 row-major with pitch ldi,
   // the observation sites point-major, work vectors
-  double *Ld = nullptr, *Linv = nullptr, *Xpts = nullptr, *wk = nullptr;
-  int* dstat = nullptr;
-  size_t cap_Ld = 0, cap_Linv = 0, cap_Xpts = 0, cap_wk = 0;
+  DevBuf<double> Ld, Linv, Xpts, wk;
+  DevBuf<int> dstat;
   int ldi = 0, cap_rows = 0;
-  size_t cap_Vscratch = 0, cap_Bscratch = 0;
+
+  ~rbo_handle() {
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+    if (own_stream) cudaStreamDestroy(own_stream);
+  }
 };
 
 static int fail(rbo_handle* h, int code, const char* fmt, ...) {
@@ -115,19 +150,10 @@ static int fail(rbo_handle* h, int code, const char* fmt, ...) {
     if (e_ != cudaSuccess) return fail(h, RBO_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
 
+// D2H of the first n elements of src into dst unless dst is NULL (stream-ordered: the caller synchronises).
 template <class T>
-static cudaError_t dev_realloc(T** p, size_t n) {
-  if (*p) { cudaFree(*p); *p = nullptr; }
-  if (n == 0) return cudaSuccess;
-  return cudaMalloc((void**)p, n * sizeof(T));
-}
-// grows only: cudaFree / cudaMalloc synchronise the device and cost ~0.1 s on a busy context
-template <class T>
-static cudaError_t dev_reserve(T** p, size_t* cap, size_t n) {
-  if (*p && *cap >= n) return cudaSuccess;
-  cudaError_t e = dev_realloc(p, n);
-  *cap = (e == cudaSuccess) ? n : 0;
-  return e;
+static cudaError_t copy_out(T* dst, const DevBuf<T>& src, size_t n, cudaStream_t stream) {
+  return dst ? cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, stream) : cudaSuccess;
 }
 
 extern "C" {
@@ -156,33 +182,28 @@ int rbo_create(rbo_handle** out, int device_id) {
   if (e != cudaSuccess || ndev == 0)
     return fail(nullptr, RBO_ERR_CUDA, "rbo_create: no CUDA device (%s); librbo has no CPU fallback", e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
   if (device_id < 0 || device_id >= ndev) return fail(nullptr, RBO_ERR_ARG, "rbo_create: device %d out of range (have %d)", device_id, ndev);
-  rbo_handle* h = new rbo_handle();
+  auto h = std::make_unique<rbo_handle>();  // released by every failure below
   h->device = device_id;
   rbo_default_solver_opts(&h->so);
   if (const char* e = getenv("RBO_FORCE_LARGE_N")) h->force_vglob = atoi(e) != 0;  // test knob: whole suites under the large-n variant
-#define CKC(call)                                                                                    \
-  do {                                                                                               \
-    cudaError_t e_ = (call);                                                                         \
-    if (e_ != cudaSuccess) { fail(nullptr, RBO_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); delete h; return RBO_ERR_CUDA; } \
-  } while (0)
-  CKC(cudaSetDevice(device_id));
+  CK(nullptr, cudaSetDevice(device_id));
   cudaDeviceProp prop;
-  CKC(cudaGetDeviceProperties(&prop, device_id));
-  if (prop.major < 10) { fail(nullptr, RBO_ERR_UNSUPPORTED, "rbo_create: device sm_%d%d is not Blackwell (sm_100a required)", prop.major, prop.minor); delete h; return RBO_ERR_UNSUPPORTED; }
+  CK(nullptr, cudaGetDeviceProperties(&prop, device_id));
+  if (prop.major < 10) return fail(nullptr, RBO_ERR_UNSUPPORTED, "rbo_create: device sm_%d%d is not Blackwell (sm_100a required)", prop.major, prop.minor);
   h->num_sms = prop.multiProcessorCount;
   h->max_smem = (int)prop.sharedMemPerBlockOptin;
-  CKC(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
+  CK(nullptr, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   h->stream = h->own_stream;
-  CKC(cudaEventCreate(&h->ev0));
-  CKC(cudaEventCreate(&h->ev1));
-  CKC(cudaMalloc((void**)&h->work_counter, 16 * sizeof(int)));  // [0] trajectory scheduler, [1..2] kernel watchdog flags
-  CKC(cudaMalloc((void**)&h->cta_done, 1024 * sizeof(unsigned long long)));
-  CKC(cudaMalloc((void**)&h->sobol_dirs, sizeof(rbo_sobol_dirs_host)));
-  CKC(cudaMemcpy(h->sobol_dirs, rbo_sobol_dirs_host, sizeof(rbo_sobol_dirs_host), cudaMemcpyHostToDevice));
-  CKC(cudaFuncSetAttribute(rbo_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem));
-  CKC(cudaFuncSetAttribute(rbo_rollout_kernel_largen, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem));
-#undef CKC
-  *out = h;
+  CK(nullptr, cudaEventCreate(&h->ev0));
+  CK(nullptr, cudaEventCreate(&h->ev1));
+  CK(nullptr, h->work_counter.reserve(16));  // [0] trajectory scheduler, [1..2] kernel watchdog flags
+  CK(nullptr, h->cta_done.reserve(1024));
+  CK(nullptr, h->sobol_dirs.reserve(sizeof(rbo_sobol_dirs_host) / sizeof(unsigned)));
+  CK(nullptr, cudaMemcpyAsync(h->sobol_dirs, rbo_sobol_dirs_host, sizeof(rbo_sobol_dirs_host), cudaMemcpyHostToDevice, h->stream));
+  CK(nullptr, cudaStreamSynchronize(h->stream));
+  CK(nullptr, cudaFuncSetAttribute(rbo_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem));
+  CK(nullptr, cudaFuncSetAttribute(rbo_rollout_kernel_largen, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem));
+  *out = h.release();
   return RBO_SUCCESS;
 }
 
@@ -190,13 +211,6 @@ int rbo_destroy(rbo_handle* h) {
   if (!h) return RBO_SUCCESS;
   cudaSetDevice(h->device);
   cudaStreamSynchronize(h->stream);
-  void* ptrs[] = {h->Xb, h->yb, h->c0, h->u0, h->Lf, h->Lb, h->Lbf, h->x0_batch, h->rn, h->starts, h->sobol_dirs, h->values, h->grad_x, h->grad_theta, h->xs, h->ys,
-                  h->gys, h->alphas, h->best_index, h->grad_case, h->status, h->n_evals, h->start_status, h->start_iters, h->work_counter, h->sums,
-                  h->dual_dirs, h->x_forced, h->cs_tape, h->gh_nodes, h->gh_weights, h->Vscratch, h->Bscratch, h->Ld, h->Linv, h->Xpts, h->wk, h->dstat, h->t_mu, h->t_sigma, h->t_dmu, h->t_dsigma, h->t_Halpha, h->order, h->cta_done};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  if (h->ev0) cudaEventDestroy(h->ev0);
-  if (h->ev1) cudaEventDestroy(h->ev1);
-  if (h->own_stream) cudaStreamDestroy(h->own_stream);
   delete h;
   return RBO_SUCCESS;
 }
@@ -239,10 +253,10 @@ static int repack_surrogate(rbo_handle* h) {
   const int N8 = (N + RBO_PR - 1) / RBO_PR * RBO_PR, nb32 = (N + BR - 1) / BR;
   h->N8 = N8; h->nb8 = N8 / RBO_PR; h->nb32 = nb32;
   const size_t nchunks = (size_t)nb32 * (nb32 + 1) / 2, nLf = (size_t)LP * BR * nchunks, nLbf = (size_t)1024 * nchunks;
-  CK(h, dev_reserve(&h->Xb, &h->cap_Xb, (size_t)d * N8));
-  CK(h, dev_reserve(&h->Lf, &h->cap_Lf, nLf));
-  CK(h, dev_reserve(&h->Lb, &h->cap_Lb, nLf));
-  CK(h, dev_reserve(&h->Lbf, &h->cap_Lbf, nLbf));
+  CK(h, h->Xb.reserve((size_t)d * N8));
+  CK(h, h->Lf.reserve(nLf));
+  CK(h, h->Lb.reserve(nLf));
+  CK(h, h->Lbf.reserve(nLbf));
   CK(h, cudaMemsetAsync(h->Lf, 0, nLf * 8, h->stream));  // the 4 pad doubles per k
   CK(h, cudaMemsetAsync(h->Lb, 0, nLf * 8, h->stream));
   rbo_layout_x_kernel<<<(d * N8 + 255) / 256, 256, 0, h->stream>>>(h->Xpts, d, N, N8, h->Xb);
@@ -254,40 +268,44 @@ static int repack_surrogate(rbo_handle* h) {
 }
 
 // Capacity of the canonical form: rows_needed rows of L0^-1 (pitch = capacity, so that rbo_condition appends rows in place).
+// Grows into new buffers (keep: with the current rows copied over) that replace the old ones only once every step succeeded,
+// so that a failure leaves the handle as it was.
 static int reserve_surrogate(rbo_handle* h, int d, int rows_needed, bool keep) {
   const int N32 = (rows_needed + RBO_BR - 1) / RBO_BR * RBO_BR;
-  if (N32 <= h->cap_rows && h->Linv && (size_t)rows_needed * d <= h->cap_Xpts) return RBO_SUCCESS;
+  if (N32 <= h->cap_rows && h->Linv && (size_t)rows_needed * d <= h->Xpts.cap) return RBO_SUCCESS;
   const int cap = (rows_needed + 64 + RBO_BR - 1) / RBO_BR * RBO_BR;
-  double *nLinv = nullptr, *nX = nullptr;
-  CK(h, cudaMalloc((void**)&nLinv, (size_t)cap * cap * 8));
-  if (cudaMalloc((void**)&nX, (size_t)cap * d * 8) != cudaSuccess) { cudaFree(nLinv); return fail(h, RBO_ERR_CUDA, "reserve_surrogate: out of device memory"); }
-  cudaMemsetAsync(nLinv, 0, (size_t)cap * cap * 8, h->stream);
+  CK(h, h->dstat.reserve(4));
+  DevBuf<double> Linv, Xpts, yb, c0, u0, wk;
+  CK(h, Linv.reserve((size_t)cap * cap));
+  CK(h, Xpts.reserve((size_t)cap * d));
+  // vectors that grow with the observation count
+  CK(h, yb.reserve(cap));
+  CK(h, c0.reserve(cap));
+  CK(h, u0.reserve(cap));
+  CK(h, wk.reserve((size_t)4 * cap + 64));
+  CK(h, cudaMemsetAsync(Linv, 0, (size_t)cap * cap * 8, h->stream));
   if (keep && h->Linv) {
     const int rows = (h->N + RBO_BR - 1) / RBO_BR * RBO_BR;
-    cudaMemcpy2DAsync(nLinv, (size_t)cap * 8, h->Linv, (size_t)h->ldi * 8, (size_t)rows * 8, rows, cudaMemcpyDeviceToDevice, h->stream);
-    cudaMemcpyAsync(nX, h->Xpts, (size_t)h->N * d * 8, cudaMemcpyDeviceToDevice, h->stream);
+    CK(h, cudaMemcpy2DAsync(Linv, (size_t)cap * 8, h->Linv, (size_t)h->ldi * 8, (size_t)rows * 8, rows, cudaMemcpyDeviceToDevice, h->stream));
+    CK(h, cudaMemcpyAsync(Xpts, h->Xpts, (size_t)h->N * d * 8, cudaMemcpyDeviceToDevice, h->stream));
   }
-  cudaStreamSynchronize(h->stream);
-  if (h->Linv) cudaFree(h->Linv);
-  if (h->Xpts) cudaFree(h->Xpts);
-  h->Linv = nLinv; h->Xpts = nX; h->ldi = cap; h->cap_rows = cap; h->cap_Xpts = (size_t)cap * d; h->cap_Linv = (size_t)cap * cap;
-  // vectors that grow with the observation count
-  double *ny = nullptr, *nc = nullptr, *nu = nullptr;
-  if (cudaMalloc((void**)&ny, (size_t)cap * 8) != cudaSuccess || cudaMalloc((void**)&nc, (size_t)cap * 8) != cudaSuccess || cudaMalloc((void**)&nu, (size_t)cap * 8) != cudaSuccess)
-    return fail(h, RBO_ERR_CUDA, "reserve_surrogate: out of device memory");
-  cudaMemsetAsync(nc, 0, (size_t)cap * 8, h->stream); cudaMemsetAsync(nu, 0, (size_t)cap * 8, h->stream); cudaMemsetAsync(ny, 0, (size_t)cap * 8, h->stream);
+  CK(h, cudaMemsetAsync(c0, 0, (size_t)cap * 8, h->stream));
+  CK(h, cudaMemsetAsync(u0, 0, (size_t)cap * 8, h->stream));
+  CK(h, cudaMemsetAsync(yb, 0, (size_t)cap * 8, h->stream));
   if (keep && h->yb) {
-    cudaMemcpyAsync(ny, h->yb, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream);
-    cudaMemcpyAsync(nc, h->c0, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream);
-    cudaMemcpyAsync(nu, h->u0, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream);
+    CK(h, cudaMemcpyAsync(yb, h->yb, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream));
+    CK(h, cudaMemcpyAsync(c0, h->c0, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream));
+    CK(h, cudaMemcpyAsync(u0, h->u0, (size_t)h->N * 8, cudaMemcpyDeviceToDevice, h->stream));
   }
-  cudaStreamSynchronize(h->stream);
-  if (h->yb) cudaFree(h->yb);
-  if (h->c0) cudaFree(h->c0);
-  if (h->u0) cudaFree(h->u0);
-  h->yb = ny; h->c0 = nc; h->u0 = nu; h->cap_yb = h->cap_c0 = h->cap_u0 = (size_t)cap;
-  CK(h, dev_reserve(&h->wk, &h->cap_wk, (size_t)4 * cap + 64));
-  if (!h->dstat) CK(h, cudaMalloc((void**)&h->dstat, 4 * sizeof(int)));
+  CK(h, cudaStreamSynchronize(h->stream));  // the old buffers are freed when the locals they are swapped into go out of scope
+  h->Linv.swap(Linv);
+  h->Xpts.swap(Xpts);
+  h->yb.swap(yb);
+  h->c0.swap(c0);
+  h->u0.swap(u0);
+  h->wk.swap(wk);
+  h->ldi = cap;
+  h->cap_rows = cap;
   return RBO_SUCCESS;
 }
 
@@ -304,10 +322,10 @@ int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, con
   if (d != h->d) {
     // buffers laid out for another input dimension are no longer valid (normals are M x (d+1) x hp1, starts d x S, ...)
     h->M = 0; h->hp1 = 0; h->S = 0; h->gh_M = 0; h->gh_depth = 0;
-    if (h->rn) { cudaFree(h->rn); h->rn = nullptr; h->cap_rn = 0; }
-    if (h->starts) { cudaFree(h->starts); h->starts = nullptr; h->cap_starts = 0; }
-    if (h->gh_nodes) { cudaFree(h->gh_nodes); h->gh_nodes = nullptr; h->cap_ghn = 0; }
-    if (h->gh_weights) { cudaFree(h->gh_weights); h->gh_weights = nullptr; h->cap_ghw = 0; }
+    h->rn.reset();
+    h->starts.reset();
+    h->gh_nodes.reset();
+    h->gh_weights.reset();
     h->cap_rows = 0;  // Xpts is sized with d
   }
   h->have_sur = false;
@@ -325,11 +343,11 @@ int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, con
   h->ymin_base = ymin;
   const int N32 = (N + RBO_BR - 1) / RBO_BR * RBO_BR;
   // H2D of what FantasySurrogate(s, h) copies (rbs.jl:345-381): X (d x N), the lower factor, y, c
-  CK(h, dev_reserve(&h->Ld, &h->cap_Ld, (size_t)N * N));
+  CK(h, h->Ld.reserve((size_t)N * N));
   CK(h, cudaMemcpy2DAsync(h->Xpts, (size_t)d * 8, X, (size_t)ldX * 8, (size_t)d * 8, N, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpy2DAsync(h->Ld, (size_t)N * 8, L, (size_t)ldL * 8, (size_t)N * 8, N, cudaMemcpyHostToDevice, h->stream));
-  CK(h, cudaMemsetAsync(h->c0, 0, h->cap_c0 * 8, h->stream));
-  CK(h, cudaMemsetAsync(h->u0, 0, h->cap_u0 * 8, h->stream));
+  CK(h, cudaMemsetAsync(h->c0, 0, h->c0.cap * 8, h->stream));
+  CK(h, cudaMemsetAsync(h->u0, 0, h->u0.cap * 8, h->stream));
   CK(h, cudaMemcpyAsync(h->yb, y, (size_t)N * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(h->c0, c, (size_t)N * 8, cudaMemcpyHostToDevice, h->stream));
   // Explicit inverse of the base factor on the device in double-double arithmetic (one rounding per stored entry): every later
@@ -411,7 +429,7 @@ int rbo_set_normals(rbo_handle* h, const double* rn, int M_total, int hp1, int m
   if (!rn || M_total < 1 || hp1 < 1 || m_begin < 0 || m_count < 1 || m_begin + m_count > M_total) return fail(h, RBO_ERR_ARG, "rbo_set_normals: bad arguments");
   CK(h, cudaSetDevice(h->device));
   const int q1 = h->d + 1;
-  CK(h, dev_reserve(&h->rn, &h->cap_rn, (size_t)m_count * q1 * hp1));
+  CK(h, h->rn.reserve((size_t)m_count * q1 * hp1));
   // strided slice [m_begin, m_begin+m_count) of the sample-fastest tensor
   CK(h, cudaMemcpy2DAsync(h->rn, (size_t)m_count * 8, rn + m_begin, (size_t)M_total * 8, (size_t)m_count * 8, (size_t)q1 * hp1, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
@@ -427,7 +445,7 @@ int rbo_generate_normals(rbo_handle* h, int M_total, int hp1, int m_begin, int m
   if (D > RBO_SOBOL_MAXDIM) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_generate_normals: %d Sobol dimensions > %d", D, RBO_SOBOL_MAXDIM);
   if ((double)M_total * hp1 >= 4294967295.0) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_generate_normals: more than 2^32 Sobol points");
   CK(h, cudaSetDevice(h->device));
-  CK(h, dev_reserve(&h->rn, &h->cap_rn, (size_t)m_count * q1 * hp1));
+  CK(h, h->rn.reserve((size_t)m_count * q1 * hp1));
   size_t total = (size_t)m_count * q1 * hp1;
   int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 8);
   rbo_normals_kernel<<<blocks, 256, 0, h->stream>>>(h->sobol_dirs, h->rn, M_total, h->d, hp1, m_begin, m_count);
@@ -450,8 +468,8 @@ int rbo_set_quadrature(rbo_handle* h, const double* nodes, const double* weights
   if (!nodes || !weights || depth < 1 || m_count < 1) return fail(h, RBO_ERR_ARG, "rbo_set_quadrature: bad arguments");
   CK(h, cudaSetDevice(h->device));
   const size_t n = (size_t)depth * m_count;
-  CK(h, dev_reserve(&h->gh_nodes, &h->cap_ghn, n));
-  CK(h, dev_reserve(&h->gh_weights, &h->cap_ghw, n));
+  CK(h, h->gh_nodes.reserve(n));
+  CK(h, h->gh_weights.reserve(n));
   CK(h, cudaMemcpyAsync(h->gh_nodes, nodes, n * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(h->gh_weights, weights, n * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
@@ -465,7 +483,7 @@ int rbo_set_starts(rbo_handle* h, const double* starts, int S) {
   if (!starts || S < 1) return fail(h, RBO_ERR_ARG, "rbo_set_starts: bad arguments");
   if (S > 65535) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_set_starts: %d starts (the kernel keeps per-start counters and the hand-out order as 16-bit values: at most 65535)", S);
   CK(h, cudaSetDevice(h->device));
-  CK(h, dev_reserve(&h->starts, &h->cap_starts, (size_t)S * h->d));
+  CK(h, h->starts.reserve((size_t)S * h->d));
   CK(h, cudaMemcpyAsync(h->starts, starts, (size_t)S * h->d * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   h->S = S;
@@ -475,25 +493,26 @@ int rbo_set_starts(rbo_handle* h, const double* starts, int S) {
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------
+// Makes the output buffers hold a launch of M trajectories (horizon hor, S starts) and records that shape.
 static int ensure_outputs(rbo_handle* h, int M, int hor, int S, int d, int nth) {
   if (h->outM == M && h->outh == hor && h->outS == S && h->outd == d && h->outnth == nth) return RBO_SUCCESS;
   const int hh = std::max(hor, 1);
-  h->outM = 0; h->outh = -1; h->xs_valid = false;  // the cache key is only valid once every buffer below exists
-  CK(h, dev_realloc(&h->values, (size_t)M));
-  CK(h, dev_realloc(&h->grad_x, (size_t)M * d));
-  CK(h, dev_realloc(&h->grad_theta, (size_t)M * nth));
-  CK(h, dev_realloc(&h->best_index, (size_t)M));
-  CK(h, dev_realloc(&h->grad_case, (size_t)M));
-  CK(h, dev_realloc(&h->status, (size_t)M));
-  CK(h, dev_realloc(&h->xs, (size_t)M * (hor + 1) * d));
-  CK(h, dev_realloc(&h->ys, (size_t)M * (hor + 1)));
-  CK(h, dev_realloc(&h->gys, (size_t)M * (hor + 1) * d));
-  CK(h, dev_realloc(&h->alphas, (size_t)M * hh));
-  CK(h, dev_realloc(&h->n_evals, (size_t)M * hh));
-  CK(h, dev_realloc(&h->start_status, (size_t)M * hh * S));
-  CK(h, dev_realloc(&h->start_iters, (size_t)M * hh * S));
+  h->outM = 0; h->outh = -1; h->xs_valid = false;  // the record is only valid once every buffer below holds its shape
+  CK(h, h->values.reserve((size_t)M));
+  CK(h, h->grad_x.reserve((size_t)M * d));
+  CK(h, h->grad_theta.reserve((size_t)M * nth));
+  CK(h, h->best_index.reserve((size_t)M));
+  CK(h, h->grad_case.reserve((size_t)M));
+  CK(h, h->status.reserve((size_t)M));
+  CK(h, h->xs.reserve((size_t)M * (hor + 1) * d));
+  CK(h, h->ys.reserve((size_t)M * (hor + 1)));
+  CK(h, h->gys.reserve((size_t)M * (hor + 1) * d));
+  CK(h, h->alphas.reserve((size_t)M * hh));
+  CK(h, h->n_evals.reserve((size_t)M * hh));
+  CK(h, h->start_status.reserve((size_t)M * hh * S));
+  CK(h, h->start_iters.reserve((size_t)M * hh * S));
   h->sums_len = 1 + 3 * (1 + d + nth) + hh + (hor + 2) + 2;
-  CK(h, dev_realloc(&h->sums, (size_t)h->sums_len + 1 + 3 * (1 + d + nth) + 2));  // + the gathered partial-sums vector (rbo_partial_sums_host)
+  CK(h, h->sums.reserve((size_t)h->sums_len + 1 + 3 * (1 + d + nth) + 2));  // + the gathered partial-sums vector (rbo_partial_sums_host)
   h->outM = M; h->outh = hor; h->outS = S; h->outd = d; h->outnth = nth;
   return RBO_SUCCESS;
 }
@@ -594,58 +613,57 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
   P.gh_nodes = h->gh_nodes; P.gh_weights = h->gh_weights; P.gh_depth = h->gh_depth;
   P.values = h->values; P.grad_x = h->grad_x; P.grad_theta = h->grad_theta; P.best_index = h->best_index; P.grad_case = h->grad_case;
   P.status = h->status; P.xs = h->xs; P.ys = h->ys; P.gys = h->gys; P.alphas = h->alphas; P.n_evals = h->n_evals;
-  P.start_status = h->tape_enabled ? h->start_status : nullptr; P.start_iters = h->tape_enabled ? h->start_iters : nullptr;
+  P.start_status = h->start_status; P.start_iters = h->start_iters;
   P.work_counter = h->work_counter;
   h->tex_valid = false;
   if (flags & RBO_FLAG_TAPE_EX) {
     if (myopic) return fail(h, RBO_ERR_ARG, "rbo_rollout: RBO_FLAG_TAPE_EX does not apply to the myopic solve");
-    const size_t n = (size_t)M * std::max(horizon, 1), dd = (size_t)h->d * h->d;
-    if (h->cap_tex < n * dd) {
-      CK(h, dev_realloc(&h->t_mu, n)); CK(h, dev_realloc(&h->t_sigma, n)); CK(h, dev_realloc(&h->t_dmu, n * h->d)); CK(h, dev_realloc(&h->t_dsigma, n * h->d));
-      CK(h, dev_realloc(&h->t_Halpha, n * dd));
-      h->cap_tex = n * dd;
-    }
+    const size_t n = (size_t)M * std::max(horizon, 1), d = h->d;
+    CK(h, h->t_mu.reserve(n));
+    CK(h, h->t_sigma.reserve(n));
+    CK(h, h->t_dmu.reserve(n * d));
+    CK(h, h->t_dsigma.reserve(n * d));
+    CK(h, h->t_Halpha.reserve(n * d * d));
     P.t_mu = h->t_mu; P.t_sigma = h->t_sigma; P.t_dmu = h->t_dmu; P.t_dsigma = h->t_dsigma; P.t_Halpha = h->t_Halpha;
     h->tex_valid = true;
   }
   const int grid = std::min(M, h->num_sms);
   // longest-first hand-out when the previous launch ran the same trajectories (same normals, nearby x0): only worth it beyond two waves
-  P.order = (h->lpt && !myopic && h->order_M == M && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) ? h->order : nullptr;
-  P.cta_done = grid <= 1024 ? h->cta_done : nullptr;
-  {
-    size_t need = (size_t)grid * (horizon + 2) * pc.NR;
-    if (h->tape_cap < need) { CK(h, dev_realloc(&h->cs_tape, need)); h->tape_cap = need; }
-    P.cs_tape = h->cs_tape;
-    if (pc.vglob) {
-      CK(h, dev_reserve(&h->Vscratch, &h->cap_Vscratch, (size_t)grid * pc.NR * pc.RP));
-      P.Vscratch = h->Vscratch;
-      P.bscratch_len = (size_t)h->N8 * 8 * ((std::max(h->d + 1, pc.W) + 7) / 8);  // widest backward pass: q1 columns (adjoint) or W (inner solve)
-      CK(h, dev_reserve(&h->Bscratch, &h->cap_Bscratch, (size_t)grid * P.bscratch_len));
-      P.Bscratch = h->Bscratch;
-    }
+  P.order = (h->lpt && !myopic && h->order_M == M && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) ? h->order.p : nullptr;
+  P.cta_done = grid <= 1024 ? h->cta_done.p : nullptr;
+  CK(h, h->cs_tape.reserve((size_t)grid * (horizon + 2) * pc.NR));
+  P.cs_tape = h->cs_tape;
+  if (pc.vglob) {
+    CK(h, h->Vscratch.reserve((size_t)grid * pc.NR * pc.RP));
+    P.Vscratch = h->Vscratch;
+    P.bscratch_len = (size_t)h->N8 * 8 * ((std::max(h->d + 1, pc.W) + 7) / 8);  // widest backward pass: q1 columns (adjoint) or W (inner solve)
+    CK(h, h->Bscratch.reserve((size_t)grid * P.bscratch_len));
+    P.Bscratch = h->Bscratch;
   }
   CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
   CK(h, cudaEventRecord(h->ev0, h->stream));
   if (pc.vglob) rbo_rollout_kernel_largen<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
   else rbo_rollout_kernel<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
   CK(h, cudaGetLastError());
-  rbo_stats_kernel<<<1, 1024, 0, h->stream>>>(h->values, mode == RBO_MODE_VALUE_GRAD ? h->grad_x : nullptr, mode == RBO_MODE_VALUE_GRAD ? h->grad_theta : nullptr,
+  rbo_stats_kernel<<<1, 1024, 0, h->stream>>>(h->values, mode == RBO_MODE_VALUE_GRAD ? h->grad_x.p : nullptr, mode == RBO_MODE_VALUE_GRAD ? h->grad_theta.p : nullptr,
                                               h->n_evals, h->best_index, h->grad_case, h->status, M, h->d, ntheta, horizon, h->sums);
   CK(h, cudaGetLastError());
   CK(h, cudaEventRecord(h->ev1, h->stream));
   if (h->lpt && !myopic && horizon > 0 && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) {
-    CK(h, dev_reserve(&h->order, &h->cap_order, (size_t)M));
+    CK(h, h->order.reserve(M));
     rbo_lpt_order_kernel<<<1, 1024, 0, h->stream>>>(h->n_evals, h->grad_case, h->best_index, M, std::max(horizon, 1), h->order);
     CK(h, cudaGetLastError());
     h->order_M = M;
   } else if (!(flags & RBO_FLAG_TEACHER_FORCED)) h->order_M = 0;
-  h->last_h = horizon; h->last_mode = mode; h->last_nth = ntheta;
+  h->last_mode = mode;
   h->xs_valid = !myopic;
   if (want_summary && summary) {
     std::vector<double> sums(h->sums_len);
     int wd[16] = {0};
+    std::vector<unsigned long long> td(grid);
     CK(h, cudaMemcpyAsync(sums.data(), h->sums, (size_t)h->sums_len * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaMemcpyAsync(wd, h->work_counter, sizeof(wd), cudaMemcpyDeviceToHost, h->stream));
+    if (P.cta_done) CK(h, cudaMemcpyAsync(td.data(), h->cta_done, (size_t)grid * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
     if (wd[1] || wd[2])
       return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", wd[1] ? "[panel pipeline wait never completed] " : "",
@@ -661,8 +679,6 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
     summary->gpu_launches = 2 + (h->order_M == M ? 1 : 0);
     summary->tail_ms = 0.0;
     if (P.cta_done) {
-      std::vector<unsigned long long> td(grid);
-      CK(h, cudaMemcpy(td.data(), h->cta_done, (size_t)grid * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
       std::sort(td.begin(), td.end());
       summary->tail_ms = (double)(td.back() - td[grid / 2]) * 1e-6;  // last CTA to finish minus the median CTA
     }
@@ -698,11 +714,34 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
   return RBO_SUCCESS;
 }
 
-static int upload_opt(rbo_handle* h, const double* src, size_t n, double** dst, size_t* cap) {
-  if (!src) return RBO_SUCCESS;
-  if (*cap < n) { CK(h, dev_realloc(dst, n)); *cap = n; }
-  CK(h, cudaMemcpyAsync(*dst, src, n * 8, cudaMemcpyHostToDevice, h->stream));
-  return RBO_SUCCESS;
+// rbo_rollout and rbo_rollout_batch: the launch on host inputs -- the dual directions (VALUE_GRAD), the forced x-path and, for a
+// batch, the B starting points x0_batch (d x B) are uploaded first -- and the per-trajectory results back to the host.
+static int rollout_host(rbo_handle* h, const double* x0, const double* x0_batch, int B, const double* theta, int ntheta, const double* lbs,
+                        const double* ubs, int horizon, double fmini, int mode, int flags, const double* dual_dirs, const double* x_forced,
+                        double* values, double* grad_x, double* grad_theta, int32_t* best_index, int32_t* grad_case, int32_t* status,
+                        rbo_summary* summary) {
+  const bool grad = mode == RBO_MODE_VALUE_GRAD;
+  const bool forced = (flags & RBO_FLAG_TEACHER_FORCED) && !(flags & RBO_FLAG_REPLAY_TAPE);
+  CK(h, cudaSetDevice(h->device));
+  const size_t Ms = (flags & RBO_FLAG_GAUSS_HERMITE) ? (size_t)h->gh_M : (size_t)h->M;
+  const size_t nd = Ms * std::max(horizon, 0) * h->d;
+  if (grad && dual_dirs) {
+    CK(h, h->dual_dirs.reserve(nd));
+    CK(h, cudaMemcpyAsync(h->dual_dirs, dual_dirs, nd * 8, cudaMemcpyHostToDevice, h->stream));
+  }
+  if (forced && x_forced) {
+    CK(h, h->x_forced.reserve(nd));
+    CK(h, cudaMemcpyAsync(h->x_forced, x_forced, nd * 8, cudaMemcpyHostToDevice, h->stream));
+  }
+  if (x0_batch) {
+    CK(h, h->x0_batch.reserve((size_t)B * h->d));
+    CK(h, cudaMemcpyAsync(h->x0_batch, x0_batch, (size_t)B * h->d * 8, cudaMemcpyHostToDevice, h->stream));
+  }
+  rbo_summary local;
+  int rc = launch_rollout(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, (grad && dual_dirs) ? h->dual_dirs.p : nullptr,
+                          forced ? h->x_forced.p : nullptr, true, summary ? summary : &local, x0_batch ? h->x0_batch.p : nullptr, B);
+  if (rc) return rc;
+  return rbo_get_results(h, values, grad ? grad_x : nullptr, grad ? grad_theta : nullptr, best_index, grad_case, status);
 }
 
 extern "C" {
@@ -713,28 +752,8 @@ int rbo_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta
   if (!h) return RBO_ERR_ARG;
   if (!values) return fail(h, RBO_ERR_ARG, "rbo_rollout: values is NULL");
   if (mode == RBO_MODE_VALUE_GRAD && (!grad_x || !grad_theta)) return fail(h, RBO_ERR_ARG, "rbo_rollout: gradient containers missing in VALUE_GRAD mode");
-  CK(h, cudaSetDevice(h->device));
-  const size_t Mrun = (flags & RBO_FLAG_GAUSS_HERMITE) ? (size_t)h->gh_M : (size_t)h->M;
-  const size_t nd = Mrun * std::max(horizon, 0) * h->d;
-  int rc = upload_opt(h, (mode == RBO_MODE_VALUE_GRAD) ? dual_dirs : nullptr, nd, &h->dual_dirs, &h->dual_cap);
-  if (rc) return rc;
-  rc = upload_opt(h, ((flags & RBO_FLAG_TEACHER_FORCED) && !(flags & RBO_FLAG_REPLAY_TAPE)) ? x_forced : nullptr, nd, &h->x_forced, &h->forced_cap);
-  if (rc) return rc;
-  rbo_summary local;
-  rc = launch_rollout(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, (mode == RBO_MODE_VALUE_GRAD && dual_dirs) ? h->dual_dirs : nullptr,
-                      ((flags & RBO_FLAG_TEACHER_FORCED) && !(flags & RBO_FLAG_REPLAY_TAPE)) ? h->x_forced : nullptr, true, summary ? summary : &local);
-  if (rc) return rc;
-  const size_t M = Mrun;
-  CK(h, cudaMemcpyAsync(values, h->values, M * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (mode == RBO_MODE_VALUE_GRAD) {
-    CK(h, cudaMemcpyAsync(grad_x, h->grad_x, M * h->d * 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(grad_theta, h->grad_theta, M * ntheta * 8, cudaMemcpyDeviceToHost, h->stream));
-  }
-  if (best_index) CK(h, cudaMemcpyAsync(best_index, h->best_index, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (grad_case) CK(h, cudaMemcpyAsync(grad_case, h->grad_case, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (status) CK(h, cudaMemcpyAsync(status, h->status, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  CK(h, cudaStreamSynchronize(h->stream));
-  return RBO_SUCCESS;
+  return rollout_host(h, x0, nullptr, 1, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs, x_forced, values, grad_x, grad_theta,
+                      best_index, grad_case, status, summary);
 }
 
 int rbo_rollout_device(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
@@ -750,24 +769,8 @@ int rbo_rollout_batch(rbo_handle* h, const double* x0s, int n_x0, const double* 
   if (!x0s || n_x0 < 1 || !values) return fail(h, RBO_ERR_ARG, "rbo_rollout_batch: bad arguments");
   if (mode == RBO_MODE_VALUE_GRAD && (!grad_x || !grad_theta)) return fail(h, RBO_ERR_ARG, "rbo_rollout_batch: gradient containers missing in VALUE_GRAD mode");
   if (!h->rn) return fail(h, RBO_ERR_STATE, "rbo_rollout_batch: no normals (rbo_set_normals / rbo_generate_normals)");
-  CK(h, cudaSetDevice(h->device));
-  const size_t Ms = (size_t)h->M, M = Ms * (size_t)n_x0, nd = Ms * std::max(horizon, 0) * h->d;
-  int rc = upload_opt(h, (mode == RBO_MODE_VALUE_GRAD) ? dual_dirs : nullptr, nd, &h->dual_dirs, &h->dual_cap);
-  if (rc) return rc;
-  CK(h, dev_reserve(&h->x0_batch, &h->cap_x0b, (size_t)n_x0 * h->d));
-  CK(h, cudaMemcpyAsync(h->x0_batch, x0s, (size_t)n_x0 * h->d * 8, cudaMemcpyHostToDevice, h->stream));
-  rbo_summary local;
-  rc = launch_rollout(h, x0s, theta, ntheta, lbs, ubs, horizon, fmini, mode, 0, (mode == RBO_MODE_VALUE_GRAD && dual_dirs) ? h->dual_dirs : nullptr, nullptr,
-                      true, summary ? summary : &local, h->x0_batch, n_x0);
-  if (rc) return rc;
-  CK(h, cudaMemcpyAsync(values, h->values, M * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (mode == RBO_MODE_VALUE_GRAD) {
-    CK(h, cudaMemcpyAsync(grad_x, h->grad_x, M * h->d * 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(grad_theta, h->grad_theta, M * ntheta * 8, cudaMemcpyDeviceToHost, h->stream));
-  }
-  if (status) CK(h, cudaMemcpyAsync(status, h->status, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  CK(h, cudaStreamSynchronize(h->stream));
-  return RBO_SUCCESS;
+  return rollout_host(h, x0s, x0s, n_x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, 0, dual_dirs, nullptr, values, grad_x, grad_theta,
+                      nullptr, nullptr, status, summary);
 }
 
 int rbo_partial_sums_device(rbo_handle* h, double* sums_device, int len) {
@@ -798,15 +801,15 @@ int rbo_partial_sums_host(rbo_handle* h, double* sums, int len) {
 int rbo_get_results(rbo_handle* h, double* values, double* grad_x, double* grad_theta, int32_t* best_index, int32_t* grad_case, int32_t* status) {
   if (!h) return RBO_ERR_ARG;
   if (h->outh < 0 || h->outM <= 0) return fail(h, RBO_ERR_STATE, "rbo_get_results: no rollout has run");
+  if ((grad_x || grad_theta) && h->last_mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_STATE, "rbo_get_results: the last rollout computed no gradients");
   CK(h, cudaSetDevice(h->device));
   const size_t M = h->outM;
-  if (values) CK(h, cudaMemcpyAsync(values, h->values, M * 8, cudaMemcpyDeviceToHost, h->stream));
-  if ((grad_x || grad_theta) && h->last_mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_STATE, "rbo_get_results: the last rollout computed no gradients");
-  if (grad_x) CK(h, cudaMemcpyAsync(grad_x, h->grad_x, M * h->outd * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (grad_theta) CK(h, cudaMemcpyAsync(grad_theta, h->grad_theta, M * h->outnth * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (best_index) CK(h, cudaMemcpyAsync(best_index, h->best_index, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (grad_case) CK(h, cudaMemcpyAsync(grad_case, h->grad_case, M * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (status) CK(h, cudaMemcpyAsync(status, h->status, M * 4, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, copy_out(values, h->values, M, h->stream));
+  CK(h, copy_out(grad_x, h->grad_x, M * h->outd, h->stream));
+  CK(h, copy_out(grad_theta, h->grad_theta, M * h->outnth, h->stream));
+  CK(h, copy_out(best_index, h->best_index, M, h->stream));
+  CK(h, copy_out(grad_case, h->grad_case, M, h->stream));
+  CK(h, copy_out(status, h->status, M, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return RBO_SUCCESS;
 }
@@ -836,13 +839,13 @@ int rbo_get_tape(rbo_handle* h, double* xs, double* ys, double* gys, double* alp
   if (h->outh < 0) return fail(h, RBO_ERR_STATE, "rbo_get_tape: no rollout has run");
   CK(h, cudaSetDevice(h->device));
   const size_t M = h->outM, hor = h->outh, hh = std::max(h->outh, 1), d = h->outd, S = h->outS;
-  if (xs) CK(h, cudaMemcpyAsync(xs, h->xs, M * (hor + 1) * d * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (ys) CK(h, cudaMemcpyAsync(ys, h->ys, M * (hor + 1) * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (gys) CK(h, cudaMemcpyAsync(gys, h->gys, M * (hor + 1) * d * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (alphas) CK(h, cudaMemcpyAsync(alphas, h->alphas, M * hh * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (n_evals) CK(h, cudaMemcpyAsync(n_evals, h->n_evals, M * hh * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (start_status) CK(h, cudaMemcpyAsync(start_status, h->start_status, M * hh * S * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (start_iters) CK(h, cudaMemcpyAsync(start_iters, h->start_iters, M * hh * S * 4, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, copy_out(xs, h->xs, M * (hor + 1) * d, h->stream));
+  CK(h, copy_out(ys, h->ys, M * (hor + 1), h->stream));
+  CK(h, copy_out(gys, h->gys, M * (hor + 1) * d, h->stream));
+  CK(h, copy_out(alphas, h->alphas, M * hh, h->stream));
+  CK(h, copy_out(n_evals, h->n_evals, M * hh, h->stream));
+  CK(h, copy_out(start_status, h->start_status, M * hh * S, h->stream));
+  CK(h, copy_out(start_iters, h->start_iters, M * hh * S, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return RBO_SUCCESS;
 }
@@ -852,11 +855,11 @@ extern "C" int rbo_get_tape_ex(rbo_handle* h, double* mu, double* sigma, double*
   if (!h->tex_valid) return fail(h, RBO_ERR_STATE, "rbo_get_tape_ex: the last rollout did not run with RBO_FLAG_TAPE_EX");
   CK(h, cudaSetDevice(h->device));
   const size_t n = (size_t)h->outM * std::max(h->outh, 0), d = h->outd;
-  if (mu) CK(h, cudaMemcpyAsync(mu, h->t_mu, n * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (sigma) CK(h, cudaMemcpyAsync(sigma, h->t_sigma, n * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (dmu) CK(h, cudaMemcpyAsync(dmu, h->t_dmu, n * d * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (dsigma) CK(h, cudaMemcpyAsync(dsigma, h->t_dsigma, n * d * 8, cudaMemcpyDeviceToHost, h->stream));
-  if (Halpha) CK(h, cudaMemcpyAsync(Halpha, h->t_Halpha, n * d * d * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, copy_out(mu, h->t_mu, n, h->stream));
+  CK(h, copy_out(sigma, h->t_sigma, n, h->stream));
+  CK(h, copy_out(dmu, h->t_dmu, n * d, h->stream));
+  CK(h, copy_out(dsigma, h->t_dsigma, n * d, h->stream));
+  CK(h, copy_out(Halpha, h->t_Halpha, n * d * d, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return RBO_SUCCESS;
 }
@@ -866,20 +869,20 @@ static int sobol_common(rbo_handle* h, int dim, int npoints, uint32_t* out_u32, 
   if (dim < 1 || dim > RBO_SOBOL_MAXDIM || npoints < 1) return fail(h, RBO_ERR_ARG, "sobol: dim %d / npoints %d out of range", dim, npoints);
   CK(h, cudaSetDevice(h->device));
   const size_t total = (size_t)dim * npoints;
-  unsigned* du = nullptr; double* df = nullptr; double* db = nullptr;
-  struct Guard { unsigned*& a; double*& b; double*& c; ~Guard() { if (a) cudaFree(a); if (b) cudaFree(b); if (c) cudaFree(c); } } guard{du, df, db};  // temporaries die on every path
-  if (out_u32) CK(h, cudaMalloc((void**)&du, total * 4));
-  if (out_f64) CK(h, cudaMalloc((void**)&df, total * 8));
+  DevBuf<unsigned> du;
+  DevBuf<double> df, db;
+  if (out_u32) CK(h, du.reserve(total));
+  if (out_f64) CK(h, df.reserve(total));
   if (lbs) {
-    CK(h, cudaMalloc((void**)&db, (size_t)2 * dim * 8));
+    CK(h, db.reserve((size_t)2 * dim));
     CK(h, cudaMemcpyAsync(db, lbs, (size_t)dim * 8, cudaMemcpyHostToDevice, h->stream));
     CK(h, cudaMemcpyAsync(db + dim, ubs, (size_t)dim * 8, cudaMemcpyHostToDevice, h->stream));
   }
   int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)h->num_sms * 8);
   rbo_sobol_kernel<<<blocks, 256, 0, h->stream>>>(h->sobol_dirs, du, df, dim, npoints, db, db ? db + dim : nullptr);
   CK(h, cudaGetLastError());
-  if (out_u32) CK(h, cudaMemcpyAsync(out_u32, du, total * 4, cudaMemcpyDeviceToHost, h->stream));
-  if (out_f64) CK(h, cudaMemcpyAsync(out_f64, df, total * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, copy_out(out_u32, du, total, h->stream));
+  CK(h, copy_out(out_f64, df, total, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return RBO_SUCCESS;
 }
@@ -926,9 +929,8 @@ int rbo_fp64_peak(rbo_handle* h, double* tflops) {
   if (!h || !tflops) return RBO_ERR_ARG;
   CK(h, cudaSetDevice(h->device));
   const int blocks = h->num_sms * 4, threads = 512, iters = 4096;
-  double* out = nullptr;
-  struct Guard { double*& p; ~Guard() { if (p) cudaFree(p); } } guard{out};
-  CK(h, cudaMalloc((void**)&out, (size_t)blocks * threads * 8));
+  DevBuf<double> out;
+  CK(h, out.reserve((size_t)blocks * threads));
   double best = 0;
   for (int rep = 0; rep < 5; ++rep) {
     CK(h, cudaEventRecord(h->ev0, h->stream));
@@ -948,10 +950,13 @@ int rbo_tr_step_batch(rbo_handle* h, int n, int B, const double* H, const double
   if (!h || !H || !g || !Delta || !p || !hit || B < 1) return RBO_ERR_ARG;
   if (n < 1 || n > RBO_MAXD) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_tr_step_batch: n = %d outside [1, %d]", n, RBO_MAXD);
   CK(h, cudaSetDevice(h->device));
-  double *dH = nullptr, *dg = nullptr, *dD = nullptr, *dp = nullptr; int* dh = nullptr;
-  struct Guard { void** p[5]; ~Guard() { for (auto q : p) if (*q) cudaFree(*q); } } guard{{(void**)&dH, (void**)&dg, (void**)&dD, (void**)&dp, (void**)&dh}};
-  CK(h, cudaMalloc((void**)&dH, (size_t)B * n * n * 8)); CK(h, cudaMalloc((void**)&dg, (size_t)B * n * 8)); CK(h, cudaMalloc((void**)&dD, (size_t)B * 8));
-  CK(h, cudaMalloc((void**)&dp, (size_t)B * n * 8)); CK(h, cudaMalloc((void**)&dh, (size_t)B * 4));
+  DevBuf<double> dH, dg, dD, dp;
+  DevBuf<int> dh;
+  CK(h, dH.reserve((size_t)B * n * n));
+  CK(h, dg.reserve((size_t)B * n));
+  CK(h, dD.reserve(B));
+  CK(h, dp.reserve((size_t)B * n));
+  CK(h, dh.reserve(B));
   CK(h, cudaMemcpyAsync(dH, H, (size_t)B * n * n * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(dg, g, (size_t)B * n * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(dD, Delta, (size_t)B * 8, cudaMemcpyHostToDevice, h->stream));
@@ -959,8 +964,8 @@ int rbo_tr_step_batch(rbo_handle* h, int n, int B, const double* H, const double
   const size_t smem = (size_t)wpb * (2 * n * n + 4 * n + 32) * 8;
   rbo_tr_step_kernel<<<(B + wpb - 1) / wpb, 32 * wpb, smem, h->stream>>>(dH, dg, dD, n, B, dp, dh);
   CK(h, cudaGetLastError());
-  CK(h, cudaMemcpyAsync(p, dp, (size_t)B * n * 8, cudaMemcpyDeviceToHost, h->stream));
-  CK(h, cudaMemcpyAsync(hit, dh, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, copy_out(p, dp, (size_t)B * n, h->stream));
+  CK(h, copy_out(hit, dh, B, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   return RBO_SUCCESS;
 }
