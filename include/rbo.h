@@ -121,7 +121,8 @@ int rbo_set_tuning(rbo_handle* h, int key, int value);
 /* The base surrogate the fantasy surrogate is built from: FantasySurrogate(s, h) (rbs.jl:345-381) reads
  * fs.X[:,1:N], fs.L[1:N,1:N], fs.y[1:N], fs.cs[1], fs.sigma_n2, fs.psi, fs.g.
  * X: d x N (ldX >= d).  L: N x N lower triangle of a column-major buffer with leading dimension ldL
- * (Julia's LowerTriangular .data).  c = K^-1 y. */
+ * (Julia's LowerTriangular .data).  c = K^-1 y.
+ * N <= 12800 bounds only the inversion into the device form; the rollout admits fewer observations (see rbo_rollout). */
 int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, const double* L, int ldL,
                       const double* y, const double* c, double sigma_n2, int kernel_id, const double* ktheta,
                       int nktheta, int rule_id, double sigma_tol);
@@ -164,6 +165,10 @@ int rbo_set_starts(rbo_handle* h, const double* starts, int S);
  *                             RBO_MODE_VALUE_GRAD (RBO_ERR_ARG otherwise), ignored in RBO_MODE_VALUE
  *   best_index, grad_case, status : int32[m_count], may be NULL (t of rollout.jl:235; case 1/2/3 of :239-251)
  *   summary                 : may be NULL
+ * Largest N: the fantasy factor block and its pitch stay in shared memory even in the large-n variant, so the largest N a
+ * rollout admits depends on d, the horizon, the number of start columns and the mode: e.g. 2640 at d = 10, h = 5 and 2296 at
+ * d = 20, h = 2 (10 start columns, with gradients, 227 KB of shared memory per block on the B200). Beyond it RBO_ERR_UNSUPPORTED;
+ * the handle stays usable (a smaller surrogate can be set).
  */
 int rbo_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs,
                 int horizon, double fmini, int mode, int flags, const double* dual_dirs, const double* x_forced,

@@ -139,6 +139,9 @@ class OracleProblem:
         p.rn, p.rn_hp1, p.starts = _ptr(self.rn), self.rn.shape[2], _ptr(self.starts)
         p.dual_dirs, p.x_forced = _ptr(self.dual_dirs), _ptr(self.x_forced)
         p.mode, p.flags, p.htol, p.nthreads = mode, flags, htol, nthreads
+        if self.x_forced is not None:  # a given x-path is followed: no inner solve runs
+            p.flags |= FLAG_TEACHER_FORCED
+            assert self.x_forced.shape == (self.d, h, self.M)
         self.gh_nodes = None if gh_nodes is None else np.asfortranarray(gh_nodes, dtype=np.float64)      # (h+1) x M
         self.gh_weights = None if gh_weights is None else np.asfortranarray(gh_weights, dtype=np.float64)
         p.gh_nodes, p.gh_weights = _ptr(self.gh_nodes), _ptr(self.gh_weights)

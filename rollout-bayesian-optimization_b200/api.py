@@ -410,14 +410,17 @@ class RolloutEngine:
             setattr(o, k, v)
         self.handle.check(self.lib.rbo_set_solver_opts(self.handle.h, C.byref(o)))
 
-    def set_tuning(self, large_n=None, large_n_slots=None, lpt=None):
-        """Execution knobs of rbo_set_tuning: force the large-n kernel variant / cap its start slots."""
+    def set_tuning(self, large_n=None, large_n_slots=None, lpt=None, row_splits=None):
+        """Execution knobs of rbo_set_tuning: force the large-n kernel variant / cap its start slots, longest-first hand-out,
+        cap the row splits of the Gram reductions (1..4, 0 = default)."""
         if large_n is not None:
             self.handle.check(self.lib.rbo_set_tuning(self.handle.h, 1, int(bool(large_n))))
         if large_n_slots is not None:
             self.handle.check(self.lib.rbo_set_tuning(self.handle.h, 2, int(large_n_slots)))
         if lpt is not None:
             self.handle.check(self.lib.rbo_set_tuning(self.handle.h, 3, int(bool(lpt))))
+        if row_splits is not None:
+            self.handle.check(self.lib.rbo_set_tuning(self.handle.h, 4, int(row_splits)))
 
     def set_htol(self, htol):
         self.handle.check(self.lib.rbo_set_htol(self.handle.h, float(htol)))

@@ -157,12 +157,26 @@ def test_sharded_normals_equal_full(pkg, orc):
     assert np.allclose(a, rn[10:27], rtol=1e-13, atol=1e-15) and np.array_equal(b, rn[10:27])
 
 
+MYOPIC_CASES = [
+    ("C2", None, "EI", None, 6, 50), ("Matern32", (0.45,), "EI", (0.0,), 3, 18), ("SquaredExponential", (0.35,), "EI", (0.0,), 3, 18),
+    ("Periodic", (0.9, 1.7), "EI", (0.0,), 3, 18), ("Matern52", (0.4,), "POI", (0.0,), 3, 18), ("Matern52", (0.4,), "LCB", (2.0,), 3, 18),
+    ("Matern52", (0.6,), "EI", (0.0,), 1, 9), ("Matern52", (0.6 * np.sqrt(31),), "EI", (0.0,), 31, 40)]
+
+
 def test_myopic_multistart_base_solve(pkg, orc):
-    wl, sur, rn, starts, dd = setup(pkg, orc, "C2", M=1, S=16)
-    ref = oracle_problem(orc, wl, sur, rn, starts, 0).multistart()
-    x = np.zeros(wl.d)
-    alpha, s = pkg.multistart_base_solve(sur, x, spatial_lbs=wl.lbs, spatial_ubs=wl.ubs, guesses=starts, θfixed=wl.theta)
-    assert relerr(x, ref["x"]) < 1e-7 and np.isclose(alpha, -ref["f"], rtol=1e-8)
+    """multistart_base_solve against the oracle's multistart: the BASELINE C2 surrogate, then the kernels and decision rules of
+    test_other_kernels_and_rules and d = 1, 31 on GP-prior data (16 + 2 starts)."""
+    for kernel, ktheta, rule, theta, d, N in MYOPIC_CASES:
+        if kernel == "C2":
+            wl, sur, rn, starts, dd = setup(pkg, orc, "C2", M=1, S=16)
+            P, lbs, ubs, theta = oracle_problem(orc, wl, sur, rn, starts, 0), wl.lbs, wl.ubs, wl.theta
+        else:
+            sur, P, rn, starts, dd, lbs, ubs, x0 = custom_case(pkg, orc, d, N, 0, 1, 16, kernel, ktheta, rule, theta)
+        assert sur.X.shape[0] == d and sur.observed == N
+        ref = P.multistart()
+        x = np.zeros(d)
+        alpha, s = pkg.multistart_base_solve(sur, x, spatial_lbs=lbs, spatial_ubs=ubs, guesses=starts, θfixed=np.array(theta, dtype=float))
+        assert relerr(x, ref["x"]) < 1e-7 and np.isclose(alpha, -ref["f"], rtol=1e-8), (kernel, rule, d, x, ref["x"], alpha, -ref["f"])
 
 
 def test_api_errors_are_loud(pkg):
@@ -187,8 +201,9 @@ def test_api_errors_are_loud(pkg):
 ORC_KERNEL = {"Matern52": "matern52", "Matern32": "matern32", "Matern12": "matern12", "SquaredExponential": "se", "Periodic": "periodic"}
 
 
-def custom_case(pkg, orc, d, N, h, M, S, kernel, ktheta, rule, theta, seed=5):
-    """A GP-prior workload with an arbitrary kernel / decision rule (the BASELINE configs all use Matern-5/2 + EI)."""
+def custom_case(pkg, orc, d, N, h, M, S, kernel, ktheta, rule, theta, seed=5, ncols=None):
+    """A GP-prior workload with an arbitrary kernel / decision rule (the BASELINE configs all use Matern-5/2 + EI).
+    ncols keeps only the first ncols of the S + 2 start columns."""
     rng = np.random.default_rng(seed)
     X = np.asfortranarray(rng.random((d, N)))
     psi = getattr(pkg, kernel)(list(ktheta))
@@ -199,19 +214,29 @@ def custom_case(pkg, orc, d, N, h, M, S, kernel, ktheta, rule, theta, seed=5):
     lbs, ubs, x0 = np.zeros(d), np.ones(d), np.full(d, 0.5)
     rn = orc.gen_low_discrepancy_sequence(M, d, h + 1)
     starts = orc.generate_initial_guesses(S, lbs, ubs)
+    if ncols is not None:
+        starts = np.asfortranarray(starts[:, :ncols])
     dd = np.asfortranarray(rng.random((d, max(h, 1), M)))
-    N_ = sur.observed
-    P = orc.OracleProblem(sur.X[:, :N_], sur.L[:N_, :N_], sur.y[:N_], sur.c[:N_], x0, lbs, ubs, rn, starts, h=h,
-                          kernel=ORC_KERNEL[kernel], ktheta=tuple(ktheta), rule=rule, theta=theta, sigma_n2=1e-6,
-                          sigma_tol=g.σtol, fmini=float(np.min(sur.y)), mode=1, dual_dirs=dd)
+    P = custom_oracle(orc, sur, x0, lbs, ubs, rn, starts, h, kernel, ktheta, rule, theta, dual_dirs=dd)
     return sur, P, rn, starts, dd, lbs, ubs, x0
 
 
-def run_custom(pkg, sur, rn, starts, dd, lbs, ubs, x0, theta, h, x_forced=None, htol=None):
+def custom_oracle(orc, sur, x0, lbs, ubs, rn, starts, h, kernel, ktheta, rule, theta, **kw):
+    """The oracle of a custom_case surrogate on any normals / starts; kw: dual_dirs, x_forced, gh_nodes, gh_weights, ..."""
+    N_ = sur.observed
+    return orc.OracleProblem(sur.X[:, :N_], sur.L[:N_, :N_], sur.y[:N_], sur.c[:N_], x0, lbs, ubs, rn, starts, h=h,
+                             kernel=ORC_KERNEL[kernel], ktheta=tuple(ktheta), rule=rule, theta=theta, sigma_n2=sur.σn2,
+                             sigma_tol=sur.g.σtol, fmini=float(np.min(sur.y)), mode=1, **kw)
+
+
+def run_custom(pkg, sur, rn, starts, dd, lbs, ubs, x0, theta, h, x_forced=None, htol=None, tuning=None, tape_ex=False):
+    """tuning: keywords of RolloutEngine.set_tuning; tape_ex also returns the extended tape under "tape_ex"."""
     eng = pkg.RolloutEngine(0)
     try:
         if htol is not None:
             eng.set_htol(htol)
+        if tuning:
+            eng.set_tuning(**tuning)
         eng.set_surrogate(pkg.FantasySurrogate(sur, h))
         eng.set_normals(rn)
         eng.set_starts(starts)
@@ -219,8 +244,10 @@ def run_custom(pkg, sur, rn, starts, dd, lbs, ubs, x0, theta, h, x_forced=None, 
         out = dict(values=np.zeros(M), grad_x=np.zeros((d, M), order="F"), grad_theta=np.zeros((len(theta), M), order="F"),
                    best_index=np.zeros(M, np.int32), grad_case=np.zeros(M, np.int32), status=np.zeros(M, np.int32))
         eng.rollout(x0, theta, lbs, ubs, h, float(np.min(sur.y)), out["values"], out["grad_x"], out["grad_theta"], dual_dirs=dd,
-                    x_forced=x_forced, best_index=out["best_index"], grad_case=out["grad_case"], status=out["status"])
+                    x_forced=x_forced, best_index=out["best_index"], grad_case=out["grad_case"], status=out["status"], tape_ex=tape_ex)
         out.update(eng.tape(h))
+        if tape_ex:
+            out["tape_ex"] = eng.tape_ex(h)
         return out
     finally:
         eng.close()
@@ -500,19 +527,25 @@ def test_full_size_properties(pkg, orc):
 
 def test_batch_of_starting_points_equals_serial_calls(pkg, orc):
     """rbo_rollout_batch (SURVEY 8 f.1: the restarts of the stochastic-ascent outer loop in one launch) is bit-identical to one
-    rbo_rollout call per starting point, and the host mirror returns one ExpectedTrajectoryOutput per column."""
-    wl, sur, rn, starts, dd = setup(pkg, orc, "C2", M=40, N=24, h=2, S=5)
+    rbo_rollout call per starting point, and the host mirror returns one ExpectedTrajectoryOutput per column. M = 64, B = 4 puts
+    more trajectories (256) in the launch than the B200 has SMs (148), so CTAs of the persistent grid take a second one."""
+    for M, B in ((40, 3), (64, 4)):
+        batch_equals_serial_calls(pkg, orc, M, B)
+
+
+def batch_equals_serial_calls(pkg, orc, M, B):
+    wl, sur, rn, starts, dd = setup(pkg, orc, "C2", M=M, N=24, h=2, S=5)
     rng = np.random.default_rng(3)
-    x0s = np.asfortranarray(wl.lbs[:, None] + (wl.ubs - wl.lbs)[:, None] * rng.random((wl.d, 3)))
+    x0s = np.asfortranarray(wl.lbs[:, None] + (wl.ubs - wl.lbs)[:, None] * rng.random((wl.d, B)))
     fmini = float(np.min(sur.y))
     eng = pkg.RolloutEngine(0)
     try:
         eng.set_surrogate(pkg.FantasySurrogate(sur, wl.h))
         eng.set_normals(rn)
         eng.set_starts(starts)
-        vb, gxb, gtb = np.zeros((wl.M, 3), order="F"), np.zeros((wl.d, wl.M, 3), order="F"), np.zeros((1, wl.M, 3), order="F")
+        vb, gxb, gtb = np.zeros((wl.M, B), order="F"), np.zeros((wl.d, wl.M, B), order="F"), np.zeros((1, wl.M, B), order="F")
         eng.rollout_batch(x0s, wl.theta, wl.lbs, wl.ubs, wl.h, fmini, vb, gxb, gtb, dual_dirs=dd)
-        for b in range(3):
+        for b in range(B):
             v, gx, gt = np.zeros(wl.M), np.zeros((wl.d, wl.M), order="F"), np.zeros((1, wl.M), order="F")
             eng.rollout(x0s[:, b], wl.theta, wl.lbs, wl.ubs, wl.h, fmini, v, gx, gt, dual_dirs=dd)
             assert np.array_equal(v, vb[:, b]) and np.array_equal(gx, gxb[:, :, b]) and np.array_equal(gt, gtb[:, :, b])
@@ -522,8 +555,8 @@ def test_batch_of_starting_points_equals_serial_calls(pkg, orc):
     T = pkg.Trajectory(sur, fs, start=wl.x0, hypers=wl.theta, horizon=wl.h)
     tp = pkg.TrajectoryParameters(wl.x0, wl.theta, wl.h, wl.M, False, wl.lbs, wl.ubs, rnstream_sequence=rn)
     etos = pkg.simulate_trajectory_mc_batch(T, tp, x0s, inner_solve_xstarts=starts, dual_directions=dd)
-    assert len(etos) == 3
-    for b in range(3):
+    assert len(etos) == B
+    for b in range(B):
         assert np.isclose(pkg.mean(etos[b]), vb[:, b].mean(), rtol=1e-13) and np.allclose(pkg.gradient(etos[b]), gxb[:, :, b].mean(axis=1), rtol=1e-12, atol=1e-15)
     # the oracle at the second starting point
     wl.x0 = x0s[:, 1].copy()

@@ -145,6 +145,22 @@ def test_oracle_vs_numpy_restatement_teacher_forced(pkg, orc):
     assert 3 in cases
 
 
+def test_oracle_follows_a_forced_x_path(pkg, orc):
+    """x_forced teacher-forces the oracle on a path that is not its own (what the parity tests feed back from the CUDA kernel): no
+    inner solve runs, the tape holds the given path, and draws and gradients are those of the numpy restatement on that path."""
+    wl, sur, rn, starts, dd, P = small_problem(pkg, orc, M=6, N=12, h=3, S=4)
+    free = P.rollout()
+    xf = np.asfortranarray(0.5 * free["xs"][:, 1:, :] + 0.25)  # inside the unit box, away from the oracle's maximisers
+    r = oracle_problem(orc, wl, sur, rn, starts, 1, dual_dirs=dd, x_forced=xf).rollout()
+    assert np.all(r["n_evals"] == 0) and np.array_equal(r["xs"][:, 1:, :], xf) and np.all(r["status"] == 0)
+    for m in range(wl.M):
+        fs, obs, grads = pr.rollout_teacher_forced(wl.X, wl.y, wl.ell, wl.sigma_n2, wl.h, wl.x0, wl.theta, rn[m], xf[:, :, m])
+        assert relerr(obs, r["ys"][:, m]) < 1e-9 and relerr(grads, r["gys"][:, :, m]) < 1e-8
+        gx, gth, case, t = pr.trajectory_gradient(fs, obs, grads, wl.theta, float(np.min(sur.y)), dd[:, :, m])
+        assert case == r["grad_case"][m] and t == r["best_index"][m]
+        assert relerr(gx, r["grad_x"][:, m], floor=max(1e-6, np.abs(gx).max())) < 1e-6
+
+
 def test_case3_gradients_are_exercised(pkg, orc):
     """With htol = 1e-4 (rollout.jl:156) and an even dimension some case-3 duals survive the det test (Q3)."""
     wl, sur, rn, starts, dd, P = small_problem(pkg, orc, name="GP:2:0.25", M=64, N=12, h=3, S=4)
