@@ -191,6 +191,48 @@ int rbo_rollout_device(rbo_handle* h, const double* x0, const double* theta, int
                        const double* ubs, int horizon, double fmini, int mode, int flags,
                        const double* dual_dirs_device, const double* x_forced_device, rbo_summary* summary);
 
+/* ---- stochastic gradient ascent of the estimator over x0 (utils.jl:235-265), all on the device --- */
+enum { RBO_OPT_SGA = 0, RBO_OPT_ADAM = 1 };                         /* StandardSGA (optimizers.jl:6-22) / Adam (optimizers.jl:25-75) */
+enum { RBO_SGA_MAXIT = 0, RBO_SGA_ESWAVS = 1, RBO_SGA_FAILED = 2 };  /* why a restart ended */
+typedef struct {
+  int32_t optimizer;      /* RBO_OPT_* */
+  int32_t max_iterations; /* estimator evaluations per restart (utils.jl:244: 50) */
+  int32_t use_eswavs;     /* stop a restart when the ESWAVS test of utils.jl:114-123 holds */
+  int32_t project;        /* 0: no projection (the reference); 1: clamp x to [lbs, ubs] after every step */
+  double eta, beta1, beta2, eps; /* step size; Adam's moment decays and denominator guard (unused by RBO_OPT_SGA) */
+} rbo_sga_opts;
+/* Adam, eta 1e-3, beta1 0.9, beta2 0.999, eps 1e-8 (optimizers.jl:35-40), 50 iterations, ESWAVS on, no projection. */
+void rbo_default_sga_opts(rbo_sga_opts* o);
+/* stochastic_solve (utils.jl:235-265) from n_x0 = B restarts at once: each restart b starts at x0s[:, b] with a fresh optimiser
+ * state and evaluates the estimator on all of this handle's samples (common random numbers across restarts and iterations, as
+ * rbo_rollout_batch). The host enqueues every iteration and synchronises once at the end. For restart b and k = 1..max_iterations:
+ *   1. the VALUE_GRAD rollout of every sample at x_k;
+ *   2. record x_k, the mean and corrected std of the values, the mean and corrected std of every grad_x row (two-pass, in a fixed
+ *      reduction order: deterministic; failed trajectories are excluded);
+ *   3. a failed trajectory ends the restart with RBO_SGA_FAILED at x_k; fail[:, b] = (first failing sample index in sample order,
+ *      as the serial reference throws there; its RBO_TRAJ_* status);
+ *   4. with use_eswavs, (1 - (M/d) * sum(g^2 / var)) > 0 (var = std^2 of the rounded std, the sum in numpy's order) ends the
+ *      restart with RBO_SGA_ESWAVS at x_k;
+ *   5. otherwise the optimiser step of api.update_optimizer / update! (optimizers.jl:16-22, 48-75), then the clamp if project.
+ * A restart that performs max_iterations evaluations ends with RBO_SGA_MAXIT and x_final is the iterate after its last step.
+ * Numerics: the step is evaluated in the reference's operation order without contractions, m = b1 m + (1-b1) g,
+ * v = b2 v + (1-b2) g g, x += (eta mhat) / (sqrt(vhat) + eps), with the bias corrections 1 - b^t computed on the host by the C
+ * library's pow: the iterates equal, bit for bit, the host mirror's update fed the recorded gradient means.
+ *   dual_dirs : d x h x m_count, shared by all restarts and iterations, or NULL = zeros
+ *   x_final   : d x B;  n_iter, end_status : B each (evaluations performed, RBO_SGA_*);  fail : 2 x B or NULL
+ *   x_hist, mean_hist, std_hist, gmean_hist, gstd_hist : NULL or d x maxit x B, maxit x B, maxit x B, d x maxit x B,
+ *               d x maxit x B (column-major); NaN past n_iter[b]
+ *   summary   : may be NULL; kernel_ms of the whole loop, gpu_launches, n_traj = trajectories run, n_failed
+ * Errors: RBO_ERR_ARG for n_x0 < 1, max_iterations < 1, an unknown optimiser or eta <= 0; RBO_ERR_STATE without surrogate,
+ * normals or starts; the plan limits of rbo_rollout (RBO_ERR_UNSUPPORTED); RBO_ERR_CUDA with the watchdog message if the rollout
+ * kernel reported a stuck pipeline (every restart stops then). Afterwards the handle keeps its surrogate, normals and starts;
+ * RBO_FLAG_REPLAY_TAPE and the per-trajectory read-backs are refused until the next rollout, because the last launch did not
+ * run every restart. One GPU only: the per-iteration statistics of several would need an all-reduce inside the loop. */
+int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
+                               const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
+                               double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail, double* x_hist,
+                               double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist, rbo_summary* summary);
+
 /* Per-handle partial statistics of the last rollout, for the multi-GPU all-reduce:
  * sums = [n, n*mean_v, M2_v, n*mean_v^2, (n*mean, M2, n*mean^2) per grad_x row..., per grad_theta row..., n_failed, watchdog]
  * length 1 + 3*(1 + d + ntheta) + 2. Written to a DEVICE buffer (e.g. a torch tensor handed to NCCL), stream-ordered.

@@ -24,6 +24,11 @@ class Summary(C.Structure):
                 ("n_evals", C.c_int64), ("gpu_launches", C.c_int32), ("tail_ms", C.c_double)]
 
 
+class SgaOpts(C.Structure):
+    _fields_ = [("optimizer", C.c_int32), ("max_iterations", C.c_int32), ("use_eswavs", C.c_int32), ("project", C.c_int32),
+                ("eta", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double)]
+
+
 # every symbol include/rbo.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "rbo_abi_version": (C.c_int, []),
@@ -50,6 +55,9 @@ SYMBOLS = {
                                      C.c_void_p, C.c_void_p, C.POINTER(Summary)]),
     "rbo_rollout_batch": (C.c_int, [C.c_void_p, _dp, C.c_int, _dp, C.c_int, _dp, _dp, C.c_int, C.c_double, C.c_int, _dp, _dp, _dp, _dp, _ip,
                                     C.POINTER(Summary)]),
+    "rbo_default_sga_opts": (None, [C.POINTER(SgaOpts)]),
+    "rbo_stochastic_solve_batch": (C.c_int, [C.c_void_p, C.POINTER(SgaOpts), _dp, C.c_int, _dp, C.c_int, _dp, _dp, C.c_int, C.c_double, _dp,
+                                             _dp, _ip, _ip, _ip, _dp, _dp, _dp, _dp, _dp, C.POINTER(Summary)]),
     "rbo_partial_sums_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "rbo_partial_sums_host": (C.c_int, [C.c_void_p, _dp, C.c_int]),
     "rbo_get_results": (C.c_int, [C.c_void_p, _dp, _dp, _dp, _ip, _ip, _ip]),

@@ -523,6 +523,27 @@ class RolloutEngine:
                                                       C.byref(s) if want_summary else None))
         return s
 
+    def stochastic_solve_batch(self, x0s, theta, lbs, ubs, horizon, fmini, dual_dirs=None, optimizer=None, max_iterations=50,
+                               use_eswavs=True, project=False):
+        """rbo_stochastic_solve_batch: stochastic_solve (utils.jl:235-265) from every column of x0s (d x B) in one library call, all
+        iterations on the device. `optimizer` (StandardSGA or an unused Adam; default Adam()) supplies the hyper-parameters only.
+        project=True clamps x to [lbs, ubs] after every step. Returns a dict: x_final (d x B), n_iter, end_status (B each: SGA_MAXIT,
+        SGA_ESWAVS, SGA_FAILED), fail (2 x B: first failing sample, its status), x_hist (d x max_iterations x B), mean_hist, std_hist
+        (max_iterations x B), gmean_hist, gstd_hist (d x max_iterations x B; NaN past n_iter) and summary."""
+        o = _sga_opts(Adam() if optimizer is None else optimizer, max_iterations, use_eswavs, project)
+        x0s, theta, lbs, ubs, dual_dirs = _sga_arrays(x0s, theta, lbs, ubs, horizon, dual_dirs, self.d, self.m_count or None)
+        d, B, T = x0s.shape[0], x0s.shape[1], int(max_iterations)
+        r = dict(x_final=np.zeros((d, B), order="F"), n_iter=np.zeros(B, np.int32), end_status=np.zeros(B, np.int32),
+                 fail=np.zeros((2, B), np.int32, order="F"), x_hist=np.zeros((d, T, B), order="F"), mean_hist=np.zeros((T, B), order="F"),
+                 std_hist=np.zeros((T, B), order="F"), gmean_hist=np.zeros((d, T, B), order="F"), gstd_hist=np.zeros((d, T, B), order="F"))
+        s = Summary()
+        self.handle.check(self.lib.rbo_stochastic_solve_batch(
+            self.handle.h, C.byref(o), dptr(x0s), B, dptr(theta), len(theta), dptr(lbs), dptr(ubs), int(horizon), float(fmini), dptr(dual_dirs),
+            dptr(r["x_final"]), iptr(r["n_iter"]), iptr(r["end_status"]), iptr(r["fail"]), dptr(r["x_hist"]), dptr(r["mean_hist"]),
+            dptr(r["std_hist"]), dptr(r["gmean_hist"]), dptr(r["gstd_hist"]), C.byref(s)))
+        r["summary"] = s
+        return r
+
     def tape(self, horizon, ntheta=1):
         M, d, S, hh = self.m_count, self.d, getattr(self, "S", 1), max(horizon, 1)
         r = dict(xs=np.zeros((d, horizon + 1, M), order="F"), ys=np.zeros((horizon + 1, M), order="F"),
@@ -593,6 +614,11 @@ def draw_dual_directions(values, best_index, d, h, rand=np.random.rand):
     return dd
 
 
+# what the reference throws where a trajectory ends with RBO_TRAJ_* status k (SURVEY.md section 5)
+_TRAJ_ERRORS = {1: "PosDefException (rbs.jl:412)", 2: "DomainError (rbs.jl:528)", 3: "PosDefException (rbs.jl:537)",
+                4: "ArgumentError: reducing over an empty collection (rbf_optim.jl:97)", 5: "SingularException (rollout.jl:188)"}
+
+
 def simulate_trajectory_mc(T, tp, *, inner_solve_xstarts, resolutions, spatial_gradients_container=None,
                            hyperparameter_gradients_container=None, dual_directions=None, device=0, keep_resident=False, rng_rand=None):
     """simulate_trajectory_mc (rollout.jl:279-340) on the GPU.
@@ -636,9 +662,7 @@ def simulate_trajectory_mc(T, tp, *, inner_solve_xstarts, resolutions, spatial_g
             eng.close()
     bad = np.nonzero(status)[0]
     if len(bad):
-        names = {1: "PosDefException (rbs.jl:412)", 2: "DomainError (rbs.jl:528)", 3: "PosDefException (rbs.jl:537)",
-                 4: "ArgumentError: reducing over an empty collection (rbf_optim.jl:97)", 5: "SingularException (rollout.jl:188)"}
-        raise RboError(f"sample {bad[0] + 1}: {names.get(int(status[bad[0]]), 'error')}")
+        raise RboError(f"sample {bad[0] + 1}: {_TRAJ_ERRORS.get(int(status[bad[0]]), 'error')}")
     μ, σ = _mean_std_rows(resolutions)
     if not want_grad:
         return ExpectedTrajectoryOutput(float(μ[0]), float(σ[0]), summary=summary)
@@ -822,3 +846,88 @@ def stochastic_solve(optimizer, T, tp, es, start, max_iterations=50, use_eswavs=
             T._engine.close()
             T._engine = None
     return tpc.x0.copy(), history
+
+
+# ----------------------------------------------------------------------------------------------------
+# The SGA loop from a batch of restarts on the device (rbo_stochastic_solve_batch)
+# ----------------------------------------------------------------------------------------------------
+SGA_MAXIT, SGA_ESWAVS, SGA_FAILED = 0, 1, 2  # RBO_SGA_*: why a restart ended
+
+
+def _sga_opts(optimizer, max_iterations, use_eswavs, project):
+    """rbo_sga_opts from a StandardSGA or Adam that supplies the hyper-parameters only: every restart starts from a fresh optimiser
+    state, so an Adam that has already stepped (t > 0) is rejected rather than silently reset."""
+    o = _lib.SgaOpts()
+    o.max_iterations, o.use_eswavs, o.project = int(max_iterations), int(bool(use_eswavs)), int(bool(project))
+    if isinstance(optimizer, Adam):
+        if optimizer.t != 0 or len(optimizer.m) or len(optimizer.v):
+            raise ValueError(f"stochastic_solve_batch: the Adam optimiser has already taken {optimizer.t} steps; every restart starts "
+                             "from a fresh state, so pass an unused Adam")
+        o.optimizer, o.eta, o.beta1, o.beta2, o.eps = 1, optimizer.η, optimizer.β1, optimizer.β2, optimizer.ε
+    elif isinstance(optimizer, StandardSGA):
+        o.optimizer, o.eta, o.beta1, o.beta2, o.eps = 0, optimizer.η, 0.0, 0.0, 0.0
+    else:
+        raise TypeError(f"stochastic_solve_batch: optimizer must be StandardSGA or Adam, not {type(optimizer).__name__}")
+    if o.max_iterations < 1:
+        raise ValueError(f"stochastic_solve_batch: max_iterations = {o.max_iterations} < 1")
+    if not o.eta > 0:
+        raise ValueError(f"stochastic_solve_batch: step size η = {o.eta} must be > 0")
+    return o
+
+
+def _sga_arrays(x0s, theta, lbs, ubs, horizon, dual_dirs, d=None, M=None):
+    """Shape checks of rbo_stochastic_solve_batch's host arrays (d, M: the engine's input dimension and samples, when known)."""
+    x0s = np.asfortranarray(x0s, dtype=np.float64)
+    if x0s.ndim != 2 or x0s.shape[1] < 1:
+        raise ValueError(f"stochastic_solve_batch: the starting points must be a d x B matrix with B >= 1, got shape {x0s.shape}")
+    if d is not None and x0s.shape[0] != d:
+        raise ValueError(f"stochastic_solve_batch: starting points of dimension {x0s.shape[0]}, the surrogate has d = {d}")
+    d = x0s.shape[0]
+    theta = np.ascontiguousarray(theta, dtype=np.float64)
+    lbs = np.ascontiguousarray(lbs, dtype=np.float64); ubs = np.ascontiguousarray(ubs, dtype=np.float64)
+    if lbs.shape != (d,) or ubs.shape != (d,):
+        raise ValueError(f"stochastic_solve_batch: bounds of shapes {lbs.shape}, {ubs.shape}; expected ({d},)")
+    if theta.ndim != 1 or len(theta) < 1:
+        raise ValueError("stochastic_solve_batch: theta must be a non-empty vector")
+    if dual_dirs is not None:
+        dual_dirs = np.asfortranarray(dual_dirs, dtype=np.float64)
+        if dual_dirs.ndim != 3 or dual_dirs.shape[:2] != (d, horizon) or (M is not None and dual_dirs.shape[2] != M):
+            raise ValueError(f"stochastic_solve_batch: dual directions of shape {dual_dirs.shape}; expected ({d}, {horizon}, M = {M})")
+    return x0s, theta, lbs, ubs, dual_dirs
+
+
+def stochastic_solve_batch(optimizer, T, tp, es, starts, max_iterations=50, use_eswavs=True, dual_directions=None, device=0):
+    """stochastic_solve (utils.jl:235-265) from every column of `starts` (d x B) at once, on the device: one library call, one
+    synchronisation. Each restart runs the loop of `stochastic_solve` with its own optimiser state (from `optimizer`'s
+    hyper-parameters; an Adam with t > 0 is rejected) and its own ESWAVS stop, on the same normals (common random numbers).
+
+    `dual_directions` (d x h x M) is shared by every restart and iteration. When None, ONE rand(d, h, M) buffer is drawn from numpy's
+    global RNG and reused, as simulate_trajectory_mc_batch does: this is not the reference's per-iteration rand(dim) consumption (Q5),
+    which `stochastic_solve` reproduces through its two-phase call.
+
+    Returns (X_final, histories): X_final is d x B (each restart's iterate after its last step, or the x at which it stopped);
+    histories[b] lists the (x, mean, grad) tuples of `stochastic_solve` for restart b. Raises RboError naming the restart and the
+    sample when a trajectory failed where the reference would have thrown."""
+    d, h, M = len(tp.x0), tp.horizon, tp.mc_iters
+    _sga_opts(optimizer, max_iterations, use_eswavs, False)
+    starts = _sga_arrays(starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, dual_directions, d, M)[0]
+    if dual_directions is None and h > 0:
+        dual_directions = np.asfortranarray(np.random.rand(d, h, M))
+    eng = RolloutEngine(device)
+    try:
+        eng.set_surrogate(T.fs)
+        eng.set_normals(tp.rnstream_sequence)
+        eng.set_starts(get_starts(es))
+        fmini = float(np.min(get_observations(T.s)))  # rollout.jl:109
+        r = eng.stochastic_solve_batch(starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, fmini, dual_dirs=dual_directions, optimizer=optimizer,
+                                       max_iterations=max_iterations, use_eswavs=use_eswavs)
+    finally:
+        eng.close()
+    failed = np.nonzero(r["end_status"] == SGA_FAILED)[0]
+    if len(failed):
+        b = int(failed[0])
+        m, code = int(r["fail"][0, b]), int(r["fail"][1, b])
+        raise RboError(f"restart {b + 1}, sample {m + 1}: {_TRAJ_ERRORS.get(code, 'error')}")
+    histories = [[(r["x_hist"][:, k, b].copy(), float(r["mean_hist"][k, b]), r["gmean_hist"][:, k, b].copy()) for k in range(int(r["n_iter"][b]))]
+                 for b in range(starts.shape[1])]
+    return r["x_final"], histories

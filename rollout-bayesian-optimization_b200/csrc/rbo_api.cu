@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "rbo_kernel.cuh"
+#include "sga_kernels.cuh"
 #include "sobol_dirs.h"
 
 namespace rbo {
@@ -126,6 +127,9 @@ struct rbo_handle {
   DevBuf<double> Ld, Linv, Xpts, wk;
   DevBuf<int> dstat;
   int ldi = 0, cap_rows = 0;
+  // rbo_stochastic_solve_batch: optimiser state, bias corrections and history (doubles); per-restart integers; the work list
+  DevBuf<double> sga_dbl;
+  DevBuf<int> sga_int, worklist;
 
   ~rbo_handle() {
     if (ev0) cudaEventDestroy(ev0);
@@ -567,9 +571,11 @@ static double f_step(double n, double d) { return 2 * n * n * (d + 1) + 2 * n * 
 // what this implementation executes per evaluation: (d+1) forward + 1 backward substitutions, Gram + two Hessian sums
 static double f_eval_exec(double n, double d) { return n * n * (d + 2) + n * (3 * d * (d + 1) + 4 * d + 40); }
 
-static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
-                          double fmini, int mode, int flags, const double* dual_dirs_dev, const double* x_forced_dev, bool want_summary,
-                          rbo_summary* summary, const double* x0_batch_dev = nullptr, int B = 1) {
+// Validates a launch, chooses its plan, makes the output and scratch buffers hold it and fills the rollout kernel's parameter block
+// P (P.order: the longest-first order of the previous launch when it applies) and its grid. Enqueues no kernel.
+static int prepare_launch(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
+                          double fmini, int mode, int flags, const double* dual_dirs_dev, const double* x_forced_dev,
+                          const double* x0_batch_dev, int B, DevProblem& P, PlanChoice& pc, int& grid) {
   const bool myopic = (flags & RBO_FLAG_MYOPIC_INTERNAL) != 0, ghq = (flags & RBO_FLAG_GAUSS_HERMITE) != 0;
   if (!h->have_sur) return fail(h, RBO_ERR_STATE, "rbo_rollout: no surrogate (rbo_set_surrogate)");
   if (ghq && !h->gh_nodes) return fail(h, RBO_ERR_STATE, "rbo_rollout: no quadrature data (rbo_set_quadrature)");
@@ -591,14 +597,12 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
     if (!(lbs[a] <= ubs[a])) return fail(h, RBO_ERR_ARG, "rbo_rollout: lower bound above upper bound in dimension %d", a);
   CK(h, cudaSetDevice(h->device));
   const int S = std::max(h->S, 1);
-  PlanChoice pc;
   if (!choose_plan(h, horizon, S, mode, &pc))
     return fail(h, RBO_ERR_UNSUPPORTED, "rbo_rollout: problem (d=%d, N=%d, h=%d) needs more than %d bytes of shared memory per CTA", h->d, h->N, horizon, h->max_smem);
   if (getenv("RBO_DEBUG")) fprintf(stderr, "[rbo] plan: W=%d RP=%d NR=%d RSmax=%d NPmax=%d xsm=%d smem=%zu B (limit %d)\n", pc.W, pc.RP, pc.NR, pc.RSmax, pc.NPmax, pc.xsm, pc.bytes, h->max_smem);
   if (getenv("RBO_DEBUG")) fprintf(stderr, "[rbo] plan: RSh=%d vglob=%d\n", pc.RSh, pc.vglob);
   int rc = ensure_outputs(h, M, horizon, S, h->d, ntheta);
   if (rc) return rc;
-  DevProblem P;
   memset(&P, 0, sizeof(P));
   P.d = h->d; P.N = h->N; P.N8 = h->N8; P.nb8 = h->nb8; P.nb32 = h->nb32; P.h = horizon; P.S = S; P.W = pc.W; P.RSmax = pc.RSmax; P.NPmax = pc.NPmax; P.xsm = pc.xsm; P.XP = h->N8 + 1;
   P.RSh = pc.RSh;
@@ -627,7 +631,7 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
     P.t_mu = h->t_mu; P.t_sigma = h->t_sigma; P.t_dmu = h->t_dmu; P.t_dsigma = h->t_dsigma; P.t_Halpha = h->t_Halpha;
     h->tex_valid = true;
   }
-  const int grid = std::min(M, h->num_sms);
+  grid = std::min(M, h->num_sms);
   // longest-first hand-out when the previous launch ran the same trajectories (same normals, nearby x0): only worth it beyond two waves
   P.order = (h->lpt && !myopic && h->order_M == M && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) ? h->order.p : nullptr;
   P.cta_done = grid <= 1024 ? h->cta_done.p : nullptr;
@@ -640,11 +644,36 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
     CK(h, h->Bscratch.reserve((size_t)grid * P.bscratch_len));
     P.Bscratch = h->Bscratch;
   }
-  CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
-  CK(h, cudaEventRecord(h->ev0, h->stream));
+  return RBO_SUCCESS;
+}
+
+// The rollout kernel of a prepared problem (the caller has cleared work_counter: the scheduler counter and the watchdog flags).
+static cudaError_t enqueue_rollout(const rbo_handle* h, const DevProblem& P, const PlanChoice& pc, int grid) {
   if (pc.vglob) rbo_rollout_kernel_largen<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
   else rbo_rollout_kernel<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
-  CK(h, cudaGetLastError());
+  return cudaGetLastError();
+}
+
+// wd: the work_counter entries the rollout kernel's watchdog writes ([1], [2] flags; [4..8] where it waited)
+static int watchdog_fail(rbo_handle* h, const int* wd) {
+  return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", wd[1] ? "[panel pipeline wait never completed] " : "",
+              wd[2] ? "[inner solve exceeded its evaluation bound]" : "", wd[4], wd[5], wd[6], wd[7], wd[8]);
+}
+
+static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
+                          double fmini, int mode, int flags, const double* dual_dirs_dev, const double* x_forced_dev, bool want_summary,
+                          rbo_summary* summary, const double* x0_batch_dev = nullptr, int B = 1) {
+  DevProblem P;
+  PlanChoice pc;
+  int grid = 0;
+  int rc = prepare_launch(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs_dev, x_forced_dev, x0_batch_dev, B, P, pc, grid);
+  if (rc) return rc;
+  flags = P.flags;
+  const bool myopic = (flags & RBO_FLAG_MYOPIC_INTERNAL) != 0;
+  const int M = P.M;
+  CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
+  CK(h, cudaEventRecord(h->ev0, h->stream));
+  CK(h, enqueue_rollout(h, P, pc, grid));
   rbo_stats_kernel<<<1, 1024, 0, h->stream>>>(h->values, mode == RBO_MODE_VALUE_GRAD ? h->grad_x.p : nullptr, mode == RBO_MODE_VALUE_GRAD ? h->grad_theta.p : nullptr,
                                               h->n_evals, h->best_index, h->grad_case, h->status, M, h->d, ntheta, horizon, h->sums);
   CK(h, cudaGetLastError());
@@ -665,9 +694,7 @@ static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, 
     CK(h, cudaMemcpyAsync(wd, h->work_counter, sizeof(wd), cudaMemcpyDeviceToHost, h->stream));
     if (P.cta_done) CK(h, cudaMemcpyAsync(td.data(), h->cta_done, (size_t)grid * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    if (wd[1] || wd[2])
-      return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", wd[1] ? "[panel pipeline wait never completed] " : "",
-                  wd[2] ? "[inner solve exceeded its evaluation bound]" : "", wd[4], wd[5], wd[6], wd[7], wd[8]);
+    if (wd[1] || wd[2]) return watchdog_fail(h, wd);
     float ms = 0;
     CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
     const int d = h->d, hh = std::max(horizon, 1), nrows = 1 + d + ntheta;
@@ -771,6 +798,143 @@ int rbo_rollout_batch(rbo_handle* h, const double* x0s, int n_x0, const double* 
   if (!h->rn) return fail(h, RBO_ERR_STATE, "rbo_rollout_batch: no normals (rbo_set_normals / rbo_generate_normals)");
   return rollout_host(h, x0s, x0s, n_x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, 0, dual_dirs, nullptr, values, grad_x, grad_theta,
                       nullptr, nullptr, status, summary);
+}
+
+void rbo_default_sga_opts(rbo_sga_opts* o) {
+  if (!o) return;
+  o->optimizer = RBO_OPT_ADAM;
+  o->max_iterations = 50;  // utils.jl:244
+  o->use_eswavs = 1;
+  o->project = 0;
+  o->eta = 1e-3;  // optimizers.jl:35-40
+  o->beta1 = 0.9;
+  o->beta2 = 0.999;
+  o->eps = 1e-8;
+}
+
+int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
+                               const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
+                               double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail_out, double* x_hist,
+                               double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist, rbo_summary* summary) {
+  if (!h) return RBO_ERR_ARG;
+  const char* me = "rbo_stochastic_solve_batch";
+  if (!o || !x0s || !x_final || !n_iter || !end_status) return fail(h, RBO_ERR_ARG, "%s: o, x0s, x_final, n_iter and end_status are required", me);
+  if (n_x0 < 1) return fail(h, RBO_ERR_ARG, "%s: n_x0 = %d < 1", me, n_x0);
+  if (o->max_iterations < 1) return fail(h, RBO_ERR_ARG, "%s: max_iterations = %d < 1", me, o->max_iterations);
+  if (o->optimizer != RBO_OPT_SGA && o->optimizer != RBO_OPT_ADAM) return fail(h, RBO_ERR_ARG, "%s: unknown optimizer %d", me, o->optimizer);
+  if (!(o->eta > 0.0)) return fail(h, RBO_ERR_ARG, "%s: eta = %g must be > 0", me, o->eta);
+  if (!h->have_sur) return fail(h, RBO_ERR_STATE, "%s: no surrogate (rbo_set_surrogate)", me);
+  if (!h->rn) return fail(h, RBO_ERR_STATE, "%s: no normals (rbo_set_normals / rbo_generate_normals)", me);
+  if (!h->starts) return fail(h, RBO_ERR_STATE, "%s: no starts (rbo_set_starts)", me);
+  CK(h, cudaSetDevice(h->device));
+  const int B = n_x0, d = h->d, Ms = h->M, maxit = o->max_iterations;
+  CK(h, h->x0_batch.reserve((size_t)B * d));
+  CK(h, cudaMemcpyAsync(h->x0_batch, x0s, (size_t)B * d * 8, cudaMemcpyHostToDevice, h->stream));
+  if (dual_dirs) {
+    const size_t nd = (size_t)Ms * std::max(horizon, 0) * d;
+    CK(h, h->dual_dirs.reserve(nd));
+    CK(h, cudaMemcpyAsync(h->dual_dirs, dual_dirs, nd * 8, cudaMemcpyHostToDevice, h->stream));
+  }
+  DevProblem P;
+  PlanChoice pc;
+  int grid = 0;
+  int rc = prepare_launch(h, x0s, theta, ntheta, lbs, ubs, horizon, fmini, RBO_MODE_VALUE_GRAD, 0, dual_dirs ? h->dual_dirs.p : nullptr, nullptr,
+                          h->x0_batch.p, B, P, pc, grid);
+  if (rc) return rc;
+  const int M = P.M;
+  // the conditions under which launch_rollout hands out longest-first; the order then follows the previous iteration's costs
+  const bool lpt = h->lpt && horizon > 0 && M > 2 * grid;
+  if (lpt) CK(h, h->order.reserve(M));
+  const int* order = P.order;
+
+  // device state: doubles [m | v | bias | x_hist | gmean_hist | gstd_hist | mean_hist | std_hist], ints [live | n_iter | end_status |
+  // fail (2 per restart) | nfail | sticky watchdog record (16)]
+  const size_t nx = (size_t)d * B, nh = (size_t)maxit * B;
+  const size_t o_bias = 2 * nx, o_xh = o_bias + 2 * (size_t)maxit, o_gmh = o_xh + nh * d, o_gsh = o_gmh + nh * d, o_mh = o_gsh + nh * d,
+               o_sh = o_mh + nh, n_dbl = o_sh + nh;
+  const size_t i_iter = B, i_end = 2 * (size_t)B, i_fail = 3 * (size_t)B, i_nfail = 5 * (size_t)B, i_sticky = 6 * (size_t)B, n_int = i_sticky + 16;
+  CK(h, h->sga_dbl.reserve(n_dbl));
+  CK(h, h->sga_int.reserve(n_int));
+  CK(h, h->worklist.reserve(M));
+  double* D = h->sga_dbl;
+  int* I = h->sga_int;
+  std::vector<double> bias(2 * (size_t)maxit);
+  for (int t = 1; t <= maxit; ++t) {  // the host mirror's 1 - beta**t: Python's float ** int is the C library's pow
+    bias[t - 1] = 1.0 - std::pow(o->beta1, (double)t);
+    bias[maxit + t - 1] = 1.0 - std::pow(o->beta2, (double)t);
+  }
+  std::vector<int> ist(n_int, 0);
+  for (int b = 0; b < B; ++b) { ist[b] = 1; ist[i_end + b] = -1; ist[i_fail + 2 * b] = -1; ist[i_fail + 2 * b + 1] = 0; }
+  CK(h, cudaMemsetAsync(D, 0, 2 * nx * 8, h->stream));
+  CK(h, cudaMemcpyAsync(D + o_bias, bias.data(), bias.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  CK(h, cudaMemsetAsync(D + o_xh, 0xff, (n_dbl - o_xh) * 8, h->stream));  // all-ones bytes: NaN past n_iter
+  CK(h, cudaMemcpyAsync(I, ist.data(), n_int * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+
+  SgaProblem S;
+  memset(&S, 0, sizeof(S));
+  S.B = B; S.Ms = Ms; S.d = d; S.maxit = maxit;
+  S.optimizer = o->optimizer; S.use_eswavs = o->use_eswavs != 0; S.project = o->project != 0;
+  S.eta = o->eta; S.beta1 = o->beta1; S.beta2 = o->beta2; S.eps = o->eps;
+  S.omb1 = 1.0 - o->beta1; S.omb2 = 1.0 - o->beta2;
+  for (int a = 0; a < d; ++a) { S.lbs[a] = lbs[a]; S.ubs[a] = ubs[a]; }
+  S.bias = D + o_bias;
+  S.values = h->values; S.grad_x = h->grad_x; S.status = h->status; S.work_counter = h->work_counter;
+  S.x = h->x0_batch; S.m = D; S.v = D + nx;
+  S.xh = D + o_xh; S.gmh = D + o_gmh; S.gsh = D + o_gsh; S.mh = D + o_mh; S.sh = D + o_sh;
+  S.live = I; S.n_iter = I + i_iter; S.end_status = I + i_end; S.fail = I + i_fail; S.nfail = I + i_nfail; S.sticky = I + i_sticky;
+
+  // every iteration enqueued at once: a launch after the last restart stopped hands out nothing
+  P.order = h->worklist;
+  int launches = 0;
+  CK(h, cudaEventRecord(h->ev0, h->stream));
+  for (int k = 0; k < maxit; ++k) {
+    rbo_sga_worklist_kernel<<<1, 1024, 0, h->stream>>>(order, S.live, Ms, M, h->worklist);
+    CK(h, cudaGetLastError());
+    CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
+    CK(h, enqueue_rollout(h, P, pc, grid));
+    rbo_sga_step_kernel<<<B, 256, 0, h->stream>>>(S, k);
+    CK(h, cudaGetLastError());
+    launches += 3;
+    if (lpt) {
+      rbo_lpt_order_kernel<<<1, 1024, 0, h->stream>>>(h->n_evals, h->grad_case, h->best_index, M, horizon, h->order);
+      CK(h, cudaGetLastError());
+      order = h->order;
+      ++launches;
+    }
+  }
+  CK(h, cudaEventRecord(h->ev1, h->stream));
+  h->order_M = lpt ? M : 0;
+  h->last_mode = RBO_MODE_VALUE_GRAD;
+  // the per-trajectory buffers now hold each restart's last iteration: no read-back and no replay until the next rollout
+  h->outM = 0; h->outh = -1; h->xs_valid = false;
+
+  std::vector<int> ires(n_int);
+  CK(h, cudaMemcpyAsync(x_final, h->x0_batch, nx * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaMemcpyAsync(ires.data(), I, n_int * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if (x_hist) CK(h, cudaMemcpyAsync(x_hist, D + o_xh, nh * d * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (gmean_hist) CK(h, cudaMemcpyAsync(gmean_hist, D + o_gmh, nh * d * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (gstd_hist) CK(h, cudaMemcpyAsync(gstd_hist, D + o_gsh, nh * d * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (mean_hist) CK(h, cudaMemcpyAsync(mean_hist, D + o_mh, nh * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (std_hist) CK(h, cudaMemcpyAsync(std_hist, D + o_sh, nh * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  std::memcpy(n_iter, ires.data() + i_iter, (size_t)B * sizeof(int));
+  std::memcpy(end_status, ires.data() + i_end, (size_t)B * sizeof(int));
+  if (fail_out) std::memcpy(fail_out, ires.data() + i_fail, 2 * (size_t)B * sizeof(int));
+  if (ires[i_sticky]) return watchdog_fail(h, ires.data() + i_sticky);
+  if (summary) {
+    float ms = 0;
+    CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+    memset(summary, 0, sizeof(*summary));
+    summary->mean = NAN;
+    summary->std = NAN;
+    summary->kernel_ms = ms;
+    summary->gpu_launches = launches;
+    long long ntraj = 0, nfailed = 0;
+    for (int b = 0; b < B; ++b) { ntraj += (long long)ires[i_iter + b] * Ms; nfailed += ires[i_nfail + b]; }
+    summary->n_traj = (int)ntraj;
+    summary->n_failed = (int)nfailed;
+  }
+  return RBO_SUCCESS;
 }
 
 int rbo_partial_sums_device(rbo_handle* h, double* sums_device, int len) {

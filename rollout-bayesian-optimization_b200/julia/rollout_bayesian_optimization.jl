@@ -12,7 +12,8 @@
 #        multistart_base_solve!(::Surrogate, xfinal; ...) rbf_optim.jl:103-134 (what both live drivers time)
 #      Julia's last-definition-wins makes this a drop-in: the drivers run unchanged;
 #   4. defines what utils.jl:235-265 calls but HEAD never defines -- simulate_adjoint_trajectory(surrogate, tp; ...) -- and re-defines
-#      stochastic_solve so that the surrogate, normals and starts stay RESIDENT on the device across the ascent iterations.
+#      stochastic_solve so that the surrogate, normals and starts stay RESIDENT on the device across the ascent iterations;
+#      stochastic_solve_batch runs the whole ascent from a batch of restarts on the device in one call.
 #
 # Resident inputs: the handle remembers a fingerprint of the surrogate / normals / starts it holds and re-uploads only what changed
 # (a BO iteration changes the surrogate; an ascent iteration changes only x0). rbo_condition! appends an observation on the device.
@@ -354,6 +355,45 @@ function stochastic_solve(; optimizer::StochasticGradientAscent, surrogate::Surr
         update!(optimizer, x = get_starting_point(tpc), ∇f = gradient(eto))                            # optimizers.jl:16-22, 48-75
     end
     return get_starting_point(tpc)
+end
+
+# Not in the reference: stochastic_solve from every column of `starts` (d x B) in ONE library call (rbo_stochastic_solve_batch): each
+# restart has its own optimiser state (from `optimizer`'s hyper-parameters; every restart starts fresh) and its own ESWAVS stop, all
+# iterations run on the device and the host synchronises once. The dual directions are one rand(d, h, M) buffer shared by every
+# restart and iteration (not the per-iteration rand(dim) consumption of stochastic_solve). Returns the d x B final iterates.
+# Like the rest of this file it is not run in the build environment (no Julia); the Python mirror api.stochastic_solve_batch drives
+# the same entry point in the tests.
+struct RboSgaOpts
+    optimizer::Int32; max_iterations::Int32; use_eswavs::Int32; project::Int32
+    eta::Float64; beta1::Float64; beta2::Float64; eps::Float64
+end
+function _rbo_sga_opts(o::StochasticGradientAscent)
+    o isa Adam || return RboSgaOpts(0, 50, 1, 0, o.η, 0.0, 0.0, 0.0)                       # StandardSGA (optimizers.jl:6-22)
+    o.t == 0 || error("stochastic_solve_batch: the Adam optimiser has already stepped; pass an unused one")
+    return RboSgaOpts(1, 50, 1, 0, o.η, o.β1, o.β2, hasproperty(o, :ϵ) ? o.ϵ : o.ε)          # optimizers.jl:25-40; utils.jl:244
+end
+function stochastic_solve_batch(; optimizer::StochasticGradientAscent, surrogate::Surrogate, tp::TrajectoryParameters, es::ExperimentSetup,
+                                starts::Matrix{Float64})
+    h = _rbo_handle()
+    T = _rbo_trajectory(surrogate, tp)
+    _rbo_sync_surrogate!(h, get_fantasy_surrogate(T))
+    _rbo_sync_normals!(h, tp.rnstream_sequence)
+    _rbo_sync_starts!(h, get_starts(es))
+    M, d, hor, B = tp.mc_iters, length(tp.x0), tp.horizon, size(starts, 2)
+    θ = Vector{Float64}(tp.θ)
+    dual = rand(d, max(hor, 1), M)
+    opts = Ref(_rbo_sga_opts(optimizer))
+    xfinal = zeros(d, B); n_iter = zeros(Int32, B); end_status = zeros(Int32, B); fail = zeros(Int32, 2, B)
+    _rbo_check(h, ccall((:rbo_stochastic_solve_batch, librbo), Cint,
+        (Ptr{Cvoid}, Ref{RboSgaOpts}, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64},
+         Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cvoid}),
+        h.ptr, opts, starts, B, θ, length(θ), tp.spatial_lbs, tp.spatial_ubs, hor, minimum(get_observations(surrogate)), dual,
+        xfinal, n_iter, end_status, fail, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL))
+    for b in 1:B
+        end_status[b] == 2 || continue                                                      # RBO_SGA_FAILED: the serial loop would throw
+        error("restart $b, sample $(fail[1, b] + 1): " * get(_RBO_STATUS, Int(fail[2, b]), "error"))
+    end
+    return xfinal
 end
 
 
