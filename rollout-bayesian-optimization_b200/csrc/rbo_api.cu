@@ -15,19 +15,12 @@
 
 #include "rbo_kernel.cuh"
 #include "sga_kernels.cuh"
+#include "support_kernels.cuh"
 #include "sobol_dirs.h"
 
 namespace rbo {
 __global__ void rbo_rollout_kernel(const __grid_constant__ DevProblem P);
 __global__ void rbo_rollout_kernel_largen(const __grid_constant__ DevProblem P);  // same source, work matrix in global memory
-__global__ void rbo_normals_kernel(const unsigned* dirs, double* out, int M_total, int d, int H, int m_begin, int m_count);
-__global__ void rbo_sobol_kernel(const unsigned* dirs, unsigned* out_u32, double* out_f64, int dim, int npoints, const double* lbs, const double* ubs);
-__global__ void rbo_stats_kernel(const double* values, const double* gx, const double* gth, const int* n_evals, const int* best_index, const int* grad_case,
-                                 const int* status, int M, int d, int nth, int h, double* sums);
-__global__ void rbo_fp64_peak_kernel(double* out, int iters);
-__global__ void rbo_tr_step_kernel(const double* H, const double* g, const double* Delta, int n, int B, double* p, int* hit);
-__global__ void rbo_gather_sums_kernel(const double* sums, int need, int idx_failed, const int* work_counter, double* out);
-__global__ void rbo_lpt_order_kernel(const int* n_evals, const int* grad_case, const int* best_index, int M, int hh, int* order);
 // surrogate_kernels.cu
 __global__ void rbo_trinv_kernel(const double* L, int N, int N32, double* Linv, int ldi);
 __global__ void rbo_pack_fwd_kernel(const double* Linv, int ldi, int nb32, double* Lf);

@@ -20,7 +20,8 @@
 // This file is compiled twice (see the Makefile): RBO_VGLOB = 0 is the kernel whose work matrix V lives in shared memory
 // (rbo_rollout_kernel; the compiler then addresses V with shared-memory instructions), RBO_VGLOB = 1 the large-n variant
 // whose V is a per-CTA scratch in global memory that stays L2-resident (rbo_rollout_kernel_largen; north_star: "L0 ... read
-// through L2 when n is large", BASELINE config C5 with n = 1000, d = 20). Everything else is the same code.
+// through L2 when n is large", BASELINE config C5 with n = 1000, d = 20). Everything else is the same code. The trust-region
+// step is in trust_region.cuh, the small kernels around a launch in support_kernels.cu.
 #include "rbo_kernel.cuh"
 
 #ifndef RBO_VGLOB
@@ -42,51 +43,32 @@
 #define RBO_KERNEL_NAME rbo_rollout_kernel
 #endif
 
-namespace rbo {
-
 #ifdef RBO_PHASE_TIMERS
+namespace rbo {
 __device__ unsigned long long g_phase_cycles[16];
-__device__ unsigned long long g_aux_cycles[16];  // tri_solve sub-phases seen by warp 0: [8*bwd + {setup, fan-pre, chunks, mma, diag, fan-post, calls}]
+__device__ unsigned long long g_aux_cycles[16];  // histogram of the per-start solver-step durations (slot_logic_warp), bins of 4000 cycles, the last one open
 __device__ unsigned long long g_tr_cycles[16];   // per-start logic, summed over all logic warps: [calls, pre, tr step, post, tr: load, householder, write-out, probes, solve, back-transform]
+}  // namespace rbo
 #define TR_T(v) long long v = clock64()
 #define TR_ADD(i, t0, t1) do { if ((threadIdx.x & 31) == 0) atomicAdd(&g_tr_cycles[i], (unsigned long long)((t1) - (t0))); } while (0)
-#define AUX_T(v) long long v = clock64()
-#define AUX_ADD(i, t0) do { } while (0)
 #define PT_DECL long long pt_t0 = clock64()
 #define PT_MARK(i) do { if (threadIdx.x == 0) { long long t1_ = clock64(); atomicAdd(&g_phase_cycles[i], (unsigned long long)(t1_ - pt_t0)); pt_t0 = t1_; } } while (0)
 #else
 #define PT_DECL
 #define PT_MARK(i)
-#define AUX_T(v)
-#define AUX_ADD(i, t0)
-#define TR_T(v)
-#define TR_ADD(i, t0, t1)
 #endif
+#include "trust_region.cuh"
+
+namespace rbo {
 
 namespace {
 
 // int-area layout
 enum { I_M = 0, I_NACT = 1, I_TSTATUS = 2, I_BEST = 3, I_EVALS = 4, I_T = 5, I_CASE = 6, I_NEXT = 7, I_ARR = 64 };
-constexpr unsigned FULL = 0xffffffffu;
 #ifndef RBO_SPIN_CAP
 #define RBO_SPIN_CAP (1u << 28)  // polls of an mbarrier before the wait is declared dead (seconds; a healthy wait takes microseconds)
 #endif
 
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(FULL, v, off);
-  return v;
-}
-__device__ __forceinline__ double warp_max(double v) {
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) v = fmax(v, __shfl_xor_sync(FULL, v, off));
-  return v;
-}
-__device__ __forceinline__ double warp_min(double v) {
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) v = fmin(v, __shfl_xor_sync(FULL, v, off));
-  return v;
-}
 // max over the warp of a value that is >= 0 in every lane: the IEEE bit pattern of non-negative doubles is monotone, so two integer
 // REDUX instructions replace five shuffle rounds (a shuffle costs ~45 cycles of latency on B200)
 __device__ __forceinline__ double warp_max_nonneg(double v) {
@@ -97,6 +79,13 @@ __device__ __forceinline__ double warp_max_nonneg(double v) {
 }
 // index of (p, q), p <= q, in the row-major upper triangle of an n x n matrix
 __device__ __forceinline__ int tri_idx(int p, int q, int n) { return p * n - (p * (p - 1)) / 2 + (q - p); }
+// sum of the RS row-split partial sums part[r * stride + e] of a reduction, in a fixed order from 0.0: results do not depend
+// on which warp computed which split
+__device__ __forceinline__ double split_sum(const double* part, int RS, int stride, int e) {
+  double s = 0.0;
+  for (int r = 0; r < RS; ++r) s += part[(size_t)r * stride + e];
+  return s;
+}
 
 __device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
@@ -277,442 +266,6 @@ __device__ __noinline__ void bwd_direct(double* V, const double* Fp, const int* 
 #endif
   }
 
-
-// ------------------------------------------------------------------------------------------------
-// Exact trust-region step by one warp for n <= 16 free coordinates (solve_tr, optim.jl:9-51; same algorithm and candidate grid
-// as oracle/rbo_oracle.cpp::tr_step and as tr_step_warp below, which stays the path for n > 16). The per-start logic is a latency
-// chain on one warp while the rest of the CTA waits (FP64: 8.4 cycles per dependent FMA, 118 per division, 86 per sqrt, ~45 per
-// shared-memory load on B200, profiles/r3_lat_bench.txt), so this version keeps everything in REGISTERS: lane l owns row l >> 1,
-// columns 8 (l & 1) .. +7 of the (zero-padded) 16 x 16 matrix and of the accumulated orthogonal factor Q; the k loop of the
-// Householder tridiagonalisation is fully unrolled (static register indices), the reflector column is fetched from row k's lanes
-// by shuffles (A is symmetric), the row sums are 8 local FMAs + one exchange with the partner lane, the reflector is normalised
-// with rsqrt + one reciprocal instead of sqrt + division, and Q <- Q (I - beta v v') rides along off the critical path so that
-// Q'g and p = Q h are single products (no serial loop over the reflectors).
-//   H, g: d x d / d (shared memory); fr[0..n): free coordinates; ta, te, yv: >= n doubles each (diagonal / sub-diagonal of T,
-//   Q'g then the step). Returns "hit_constraint"; the step p is left in yv[0..n).
-// ------------------------------------------------------------------------------------------------
-// Branch-free reciprocal / reciprocal square root for NORMAL positive arguments (no special cases; ~1 ulp). The library versions end
-// in a slow-path branch that keeps the compiler from interleaving independent chains (the two candidate shifts of a lane ran one
-// after the other: 310 cycles per pivot instead of ~90, profiles/r3_tr_bench.txt).
-__device__ __forceinline__ double rcp_fast(double x) {
-  double r;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
-  double e = fma(-x, r, 1.0);
-  r = fma(r, e, r);
-  e = fma(-x, r, 1.0);
-  return fma(r, e, r);
-}
-__device__ __forceinline__ double rsqrt_fast(double x) {
-  double r;
-  asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
-  const double e = fma(-x, r * r, 1.0);  // 1 - x r^2
-  return fma(r * e, fma(0.375, e, 0.5), r);
-}
-__device__ __forceinline__ double rowsum16(double v) {  // sum over the 16 rows; the two lanes of a row hold the same value
-  v += __shfl_xor_sync(FULL, v, 2); v += __shfl_xor_sync(FULL, v, 4); v += __shfl_xor_sync(FULL, v, 8); v += __shfl_xor_sync(FULL, v, 16);
-  return v;
-}
-// Two candidate shifts per lane: 0 = admissible, 1 = positive definite but |h(lam)| > Delta, 2 = not positive definite.
-// Forward LDL' recurrences of T + lam I (pivots d_i, z = L^-1 b) and their lam-derivatives (d_i', z_i'), no storage:
-// |h(lam)|^2 = b'(T + lam I)^-2 b = -d/dlam sum z_i^2 / d_i = sum q_i (q_i d_i' - 2 z_i'), q_i = z_i / d_i.
-__device__ __forceinline__ void tri_probe2_t(const double* ta, const double* te, const double* yv, int n, double lamA, double lamB, double D2, int& outA, int& outB) {
-  const double lam[2] = {lamA, lamB};
-  double q[2], r[2], dd[2], zd[2], acc[2];
-  bool ok[2];
-  const double b0 = yv[0], a0 = ta[0];
-#pragma unroll
-  for (int c = 0; c < 2; ++c) {
-    const double dn = a0 + lam[c];
-    ok[c] = dn > 0.0; r[c] = rcp_fast(dn); dd[c] = 1.0; zd[c] = 0.0; q[c] = b0 * r[c]; acc[c] = q[c] * q[c];
-  }
-#pragma unroll 2
-  for (int i = 1; i < n; ++i) {
-    const double e = te[i - 1], a = ta[i], b = yv[i];
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const double er = e * r[c], dn = fma(-e, er, a + lam[c]);
-      const double ddn = fma(er * er, dd[c], 1.0), zn = fma(-e, q[c], b), zdn = er * fma(q[c], dd[c], -zd[c]);
-      ok[c] = ok[c] && dn > 0.0;
-      r[c] = rcp_fast(dn);
-      q[c] = zn * r[c];
-      acc[c] = fma(q[c], fma(q[c], ddn, -2.0 * zdn), acc[c]);
-      dd[c] = ddn; zd[c] = zdn;
-    }
-  }
-  outA = ok[0] ? (acc[0] <= D2 ? 0 : 1) : 2;
-  outB = ok[1] ? (acc[1] <= D2 ? 0 : 1) : 2;
-}
-// lane i: component i of -(T + lam I)^-1 b, b[0..n) in shared memory; the pivots must be positive
-__device__ __forceinline__ double tri_solve_dist_t(const double* ta, const double* te, const double* b, int n, double lam, int lane) {
-  double myr = 0.0, myz = 0.0, r = 0.0, z = 0.0;
-  for (int i = 0; i < n; ++i) {
-    const double bi = b[i];
-    if (i == 0) { r = rcp_fast(ta[0] + lam); z = bi; }
-    else { const double e = te[i - 1], er = e * r; r = rcp_fast(fma(-e, er, ta[i] + lam)); z = fma(-er, z, bi); }
-    if (lane == i) { myr = r; myz = z; }
-  }
-  const double e_up = (lane + 1 < n) ? te[lane] : 0.0;
-  double hv = 0.0;
-  for (int i = n - 1; i >= 0; --i) {
-    const double hn = __shfl_sync(FULL, hv, (i + 1) & 31);
-    if (lane == i) hv = (myz - ((i + 1 < n) ? e_up * hn : 0.0)) * myr;
-  }
-  return -hv;
-}
-__device__ __noinline__ bool tr_step16(const double* H, const double* g, const int* fr, int n, int d, double Delta, double* ta, double* te, double* yv) {
-  // the lane id is read through a volatile asm so that nothing derived from it is hoisted out of the solver loop and kept live
-  // across the tensor-core phases (the kernel sits at the 128-register cap)
-  int lane;
-  asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane));
-  const int row = lane >> 1, hf = lane & 1, c0 = 8 * hf;
-  const bool rin = row < n;
-  const int fi = rin ? fr[row] : 0;
-  TR_T(q0_);
-  double a[8], Q[8];  // my 8 columns of the matrix row and of the row of Q
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int j = c0 + c;
-    a[c] = 0.0;
-    if (rin && j < n) a[c] = H[fi * d + fr[j]];
-    Q[c] = (row == j) ? 1.0 : 0.0;
-  }
-  const double gi = rin ? g[fi] : 0.0;
-  const double gn = sqrt(rowsum16(gi * gi));
-  TR_T(q1_); TR_ADD(4, q0_, q1_);
-  // ---- Householder tridiagonalisation H_FF = Q T Q'. Step k with x = column k below the diagonal,
-  // v = x - alpha e1, beta = 2 / |v|^2, p = beta A v, w = p - (beta p'v / 2) v, A <- A - v w' - w v'. A warp shuffle costs ~45 cycles
-  // of latency and ~5-8 of issue on B200 (profiles/r3_shfl_bench.txt): the step is arranged for the fewest shuffles (24 doubles).
-#pragma unroll
-  for (int k = 0; k < 14; ++k) {
-    if (k + 2 < n) {
-      // column k below the diagonal = row k right of the diagonal: fetched from row k's lanes
-      double v[8];
-#pragma unroll
-      for (int c = 0; c < 8; ++c) { const double t = __shfl_sync(FULL, a[c], 2 * k + hf); v[c] = (c0 + c > k) ? t : 0.0; }
-      double vi = __shfl_sync(FULL, a[k & 7], (lane & ~1) | (k >> 3));  // A[row][k]
-      if (row <= k) vi = 0.0;
-      const double x0 = __shfl_sync(FULL, a[(k + 1) & 7], 2 * k + ((k + 1) >> 3));            // A[k][k+1]
-      const double aik1 = __shfl_sync(FULL, a[(k + 1) & 7], (lane & ~1) | ((k + 1) >> 3));    // A[row][k+1]
-      const double qk1 = __shfl_sync(FULL, Q[(k + 1) & 7], (lane & ~1) | ((k + 1) >> 3));     // Q[row][k+1]
-      double s0 = 0.0, s1 = 0.0, t0 = 0.0, t1 = 0.0, u0 = 0.0, u1 = 0.0;
-#pragma unroll
-      for (int c = 0; c < 8; c += 2) {
-        s0 = fma(v[c], v[c], s0); s1 = fma(v[c + 1], v[c + 1], s1);
-        t0 = fma(a[c], v[c], t0); t1 = fma(a[c + 1], v[c + 1], t1);
-        u0 = fma(Q[c], v[c], u0); u1 = fma(Q[c + 1], v[c + 1], u1);
-      }
-      const double sl = s0 + s1, tl = t0 + t1, ul = u0 + u1;
-      const double xn2 = sl + __shfl_xor_sync(FULL, sl, 1);
-      const double traw = tl + __shfl_xor_sync(FULL, tl, 1);  // (A x)_row
-      const double uraw = ul + __shfl_xor_sync(FULL, ul, 1);  // (Q x)_row
-      if (!(xn2 - x0 * x0 > 0.0)) continue;                   // column already reduced (uniform)
-      const double rs = rsqrt_fast(xn2), sq = xn2 * rs;        // |x|
-      const double alpha = x0 > 0.0 ? -sq : sq;
-      const double bk = rcp_fast(fma(fabs(x0), sq, xn2));      // beta = 2 / |x - alpha e1|^2
-      const double v1 = x0 - alpha;
-      if (row == k + 1) vi = v1;
-      if (((k + 1) >> 3) == hf) v[(k + 1) & 7] = v1;
-      const double pw = (row > k) ? bk * fma(-aik1, alpha, traw) : 0.0;  // beta (A v)_row, A v = A x - alpha A[:, k+1]
-      double w[8];
-#pragma unroll
-      for (int c = 0; c < 8; ++c) w[c] = __shfl_sync(FULL, pw, 2 * (c0 + c));  // p_j for my columns
-      double q0 = 0.0, q1 = 0.0;
-#pragma unroll
-      for (int c = 0; c < 8; c += 2) { q0 = fma(w[c], v[c], q0); q1 = fma(w[c + 1], v[c + 1], q1); }
-      const double ql = q0 + q1;
-      const double pv = ql + __shfl_xor_sync(FULL, ql, 1);
-      const double nkk = -0.5 * bk * pv, wi = fma(nkk, vi, pw);
-#pragma unroll
-      // The update must keep A BITWISE symmetric (the reflector column is read from row k): v_i w_j + w_i v_j is formed from two
-      // rounded products and one commutative addition, never contracted into FMAs. With a merely approximately symmetric A the
-      // two copies of a rounding-noise column differ by O(1) relative and the transformation stops being a similarity -- that
-      // corrupted the near-zero eigenvalues of rank-deficient Hessians (tests: test_trust_region_step_matches_the_oracle_step).
-      for (int c = 0; c < 8; ++c) { const double wj = fma(nkk, v[c], w[c]); a[c] = __dsub_rn(a[c], __dadd_rn(__dmul_rn(vi, wj), __dmul_rn(wi, v[c]))); }
-      if (lane == 2 * (k + 1) + (k >> 3)) a[k & 7] = alpha;                       // sub-diagonal of T
-      // Q <- Q (I - beta v v'): off the critical path
-      const double tq = bk * fma(-qk1, alpha, uraw);
-#pragma unroll
-      for (int c = 0; c < 8; ++c) Q[c] = fma(-tq, v[c], Q[c]);
-    }
-  }
-  TR_T(q2_); TR_ADD(5, q1_, q2_);
-  // T and Q'g to shared memory: every lane needs all of them for the shift search
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int j = c0 + c;
-    if (row == j && rin) ta[row] = a[c];
-    if (row == j + 1 && rin) te[j] = a[c];
-  }
-  {
-    // (Q'g)_j = sum over the rows of Q[row][j] g_row as a reduce-scatter: every round halves the columns a lane keeps and doubles
-    // the rows they cover (8 double shuffles instead of 32); the lane ends with column c0 + 4 b4 + 2 b3 + b2 (bK = bit K of the lane)
-    const bool b4 = (lane & 16) != 0, b3 = (lane & 8) != 0, b2 = (lane & 4) != 0;
-    double k4[4], k2[2];
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      const double lo_ = Q[c] * gi, hi_ = Q[c + 4] * gi;
-      k4[c] = (b4 ? hi_ : lo_) + __shfl_xor_sync(FULL, b4 ? lo_ : hi_, 16);
-    }
-#pragma unroll
-    for (int c = 0; c < 2; ++c) k2[c] = (b3 ? k4[c + 2] : k4[c]) + __shfl_xor_sync(FULL, b3 ? k4[c] : k4[c + 2], 8);
-    double k1 = (b2 ? k2[1] : k2[0]) + __shfl_xor_sync(FULL, b2 ? k2[0] : k2[1], 4);
-    k1 += __shfl_xor_sync(FULL, k1, 2);
-    const int j = c0 + (b4 ? 4 : 0) + (b3 ? 2 : 0) + (b2 ? 1 : 0);
-    if ((lane & 2) == 0 && j < n) yv[j] = k1;
-  }
-  __syncwarp();
-  const bool in = lane < n;
-  double glo = INFINITY;
-  if (in) glo = ta[lane] - (lane > 0 ? fabs(te[lane - 1]) : 0.0) - (lane + 1 < n ? fabs(te[lane]) : 0.0);
-  glo = warp_min(glo);  // Gershgorin lower bound of lambda_min(T)
-  const double D2 = Delta * Delta;
-  double lo = 0.0, hi = fmax(0.0, -glo) + gn / Delta;
-  bool hit = true, lo_notpd = false;
-  TR_T(q3_); TR_ADD(6, q2_, q3_);
-  for (int round = 0; round < RBO_TR_ROUNDS; ++round) {
-    // 64 candidates per round, two per lane (c = lane, lane + 32); the last one is hi, known to be admissible
-    const double base = lo, wd = hi - lo;
-    const double lamA = (round == 0) ? wd * (double)lane / 63.0 : base + wd * (double)(lane + 1) / 64.0;
-    const double lamB = (round == 0) ? wd * (double)(lane + 32) / 63.0 : base + wd * (double)(lane + 33) / 64.0;
-    int oa, ob;
-    tri_probe2_t(ta, te, yv, n, lamA, lamB, D2, oa, ob);
-    const unsigned long long adm = ((unsigned long long)__ballot_sync(FULL, ob == 0) << 32) | __ballot_sync(FULL, oa == 0) | (1ull << 63);
-    const unsigned long long pdm = ((unsigned long long)__ballot_sync(FULL, ob != 2) << 32) | __ballot_sync(FULL, oa != 2);
-    const int cf = __ffsll((long long)adm) - 1;
-    if (round == 0) {
-      if (cf == 0) { hi = 0.0; hit = false; break; }
-      lo_notpd = ((pdm >> (cf - 1)) & 1ull) == 0ull;
-      hi = (cf == 63) ? hi : wd * (double)cf / 63.0;
-      lo = wd * (double)(cf - 1) / 63.0;
-    } else {
-      if (cf > 0) lo_notpd = ((pdm >> (cf - 1)) & 1ull) == 0ull;
-      hi = (cf == 63) ? hi : base + wd * (double)(cf + 1) / 64.0;
-      lo = (cf == 0) ? base : base + wd * (double)cf / 64.0;
-    }
-  }
-  TR_T(q4_); TR_ADD(7, q3_, q4_);
-  double h = tri_solve_dist_t(ta, te, yv, n, hi, lane);
-  if (hit && lo_notpd) {
-    const double hn2 = warp_sum(in ? h * h : 0.0);
-    if (hn2 < D2) {  // hard case (to the resolution of the search): complete along the lowest eigenvector of T
-      __syncwarp();
-      if (in) yv[lane] = 1.0;
-      __syncwarp();
-      double z = 0.0;
-      for (int itn = 0; itn < 2; ++itn) {
-        const double z2 = tri_solve_dist_t(ta, te, yv, n, hi, lane);
-        const double zn = 1.0 / sqrt(warp_sum(in ? z2 * z2 : 0.0));
-        z = in ? z2 * zn : 0.0;
-        __syncwarp();
-        if (in) yv[lane] = z;
-        __syncwarp();
-      }
-      const double hz = warp_sum(in ? h * z : 0.0);
-      const double tau = -hz + sqrt(fmax(hz * hz + (D2 - hn2), 0.0));
-      h += tau * z;
-    }
-  }
-  TR_T(q5_); TR_ADD(8, q4_, q5_);
-  // ---- p = Q h, row layout again
-  __syncwarp();
-  if (in) yv[lane] = h;
-  __syncwarp();
-  double p0 = 0.0, p1 = 0.0;
-#pragma unroll
-  for (int c = 0; c < 8; c += 2) {
-    const double h0 = (c0 + c < n) ? yv[c0 + c] : 0.0, h1 = (c0 + c + 1 < n) ? yv[c0 + c + 1] : 0.0;
-    p0 = fma(Q[c], h0, p0); p1 = fma(Q[c + 1], h1, p1);
-  }
-  const double pl_ = p0 + p1;
-  const double pr = pl_ + __shfl_xor_sync(FULL, pl_, 1);
-  __syncwarp();
-  if (hf == 0 && rin) yv[row] = pr;
-  __syncwarp();
-  TR_T(q6_); TR_ADD(9, q5_, q6_);
-  return hit;
-}
-
-// ------------------------------------------------------------------------------------------------
-// Exact trust-region step by one warp (solve_tr, optim.jl:9-51): minimise g'p + p'Hp/2, |p|_2 <= Delta over the free
-// coordinates fr[0..n). Lane i < n owns row i / component i of the reduced system; the step p is left in yv[0..n). General n <= 32; tr_step16 is the fast path. A: n x n scratch.
-// Householder tridiagonalisation H_FF = Q T Q' (reflectors kept in A below the sub-diagonal), then the admissible shifts
-// S = {lam >= 0: T + lam I positive definite, |h(lam)| <= Delta} = [lam*, inf) are searched by RBO_TR_ROUNDS rounds of 32-way
-// multisection -- lane j tests one candidate with the forward LDL' recurrences and their lam-derivatives (no storage) --;
-// lam* = 0 is the interior Newton step, the hard case is completed along the lowest eigenvector (optim.jl:39-46).
-// Same algorithm, candidate grid included, as oracle/rbo_oracle.cpp::tr_step.
-// ------------------------------------------------------------------------------------------------
-// Two candidate shifts per lane: 0 = admissible, 1 = positive definite but |h(lam)| > Delta, 2 = not positive definite.
-// yv[i] = component i of Q'g (shared memory). Forward LDL' recurrences of T + lam I and their lam-derivatives:
-// |h(lam)|^2 = b'(T + lam I)^-2 b = -d/dlam sum z_i^2 / d_i, no storage, no backward pass.
-__device__ __forceinline__ void tri_probe2(const double* A, const double* yv, int n, double lamA, double lamB, double D2, int& outA, int& outB) {
-  const double lam[2] = {lamA, lamB};
-  double z[2], r[2], dd[2], zd[2], acc[2];
-  bool ok[2];
-  const double b0 = yv[0], a0 = A[0];
-#pragma unroll
-  for (int c = 0; c < 2; ++c) {
-    const double dn = a0 + lam[c];
-    ok[c] = dn > 0.0; r[c] = 1.0 / dn; dd[c] = 1.0; zd[c] = 0.0; z[c] = b0; acc[c] = (b0 * b0) * r[c] * r[c];
-  }
-  for (int i = 1; i < n; ++i) {
-    const double e = A[i * n + i - 1], a = A[i * n + i], b = yv[i];
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const double er = e * r[c], dn = a + lam[c] - e * er;
-      const double ddn = fma(er * er, dd[c], 1.0), zn = b - er * z[c], zdn = er * (r[c] * dd[c] * z[c] - zd[c]);
-      ok[c] = ok[c] && dn > 0.0;
-      r[c] = 1.0 / dn;
-      acc[c] += (zn * zn * ddn - 2.0 * zn * zdn * dn) * r[c] * r[c];
-      dd[c] = ddn; z[c] = zn; zd[c] = zdn;
-    }
-  }
-  outA = ok[0] ? (acc[0] <= D2 ? 0 : 1) : 2;
-  outB = ok[1] ? (acc[1] <= D2 ? 0 : 1) : 2;
-}
-// lane i: component i of -(T + lam I)^-1 b, b[0..n) in shared memory; the pivots must be positive
-__device__ __forceinline__ double tri_solve_dist(const double* A, const double* b, int n, double lam, int lane) {
-  double myr = 0.0, myz = 0.0, r = 0.0, z = 0.0;
-  for (int i = 0; i < n; ++i) {
-    const double bi = b[i];
-    if (i == 0) { r = 1.0 / (A[0] + lam); z = bi; }
-    else { const double e = A[i * n + i - 1], er = e * r; r = 1.0 / (A[i * n + i] + lam - e * er); z = bi - er * z; }
-    if (lane == i) { myr = r; myz = z; }
-  }
-  const double te = (lane + 1 < n) ? A[(lane + 1) * n + lane] : 0.0;
-  double hv = 0.0;
-  for (int i = n - 1; i >= 0; --i) {
-    const double hn = __shfl_sync(FULL, hv, (i + 1) & 31);
-    if (lane == i) hv = (myz - ((i + 1 < n) ? te * hn : 0.0)) * myr;
-  }
-  return -hv;
-}
-// A: n x n scratch; yv: n-vector scratch (shared memory, per slot)
-__device__ __noinline__ bool tr_step_warp(const double* H, const double* g, const int* fr, int n, int d, double Delta, double* A, double* yv) {
-  const int lane = threadIdx.x & 31;
-  const bool in = lane < n;
-  const int myc = in ? fr[lane] : 0;
-  const double gF = in ? g[myc] : 0.0;
-  if (n == 1) {
-    const double hh = H[fr[0] * d + fr[0]], g0 = g[fr[0]];
-    const bool inside = hh > 0.0 && fabs(g0 / hh) <= Delta;
-    __syncwarp();
-    if (lane == 0) yv[0] = inside ? -g0 / hh : (g0 > 0.0 ? -Delta : Delta);
-    __syncwarp();
-    return !inside;
-  }
-  for (int e = lane; e < n * n; e += 32) { const int i = e / n, j = e - i * n; A[e] = H[fr[i] * d + fr[j]]; }
-  if (in) yv[lane] = gF;
-  double gn = 0.0;
-  for (int i = 0; i < n; ++i) { const double t = g[fr[i]]; gn = fma(t, t, gn); }
-  gn = sqrt(gn);
-  __syncwarp();
-  // ---- Householder tridiagonalisation H_FF = Q T Q' with y <- Q'y fused in. Every lane evaluates the short dot products
-  // itself from shared memory (cheaper than FP64 shuffle reductions at these sizes). After step k: column k below the
-  // sub-diagonal keeps v_k (rows k+2..), A[k][k+1] its first component and A[k][k+2] beta_k.
-  for (int k = 0; k + 2 < n; ++k) {
-    double xa = 0.0, xb = 0.0;
-    for (int i = k + 1; i + 1 < n; i += 2) { const double u0 = A[i * n + k], u1 = A[(i + 1) * n + k]; xa = fma(u0, u0, xa); xb = fma(u1, u1, xb); }
-    if (((n - k - 1) & 1) != 0) { const double u0 = A[(n - 1) * n + k]; xa = fma(u0, u0, xa); }
-    const double xn2 = xa + xb, x0 = A[(k + 1) * n + k];
-    const double alpha = (x0 > 0.0 ? -1.0 : 1.0) * sqrt(xn2);
-    const double vtv = xn2 - 2.0 * alpha * x0 + alpha * alpha;
-    if (!(vtv > 0.0) || !(xn2 - x0 * x0 > 0.0)) {  // column already reduced (uniform)
-      __syncwarp();
-      if (lane == 0) { A[k * n + k + 2] = 0.0; }
-      __syncwarp();
-      continue;
-    }
-    const double bk = 2.0 / vtv, v1 = x0 - alpha;
-    const bool mine = lane > k && in;
-    const double vi = (lane == k + 1) ? v1 : (mine ? A[lane * n + k] : 0.0);
-    double t = 0.0;
-    if (mine) {
-      t = A[lane * n + k + 1] * v1;
-      for (int j = k + 2; j < n; ++j) t = fma(A[lane * n + j], A[j * n + k], t);
-    }
-    const double pw = bk * t;
-    if (mine) A[k * n + lane] = pw;  // row k beyond the diagonal is free: scratch for p
-    __syncwarp();
-    double pv = A[k * n + k + 1] * v1, vy = v1 * yv[k + 1];
-    for (int j = k + 2; j < n; ++j) { const double vj = A[j * n + k]; pv = fma(A[k * n + j], vj, pv); vy = fma(vj, yv[j], vy); }
-    const double kk = 0.5 * bk * pv, wi = pw - kk * vi;
-    __syncwarp();
-    if (mine) {
-      yv[lane] -= bk * vy * vi;
-      A[lane * n + k + 1] -= vi * (A[k * n + k + 1] - kk * v1) + wi * v1;
-      for (int j = k + 2; j < n; ++j) { const double vj = A[j * n + k]; A[lane * n + j] -= vi * (A[k * n + j] - kk * vj) + wi * vj; }
-    }
-    __syncwarp();
-    if (lane == k + 1) A[lane * n + k] = alpha;                                 // sub-diagonal of T
-    if (lane == k) { A[k * n + k + 1] = v1; A[k * n + k + 2] = bk; }            // first component of v_k, beta_k
-    __syncwarp();
-  }
-  double glo = INFINITY;
-  if (in) glo = A[lane * n + lane] - (lane > 0 ? fabs(A[lane * n + lane - 1]) : 0.0) - (lane + 1 < n ? fabs(A[(lane + 1) * n + lane]) : 0.0);
-  glo = warp_min(glo);  // Gershgorin lower bound of lambda_min(T)
-  const double D2 = Delta * Delta;
-  double lo = 0.0, hi = fmax(0.0, -glo) + gn / Delta;
-  bool hit = true, lo_notpd = false;
-  for (int round = 0; round < RBO_TR_ROUNDS; ++round) {
-    // 64 candidates per round, two per lane (c = lane, lane + 32); the last one is hi, known to be admissible
-    const double base = lo, wd = hi - lo;
-    const double lamA = (round == 0) ? wd * (double)lane / 63.0 : base + wd * (double)(lane + 1) / 64.0;
-    const double lamB = (round == 0) ? wd * (double)(lane + 32) / 63.0 : base + wd * (double)(lane + 33) / 64.0;
-    int oa, ob;
-    tri_probe2(A, yv, n, lamA, lamB, D2, oa, ob);
-    const unsigned long long adm = ((unsigned long long)__ballot_sync(FULL, ob == 0) << 32) | __ballot_sync(FULL, oa == 0) | (1ull << 63);
-    const unsigned long long pdm = ((unsigned long long)__ballot_sync(FULL, ob != 2) << 32) | __ballot_sync(FULL, oa != 2);
-    const int cf = __ffsll((long long)adm) - 1;
-    if (round == 0) {
-      if (cf == 0) { hi = 0.0; hit = false; break; }
-      lo_notpd = ((pdm >> (cf - 1)) & 1ull) == 0ull;
-      hi = (cf == 63) ? hi : wd * (double)cf / 63.0;
-      lo = wd * (double)(cf - 1) / 63.0;
-    } else {
-      if (cf > 0) lo_notpd = ((pdm >> (cf - 1)) & 1ull) == 0ull;
-      hi = (cf == 63) ? hi : base + wd * (double)(cf + 1) / 64.0;
-      lo = (cf == 0) ? base : base + wd * (double)cf / 64.0;
-    }
-  }
-  double h = tri_solve_dist(A, yv, n, hi, lane);
-  if (hit && lo_notpd) {
-    const double hn2 = warp_sum(in ? h * h : 0.0);
-    if (hn2 < D2) {  // hard case (to the resolution of the search): complete along the lowest eigenvector of T
-      __syncwarp();
-      if (in) yv[lane] = 1.0;
-      __syncwarp();
-      double z = 0.0;
-      for (int itn = 0; itn < 2; ++itn) {
-        const double z2 = tri_solve_dist(A, yv, n, hi, lane);
-        const double zn = 1.0 / sqrt(warp_sum(in ? z2 * z2 : 0.0));
-        z = in ? z2 * zn : 0.0;
-        __syncwarp();
-        if (in) yv[lane] = z;
-        __syncwarp();
-      }
-      const double hz = warp_sum(in ? h * z : 0.0);
-      const double tau = -hz + sqrt(fmax(hz * hz + (D2 - hn2), 0.0));
-      h += tau * z;
-    }
-  }
-  // ---- p = Q h: reflectors in descending order
-  __syncwarp();
-  if (in) yv[lane] = h;
-  __syncwarp();
-  for (int k = n - 3; k >= 0; --k) {
-    const double bk = A[k * n + k + 2], v1 = A[k * n + k + 1];
-    if (bk == 0.0) continue;
-    double dot = v1 * yv[k + 1];
-    for (int j = k + 2; j < n; ++j) dot = fma(A[j * n + k], yv[j], dot);
-    const double vi = (lane == k + 1) ? v1 : ((lane > k + 1 && in) ? A[lane * n + k] : 0.0);
-    __syncwarp();
-    if (lane > k && in) yv[lane] -= bk * dot * vi;
-    __syncwarp();
-  }
-  return hit;
-}
-
-
 struct K {
   const DevProblem& P;
   const SmemPlan& pl;
@@ -754,8 +307,6 @@ struct K {
     return j < P.N8 ? (P.xsm ? Xs[p * P.XP + j] : __ldg(P.Xb + (size_t)p * P.N8 + j)) : Xf[(j - P.N8) * P.d + p];
   }
   __device__ __forceinline__ bool row_active(int j) const { return j < P.N || (j >= P.N8 && j < P.N8 + nf); }
-  __device__ __forceinline__ int nact_rows() const { return P.N + nf; }
-  __device__ __forceinline__ int act_row(int a) const { return a < P.N ? a : P.N8 + (a - P.N); }
 
   // (p, q) table of the upper triangle of size d, packed p | q << 8
   __device__ void build_tables() {
@@ -1133,10 +684,6 @@ RBO_ROW_UNROLL
     const int nbatch = (ngroups + GPB - 1) / GPB;
     const unsigned chunks_per_pass = (unsigned)(nb * (nb + 1) / 2);
     const int ncons = min(ngroups, GPB) * NRQ;  // consumer warps of this pass: warps 0 .. ncons-1
-    AUX_T(ts0_);
-    AUX_ADD(0, ts0_);
-#ifdef RBO_PHASE_TIMERS
-#endif
     if (warp == RBO_NCONS) {
       // ---------------- producer warp ----------------
       if (lane == 0) {
@@ -1172,7 +719,6 @@ RBO_ROW_UNROLL
       double* fv = V + cB;
       const int fp = tg;
 
-      AUX_T(tf0_);
       if (!FWD && nfan > 0 && wact) {
         if (rq == 0) {
           // w_bot = Ginv^T t restricted to the active rows: w_r = sum_kk Ginv[kk][r] t[kk], Ginv[kk][r] = Fp[(N8 + r)*8 + kk]
@@ -1202,8 +748,6 @@ RBO_ROW_UNROLL
         group_sync(NRQ, gl);
       }
 
-      AUX_ADD(1, tf0_);
-      AUX_T(tc0_);
       double c[MTW][2];
 #pragma unroll
       for (int mt = 0; mt < MTW; ++mt) { c[mt][0] = 0.0; c[mt][1] = 0.0; }
@@ -1221,7 +765,6 @@ RBO_ROW_UNROLL
           if (tid == 0) atomicAdd(&g_phase_cycles[FWD ? 12 : 13], (unsigned long long)(clock64() - tw0));
 #endif
           const double* buf = stage + (size_t)(q % RBO_NSTAGE) * RBO_CHUNK_K * RBO_LP + rofs;
-          AUX_T(tm0_);
           if (wact) {
             const int nt = (N8 - rb - rofs + 7) >> 3;  // row tiles of this warp that lie below N8 (<= 0: none)
             if (cc < nc - 1) {
@@ -1230,7 +773,6 @@ RBO_ROW_UNROLL
             } else {
               // last chunk of the panel = diagonal block of the inverse applied to the panel's own right-hand-side rows
               mma_chunk<MTW>(buf, V + (size_t)rb * RP, cB, g, tg, c, nt);
-              AUX_T(td0_);
               group_sync(NRQ, gl);  // every warp of the group has read the right-hand-side rows
 #pragma unroll
               for (int mt = 0; mt < MTW; ++mt) {
@@ -1242,16 +784,13 @@ RBO_ROW_UNROLL
                 c[mt][0] = 0.0; c[mt][1] = 0.0;
               }
               asm volatile("" ::: "memory");  // keeps the stores of this panel ahead of the next panel's loads in program order (and the register allocation compact)
-              AUX_ADD(4, td0_);
             }
           }
           __syncwarp();
-          AUX_ADD(3, tm0_);
           if (lane == 0) empty_arrive(q);
         }
       }
 
-      AUX_ADD(2, tc0_);
       // the fantasy-row product below reads ALL top rows of the group's columns: the other warps of the group must have stored
       // their rows of the last block row first
       if (FWD && nfan > 0 && wact && NRQ > 1) group_sync(NRQ, gl);
@@ -1298,14 +837,12 @@ RBO_ROW_UNROLL
     double* dmu = sm + pl.sdmu + sl * d; double* dsig = sm + pl.sdsig + sl * d; double* ga = sm + pl.sga + sl * d;
     double* Ht = sm + pl.sHt + sl * dd; double* gh = sm + pl.sgh + sl * 8;
     auto pre = [&](int e) {
-      double s = 0.0;
-      if (RSpre < 0) { for (int r = 0; r < RS1; ++r) s += p1[(size_t)r * nout1 + e * (-RSpre) + q1]; }  // V_e . u from the fused product
-      else for (int r = 0; r < RSpre; ++r) s += ppre[(size_t)r * nout_pre + aidx * q1 + e];
-      return s;
+      if (RSpre < 0) return split_sum(p1, RS1, nout1, e * (-RSpre) + q1);  // V_e . u from the fused product
+      return split_sum(ppre, RSpre, nout_pre, aidx * q1 + e);
     };
-    auto one = [&](int e) { double s = 0.0; for (int r = 0; r < RS1; ++r) s += p1[(size_t)r * nout1 + e]; return s; };
-    auto gramf = [&](int p, int q) { double s = 0.0; for (int r = 0; r < RSg; ++r) s += pg[(size_t)r * noutg + goff + p * gld + q]; return s; };
-    auto hes = [&](int which, int e) { double s = 0.0; const int RS = which ? RShw : RShc; for (int r = 0; r < RS; ++r) s += phess[((size_t)(r * np + aidx) * 2 + which) * (T2 + 1) + e]; return s; };
+    auto one = [&](int e) { return split_sum(p1, RS1, nout1, e); };
+    auto gramf = [&](int p, int q) { return split_sum(pg, RSg, noutg, goff + p * gld + q); };
+    auto hes = [&](int which, int e) { return split_sum(phess, which ? RShw : RShc, np * 2 * (T2 + 1), (aidx * 2 + which) * (T2 + 1) + e); };
     const double mu = pre(0);
     const double var = P.k0 - one(0);  // rbs.jl:528 (kx.w == |L^-1 kx|^2)
     const double sigma = sqrt(var), isg = 1.0 / sigma;
@@ -1336,25 +873,6 @@ RBO_ROW_UNROLL
       gh[7] = fin ? 1.0 : 0.0;
     }
     __syncwarp();
-  }
-
-  // Cholesky of the n x n row-major matrix A (n <= 32) by one warp; lane i owns row i; the diagonal of the result holds
-  // 1 / l_jj. Returns false if not PD.
-  __device__ bool chol_warp(double* A, int n) const {
-    for (int j = 0; j < n; ++j) {
-      double t = 0.0;
-      if (lane >= j && lane < n) {
-        t = A[lane * n + j];
-        for (int k = 0; k < j; ++k) t = fma(-A[lane * n + k], A[j * n + k], t);
-      }
-      const double tj = __shfl_sync(FULL, t, j);
-      if (!(tj > 0.0) || !isfinite(tj)) return false;
-      const double inv = rsqrt(tj);  // the diagonal stores 1 / l_jj: the substitutions multiply instead of dividing
-      if (lane == j) A[j * n + j] = inv;
-      else if (lane > j && lane < n) A[lane * n + j] = t * inv;
-      __syncwarp();
-    }
-    return true;
   }
 
   // ------------------------------------------------------------------------------------------------
@@ -1658,6 +1176,116 @@ RBO_ROW_UNROLL
     }
     __syncthreads();
   }
+
+  // ================================================================================================
+  // Phases of one trajectory m, each called from exactly one place in the kernel. The joint draw + condition! and the adjoint
+  // stay in the kernel body: as member functions they moved ptxas's spills into the multistart loop (268 B of spill stores
+  // instead of 104 in the shared-memory build).
+  // ================================================================================================
+  // Sample index (normals, dual directions, forced locations, nodes) and starting point of trajectory m: recomputed at the few
+  // places they are needed instead of being kept live across the whole trajectory.
+  __device__ __forceinline__ int sample(int m) const { return m % P.Ms; }
+  __device__ __forceinline__ int start_point(int m) const { return m / P.Ms; }
+
+  // trajectory init: reset!(fs) (rbs.jl:476-480)
+  __device__ __forceinline__ void begin_trajectory() {
+    const int N8 = P.N8, NR = P.NR, RP = P.RP;
+    for (int i = tid; i < (N8 + RBO_MAXFAN) * 8; i += RBO_THREADS) Fp[i] = 0.0;
+    for (int i = tid; i < 64; i += RBO_THREADS) G[i] = ((i >> 3) == (i & 7)) ? 1.0 : 0.0;
+    for (int i = tid; i < NR; i += RBO_THREADS) { double c = (i < N8) ? __ldg(P.c0 + i) : 0.0; cst[i] = c; V[(size_t)i * RP + CCOL] = c; }
+    for (int i = tid; i < NR; i += RBO_THREADS) { double u0 = (i < N8) ? __ldg(P.u0 + i) : 0.0; u[i] = u0; V[(size_t)i * RP + UCOL] = u0; }
+    __syncthreads();
+    if (tid < 8) Fp[(size_t)(N8 + tid) * 8 + tid] = 1.0;  // inverse of the identity fantasy block
+    if (tid == 0) { misc[1] = P.ymin_base; si[I_TSTATUS] = RBO_TRAJ_OK; }
+    nf = 0;
+    __syncthreads();
+  }
+
+  // Chooses the location x_step into bestx: x0 at step 0, else the policy solve (or the caller's x-path when teacher-forced),
+  // followed by the extended tape's single evaluation at the chosen point. Holds the one call of multistart().
+  __device__ __forceinline__ void choose_location(int m, int step) {
+    const int d = P.d, h = P.h;
+    const bool myopic = (P.flags & RBO_FLAG_MYOPIC_INTERNAL) != 0;
+    if (step == 0) {
+      if (tid < d) bestx[tid] = P.x0_batch ? __ldg(P.x0_batch + (size_t)start_point(m) * d + tid) : P.x0[tid];  // rollout.jl:46
+      __syncthreads();
+    } else {
+      for (int pass = 0; pass < 2; ++pass) {
+        const bool single = pass == 1;  // pass 1: the extended tape's evaluation at the chosen point
+        if (single && (myopic || !(P.flags & RBO_FLAG_TAPE_EX))) break;
+        if (!single && !myopic && (P.flags & RBO_FLAG_TEACHER_FORCED)) {
+          // teacher forcing: the caller's x-path, or (RBO_FLAG_REPLAY_TAPE) the x-path the previous rollout left on the device
+          if (tid < d) bestx[tid] = (P.flags & RBO_FLAG_REPLAY_TAPE) ? P.xs[((size_t)m * (h + 1) + step) * d + tid] : P.x_forced[((size_t)sample(m) * h + (step - 1)) * d + tid];
+          if (tid == 0) { si[I_EVALS] = 0; misc[0] = nan(""); }
+        } else {
+          // multistart_base_solve!(fs, xnext; fantasy_index = step-1) (rollout.jl:58-66, rbf_optim.jl:68-101) -- column CCOL holds
+          // cs[fantasy_index + 2] (1-based) = the coefficients after `step` fantasies -- or, myopic,
+          // multistart_base_solve!(::Surrogate, ...) (rbf_optim.jl:103-134): the base surrogate, no fantasies
+          if (single) __syncthreads();
+          multistart(single ? 0 : (myopic ? (size_t)m * P.S : ((size_t)m * h + (step - 1)) * P.S), single, !single && step == 1);
+        }
+        __syncthreads();
+        if (!single) {
+          if (!myopic && tid == 0) {
+            if (P.n_evals) P.n_evals[(size_t)m * h + step - 1] = si[I_EVALS];
+            if (P.alphas) P.alphas[(size_t)m * h + step - 1] = -misc[0];
+          }
+        } else {
+          // extended tape (SURVEY.md section 7.4): sx = fs(x_step, theta; fantasy_index = step - 1), the surrogate evaluation the
+          // policy solve of this step maximised (rbs.jl:482-581); slot 0 holds it after the single evaluation
+          const size_t o = (size_t)m * h + step - 1;
+          const double* gh = sm + pl.sgh;
+          if (tid == 0) { P.t_mu[o] = gh[6]; P.t_sigma[o] = gh[5]; if (P.alphas) P.alphas[o] = gh[0]; }
+          for (int i = tid; i < d; i += RBO_THREADS) { P.t_dmu[o * d + i] = (sm + pl.sdmu)[i]; P.t_dsigma[o * d + i] = (sm + pl.sdsig)[i]; }
+          for (int i = tid; i < d * d; i += RBO_THREADS) P.t_Halpha[o * d * d + i] = (sm + pl.sHref)[i];
+          __syncthreads();
+        }
+      }
+    }
+  }
+
+  // the result of the myopic solve (rbf_optim.jl:103-134): the maximiser and its value
+  __device__ __forceinline__ void store_myopic(int m) {
+    const int d = P.d;
+    if (tid < d) P.xs[(size_t)m * d + tid] = bestx[tid];
+    if (tid == 0) {
+      P.values[m] = -misc[0];
+      if (P.n_evals) P.n_evals[m] = si[I_EVALS];
+      if (P.status) P.status[m] = si[I_TSTATUS];
+      if (P.best_index) P.best_index[m] = si[I_BEST];
+      if (P.grad_case) P.grad_case[m] = 0;
+    }
+  }
+
+  // resolve (rollout.jl:108-111): the value, the index t of the best observation, the gradient case, and the trajectory's tape
+  __device__ __forceinline__ void resolve(int m) {
+    const int d = P.d, h = P.h;
+    if (tid == 0) {
+      double best = yf[0];
+      int t = 0;
+      for (int j = 1; j <= h; ++j) if (yf[j] < best) { best = yf[j]; t = j; }  // findmin: first minimum (rollout.jl:77-82)
+      double val = fmax(P.fmini - best, 0.0);
+      if (P.flags & RBO_FLAG_GAUSS_HERMITE) {
+        // resolve(gho; fmini) (observables.jl:66-72); get_gradient(gho; at) = weights[at] * gradients[:, at] (observables.jl:157)
+        const double* wq = P.gh_weights + (size_t)sample(m) * P.gh_depth;
+        val = __ldg(wq + t) * val / 1.7724538509055159;
+        for (int j = 0; j <= h; ++j)
+          for (int a = 0; a < d; ++a) gyf[j * d + a] *= __ldg(wq + j);
+      }
+      P.values[m] = val;
+      si[I_T] = t;
+      int tc = 0;
+      if (P.mode == RBO_MODE_VALUE_GRAD) tc = (P.fmini <= best) ? 1 : (t == 0 ? 2 : 3);  // rollout.jl:241-251
+      si[I_CASE] = tc;
+      if (P.best_index) P.best_index[m] = t;
+      if (P.grad_case) P.grad_case[m] = tc;
+    }
+    __syncthreads();
+    if (P.xs) for (int i = tid; i < (h + 1) * d; i += RBO_THREADS) P.xs[(size_t)m * (h + 1) * d + i] = Xf[i];
+    if (P.gys) for (int i = tid; i < (h + 1) * d; i += RBO_THREADS) P.gys[(size_t)m * (h + 1) * d + i] = gyf[i];
+    if (P.ys) for (int i = tid; i <= h; i += RBO_THREADS) P.ys[(size_t)m * (h + 1) + i] = yf[i];
+    __syncthreads();
+  }
 };
 
 }  // namespace
@@ -1688,72 +1316,16 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
     __syncthreads();
     const int m = si[I_M];
     if (m >= P.M) break;
-    // sample index (normals, dual directions, forced locations, nodes) and starting point of trajectory m: recomputed at the
-    // few places they are needed instead of being kept live across the whole trajectory
-#define RBO_MS (m % P.Ms)
-#define RBO_MB (m / P.Ms)
 
-    // ---- trajectory init: reset!(fs) (rbs.jl:476-480) ----
-    for (int i = tid; i < (N8 + RBO_MAXFAN) * 8; i += RBO_THREADS) k.Fp[i] = 0.0;
-    for (int i = tid; i < 64; i += RBO_THREADS) k.G[i] = ((i >> 3) == (i & 7)) ? 1.0 : 0.0;
-    for (int i = tid; i < NR; i += RBO_THREADS) { double c = (i < N8) ? __ldg(P.c0 + i) : 0.0; k.cst[i] = c; k.V[(size_t)i * RP + k.CCOL] = c; }
-    for (int i = tid; i < NR; i += RBO_THREADS) { double u0 = (i < N8) ? __ldg(P.u0 + i) : 0.0; k.u[i] = u0; k.V[(size_t)i * RP + k.UCOL] = u0; }
-    __syncthreads();
-    if (tid < 8) k.Fp[(size_t)(N8 + tid) * 8 + tid] = 1.0;  // inverse of the identity fantasy block
-    if (tid == 0) { misc[1] = P.ymin_base; si[I_TSTATUS] = RBO_TRAJ_OK; }
-    k.nf = 0;
-    __syncthreads();
-
-    // multistart() is inlined at exactly ONE call site (a second or third copy pushes the kernel over its register budget):
-    // the myopic solve, the policy solves of the rollout and the single evaluation of the extended tape all go through it.
+    k.begin_trajectory();
+    // multistart() is inlined at exactly ONE call site, in choose_location() (a second or third copy pushes the kernel over its
+    // register budget): the myopic solve, the policy solves of the rollout and the single evaluation of the extended tape all go
+    // through it.
     const bool myopic = (P.flags & RBO_FLAG_MYOPIC_INTERNAL) != 0;
     for (int step = myopic ? 1 : 0; step <= (myopic ? 1 : h); ++step) {
-      // ============ choose the location x_step ============
-      if (step == 0) {
-        if (tid < d) bestx[tid] = P.x0_batch ? __ldg(P.x0_batch + (size_t)RBO_MB * d + tid) : P.x0[tid];  // rollout.jl:46
-        __syncthreads();
-      } else {
-        for (int pass = 0; pass < 2; ++pass) {
-          const bool single = pass == 1;  // pass 1: the extended tape's evaluation at the chosen point
-          if (single && (myopic || !(P.flags & RBO_FLAG_TAPE_EX))) break;
-          if (!single && !myopic && (P.flags & RBO_FLAG_TEACHER_FORCED)) {
-            // teacher forcing: the caller's x-path, or (RBO_FLAG_REPLAY_TAPE) the x-path the previous rollout left on the device
-            if (tid < d) bestx[tid] = (P.flags & RBO_FLAG_REPLAY_TAPE) ? P.xs[((size_t)m * (h + 1) + step) * d + tid] : P.x_forced[((size_t)RBO_MS * h + (step - 1)) * d + tid];
-            if (tid == 0) { si[I_EVALS] = 0; misc[0] = nan(""); }
-          } else {
-            // multistart_base_solve!(fs, xnext; fantasy_index = step-1) (rollout.jl:58-66, rbf_optim.jl:68-101) -- column CCOL holds
-            // cs[fantasy_index + 2] (1-based) = the coefficients after `step` fantasies -- or, myopic,
-            // multistart_base_solve!(::Surrogate, ...) (rbf_optim.jl:103-134): the base surrogate, no fantasies
-            if (single) __syncthreads();
-            k.multistart(single ? 0 : (myopic ? (size_t)m * P.S : ((size_t)m * h + (step - 1)) * P.S), single, !single && step == 1);
-          }
-          __syncthreads();
-          if (!single) {
-            if (!myopic && tid == 0) {
-              if (P.n_evals) P.n_evals[(size_t)m * h + step - 1] = si[I_EVALS];
-              if (P.alphas) P.alphas[(size_t)m * h + step - 1] = -misc[0];
-            }
-          } else {
-            // extended tape (SURVEY.md section 7.4): sx = fs(x_step, theta; fantasy_index = step - 1), the surrogate evaluation the
-            // policy solve of this step maximised (rbs.jl:482-581); slot 0 holds it after the single evaluation
-            const size_t o = (size_t)m * h + step - 1;
-            const double* gh = smem + k.pl.sgh;
-            if (tid == 0) { P.t_mu[o] = gh[6]; P.t_sigma[o] = gh[5]; if (P.alphas) P.alphas[o] = gh[0]; }
-            for (int i = tid; i < d; i += RBO_THREADS) { P.t_dmu[o * d + i] = (smem + k.pl.sdmu)[i]; P.t_dsigma[o * d + i] = (smem + k.pl.sdsig)[i]; }
-            for (int i = tid; i < d * d; i += RBO_THREADS) P.t_Halpha[o * d * d + i] = (smem + k.pl.sHref)[i];
-            __syncthreads();
-          }
-        }
-      }
+      k.choose_location(m, step);
       if (myopic) {
-        if (tid < d) P.xs[(size_t)m * d + tid] = bestx[tid];
-        if (tid == 0) {
-          P.values[m] = -misc[0];
-          if (P.n_evals) P.n_evals[m] = si[I_EVALS];
-          if (P.status) P.status[m] = si[I_TSTATUS];
-          if (P.best_index) P.best_index[m] = si[I_BEST];
-          if (P.grad_case) P.grad_case[m] = 0;
-        }
+        k.store_myopic(m);
         break;
       }
 
@@ -1781,8 +1353,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
         // Sigma = Dk(0) - A K^-1 A' = Dk(0) - V'V (rbs.jl:531-536)
         double* Sg = misc + 8;  // (d+1) x (d+1)
         for (int e = tid; e < nsg; e += RBO_THREADS) {
-          double acc = 0.0;
-          for (int r = 0; r < RSpost; ++r) acc += (smem + k.pl.ppost)[(size_t)r * nsg + e];
+          const double acc = split_sum(smem + k.pl.ppost, RSpost, nsg, e);
           if (e < q1 * q1) {
             const int p = e / q1, q = e - p * q1;
             const double dk = (p == q) ? (p == 0 ? P.k0 : -P.d2k0) : 0.0;  // eval_Dk(kernel, 0) rbf.jl:152-159
@@ -1791,11 +1362,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
             if (e == 0) misc[4] = acc;  // |l|^2
           } else misc[5] = acc;         // l . u
         }
-        if (tid < q1) {
-          double acc = 0.0;
-          for (int r = 0; r < RSpre; ++r) acc += (smem + k.pl.ppre)[(size_t)r * q1 + tid];
-          misc[8 + q1 * q1 + tid] = acc;  // [mu, grad mu]
-        }
+        if (tid < q1) misc[8 + q1 * q1 + tid] = split_sum(smem + k.pl.ppre, RSpre, q1, tid);  // [mu, grad mu]
         __syncthreads();
         if (tid == 0) {
           const int r = k.nf;  // index of the new fantasy row
@@ -1806,13 +1373,13 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
             const double* raw = misc + 8 + q1 * q1 + q1;
             const double var = P.k0 - raw[0];  // rbs.jl:528
             if (!(var >= 0.0) && si[I_TSTATUS] == RBO_TRAJ_OK) si[I_TSTATUS] = RBO_TRAJ_NEG_VARIANCE;
-            const double sigma = sqrt(var), node = __ldg(P.gh_nodes + (size_t)RBO_MS * P.gh_depth + step), s2n = 1.4142135623730951 * node;
+            const double sigma = sqrt(var), node = __ldg(P.gh_nodes + (size_t)k.sample(m) * P.gh_depth + step), s2n = 1.4142135623730951 * node;
             yv = dmu[0] + s2n * sigma;
             for (int a = 0; a < d; ++a) k.gyf[r * d + a] = dmu[1 + a] + s2n * (-raw[1 + a] / sigma);  // rbs.jl:529
           } else {
             bool pd = chol_inplace(Sg, q1, q1);
             if (!pd && si[I_TSTATUS] == RBO_TRAJ_OK) si[I_TSTATUS] = RBO_TRAJ_NOT_PD_JOINT;
-            const double* rnm = P.rn + (size_t)RBO_MS + (size_t)P.Ms * q1 * step;
+            const double* rnm = P.rn + (size_t)k.sample(m) + (size_t)P.Ms * q1 * step;
             yv = dmu[0] + Sg[0] * __ldg(rnm);
             for (int a = 0; a < d; ++a) {
               double v = dmu[1 + a];
@@ -1861,33 +1428,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
     }
 
     if (myopic) continue;
-    // ============ resolve (rollout.jl:108-111) and bookkeeping ============
-    if (tid == 0) {
-      double best = k.yf[0];
-      int t = 0;
-      for (int j = 1; j <= h; ++j) if (k.yf[j] < best) { best = k.yf[j]; t = j; }  // findmin: first minimum (rollout.jl:77-82)
-      double val = fmax(P.fmini - best, 0.0);
-      if (P.flags & RBO_FLAG_GAUSS_HERMITE) {
-        // resolve(gho; fmini) (observables.jl:66-72); get_gradient(gho; at) = weights[at] * gradients[:, at] (observables.jl:157)
-        const double* wq = P.gh_weights + (size_t)RBO_MS * P.gh_depth;
-        val = __ldg(wq + t) * val / 1.7724538509055159;
-        for (int j = 0; j <= h; ++j)
-          for (int a = 0; a < d; ++a) k.gyf[j * d + a] *= __ldg(wq + j);
-      }
-      P.values[m] = val;
-      si[I_T] = t;
-      int tc = 0;
-      if (P.mode == RBO_MODE_VALUE_GRAD) tc = (P.fmini <= best) ? 1 : (t == 0 ? 2 : 3);  // rollout.jl:241-251
-      si[I_CASE] = tc;
-      if (P.best_index) P.best_index[m] = t;
-      if (P.grad_case) P.grad_case[m] = tc;
-    }
-    __syncthreads();
-    if (P.xs) for (int i = tid; i < (h + 1) * d; i += RBO_THREADS) P.xs[(size_t)m * (h + 1) * d + i] = k.Xf[i];
-    if (P.gys) for (int i = tid; i < (h + 1) * d; i += RBO_THREADS) P.gys[(size_t)m * (h + 1) * d + i] = k.gyf[i];
-    if (P.ys) for (int i = tid; i <= h; i += RBO_THREADS) P.ys[(size_t)m * (h + 1) + i] = k.yf[i];
-    __syncthreads();
-
+    k.resolve(m);
     // ============ gradient(T) (rollout.jl:233-277) ============
     PT_DECL;
     if (P.mode == RBO_MODE_VALUE_GRAD) {
@@ -1905,7 +1446,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
         __syncthreads();
         if (tid == 0) ybars[t + 1] = 1.0;  // rollout.jl:256
         const int CB_RAW = 0, CB_SOL = d + 3, CB_U = 2 * d + 4, CB_Q = 3 * d + 5;
-        const double* dd_m = P.dual_dirs ? P.dual_dirs + (size_t)RBO_MS * h * d : nullptr;
+        const double* dd_m = P.dual_dirs ? P.dual_dirs + (size_t)k.sample(m) * h * d : nullptr;
         for (int i = t; i >= 1; --i) {
           // ---- re-evaluate policy solve i: fs(x_i, theta; fantasy_index = i-1) (rollout.jl:114-124) ----
           k.nf = i;
@@ -2008,8 +1549,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
             __syncthreads();
             double* uw = misc + 8;  // [q1]
             for (int e = tid; e < 2 * q1; e += RBO_THREADS) {
-              double acc = 0.0;
-              for (int r = 0; r < RSb; ++r) acc += (smem + k.pl.ppost)[(size_t)r * 2 * q1 + e];
+              const double acc = split_sum(smem + k.pl.ppost, RSb, 2 * q1, e);
               if (e >= q1) uw[e - q1] = acc; else k.V[(size_t)rowp * RP + CB_Q + e] = acc;
             }
             for (int q = tid; q < q1; q += RBO_THREADS) k.colidx[q] = CB_Q + q;
@@ -2030,7 +1570,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
               const int q = tid;
               const double* gh = smem + k.pl.sgh; const double* dmu = smem + k.pl.sdmu; const double* dsg = smem + k.pl.sdsig;
               const double* rowp_v = k.V + (size_t)rowp * RP;
-              auto dq = [&](int w) { double acc = 0.0; for (int r = 0; r < RSd; ++r) acc += (smem + k.pl.ppost)[(size_t)r * nD + w * q1 + q]; return acc; };
+              auto dq = [&](int w) { return split_sum(smem + k.pl.ppost, RSd, nD, w * q1 + q); };
               const double cp = rowp_v[k.CCOL], wp = rowp_v[CB_SOL];
               double dxv[RBO_MAXD];
               for (int a = 0; a < d; ++a) dxv[a] = (q < d) ? (a == q ? 1.0 : 0.0) : (dd_m ? dd_m[(size_t)p * d + a] : 0.0);
@@ -2077,11 +1617,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
           const int RSpre = k.choose_rs(K::nblk16(q1));
           k.colprod(1, q1, smem + k.pl.ppre, RSpre);
           __syncthreads();
-          for (int a = tid; a < d; a += RBO_THREADS) {
-            double dmu = 0.0;
-            for (int r = 0; r < RSpre; ++r) dmu += (smem + k.pl.ppre)[(size_t)r * q1 + 1 + a];
-            P.grad_x[(size_t)m * d + a] = -(dmu * ybars[1] + gxa[a]);
-          }
+          for (int a = tid; a < d; a += RBO_THREADS) P.grad_x[(size_t)m * d + a] = -(split_sum(smem + k.pl.ppre, RSpre, q1, 1 + a) * ybars[1] + gxa[a]);
           for (int a = tid; a < nth; a += RBO_THREADS) P.grad_theta[(size_t)m * nth + a] = (a == 0) ? -gtha[0] : 0.0;
         }
         k.nf = h + 1;
@@ -2094,198 +1630,6 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
   k.pipe_fini();
   if (tid == 0 && P.cta_done) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); P.cta_done[blockIdx.x] = t; }
 }
-
-#if !RBO_VGLOB
-// ----------------------------------------------------------------------------------------------------
-// gen_low_discrepancy_sequence (utils.jl:65-74) on the device: Sobol (utils.jl:4-13, Joe-Kuo direction numbers,
-// Gray-code order, origin skipped) -> Box-Muller with log10 and pair indexing (utils.jl:23-43, Q8) -> the
-// column-major reshape(N, M, D, H) and removal of the padding coordinate.
-// ----------------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned sobol_point(const unsigned* dirs, int dim, unsigned k) {
-  unsigned g = k ^ (k >> 1), x = 0;
-  const unsigned* v = dirs + dim * 32;
-  for (int b = 0; g != 0u; ++b, g >>= 1)
-    if (g & 1u) x ^= v[b];
-  return x;
-}
-
-__global__ void rbo_normals_kernel(const unsigned* __restrict__ dirs, double* __restrict__ out, int M_total, int d, int H, int m_begin, int m_count) {
-  const int q1 = d + 1, D = q1 + ((q1 & 1) ? 1 : 0);
-  const size_t total = (size_t)m_count * q1 * H;
-  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
-    int ml = (int)(idx % m_count);
-    int kq = (int)((idx / m_count) % q1);
-    int t = (int)(idx / ((size_t)m_count * q1));
-    size_t q = (size_t)(m_begin + ml) + (size_t)M_total * kq + (size_t)M_total * D * t;  // flat index into the D x (M*H) normals
-    int coord = (int)(q % D);
-    unsigned pnt = (unsigned)(q / D) + 1u;  // Sobol point index (the origin is skipped)
-    int c0 = coord & ~1;                    // pair (c0, c0+1)
-    double u1 = (double)sobol_point(dirs, c0, pnt) * (1.0 / 4294967296.0);
-    double u2 = (double)sobol_point(dirs, c0 + 1, pnt) * (1.0 / 4294967296.0);
-    double rad = sqrt(-2.0 * log10(u1));
-    const double two_pi = 6.283185307179586;
-    out[idx] = (coord & 1) ? rad * sin(two_pi * u2) : rad * cos(two_pi * u2);
-  }
-}
-
-__global__ void rbo_sobol_kernel(const unsigned* __restrict__ dirs, unsigned* __restrict__ out_u32, double* __restrict__ out_f64, int dim, int npoints,
-                                 const double* __restrict__ lbs, const double* __restrict__ ubs) {
-  const size_t total = (size_t)dim * npoints;
-  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
-    int a = (int)(idx % dim);
-    unsigned pnt = (unsigned)(idx / dim) + 1u;
-    unsigned x = sobol_point(dirs, a, pnt);
-    if (out_u32) out_u32[idx] = x;
-    if (out_f64) {
-      double uu = (double)x * (1.0 / 4294967296.0);
-      out_f64[idx] = lbs ? lbs[a] + (ubs[a] - lbs[a]) * uu : uu;
-    }
-  }
-}
-
-// Per-handle statistics of the last rollout: sums[0] = n, then [n*mean, M2, n*mean^2] for the value and every gradient
-// row (two-pass: mean first, then centred squares -- rollout.jl:328-337), then the acquisition evaluations per step
-// (max(h,1) entries), then a histogram over t = 0..h of the case-3 trajectories, then the number of failed trajectories.
-// One CTA; M is at most a few 10^5.
-__global__ void rbo_stats_kernel(const double* __restrict__ values, const double* __restrict__ gx, const double* __restrict__ gth,
-                                 const int* __restrict__ n_evals, const int* __restrict__ best_index, const int* __restrict__ grad_case,
-                                 const int* __restrict__ status, int M, int d, int nth, int h, double* __restrict__ sums) {
-  __shared__ double red[32];
-  __shared__ double s_mean;
-  const int nrows = 1 + d + nth, nw = blockDim.x >> 5;
-  auto block_sum = [&](double acc) -> double {
-    for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    double tot = 0.0;
-    for (int w = 0; w < nw; ++w) tot += red[w];
-    return tot;
-  };
-  // trajectories that failed (status != 0: the reference would have thrown, SURVEY.md section 5) are excluded from n and from
-  // every sum -- a half-factorised joint covariance yields finite garbage that must not leak into the estimate; their count is
-  // reported next to the sums and travels through the same all-reduce (rbo_partial_sums_device)
-  auto okay = [&](int i) { return !status || status[i] == 0; };
-  double nok_acc = 0.0;
-  for (int i = threadIdx.x; i < M; i += blockDim.x) nok_acc += okay(i) ? 1.0 : 0.0;
-  const double nok = block_sum(nok_acc);
-  for (int row = 0; row < nrows; ++row) {
-    const double* base; int stride;
-    if (row == 0) { base = values; stride = 1; }
-    else if (row <= d) { base = gx ? gx + (row - 1) : nullptr; stride = d; }
-    else { base = gth ? gth + (row - 1 - d) : nullptr; stride = nth; }
-    double mean = 0.0, m2 = 0.0;
-    if (base && nok > 0.0) {
-      double acc = 0.0;
-      for (int i = threadIdx.x; i < M; i += blockDim.x) if (okay(i)) acc += base[(size_t)i * stride];
-      mean = block_sum(acc) / nok;
-      if (threadIdx.x == 0) s_mean = mean;
-      __syncthreads();
-      mean = s_mean;
-      acc = 0.0;
-      for (int i = threadIdx.x; i < M; i += blockDim.x) if (okay(i)) { double v = base[(size_t)i * stride] - mean; acc += v * v; }
-      m2 = block_sum(acc);
-    }
-    if (threadIdx.x == 0) {
-      if (row == 0) sums[0] = nok;
-      sums[1 + 3 * row + 0] = nok * mean;
-      sums[1 + 3 * row + 1] = m2;
-      sums[1 + 3 * row + 2] = nok * mean * mean;
-    }
-  }
-  const int hh = h > 1 ? h : 1;
-  double* ev = sums + 1 + 3 * nrows;
-  for (int j = 0; j < hh; ++j) {
-    double acc = 0.0;
-    if (n_evals && h > 0) for (int i = threadIdx.x; i < M; i += blockDim.x) acc += n_evals[(size_t)i * h + j];
-    double tot = block_sum(acc);
-    if (threadIdx.x == 0) ev[j] = tot;
-  }
-  double* hist = ev + hh;
-  for (int t = 0; t <= h + 1; ++t) {
-    double acc = 0.0;
-    for (int i = threadIdx.x; i < M; i += blockDim.x) {
-      if (t <= h) acc += (grad_case && best_index && grad_case[i] == 3 && best_index[i] == t) ? 1.0 : 0.0;
-      else acc += (status && status[i] != 0) ? 1.0 : 0.0;
-    }
-    double tot = block_sum(acc);
-    if (threadIdx.x == 0) hist[t + (t > h ? 1 : 0)] = tot;
-  }
-}
-
-// Longest-processing-time order for the NEXT launch on the same samples (common random numbers: the outer ascent loop and the
-// bench re-evaluate the same trajectories at a nearby x0, so the evaluation counts of this launch predict the next one's costs):
-// counting sort of the trajectories by descending cost. One CTA; ties in arbitrary order (scheduling only).
-__global__ void rbo_lpt_order_kernel(const int* __restrict__ n_evals, const int* __restrict__ grad_case, const int* __restrict__ best_index, int M, int hh,
-                                     int* __restrict__ order) {
-  constexpr int NB = 2048;
-  __shared__ int hist[NB];
-  __shared__ int smax;
-  auto cost = [&](int m) {
-    int c = 1;
-    for (int j = 0; j < hh; ++j) c += n_evals[(size_t)m * hh + j];
-    if (grad_case[m] == 3) { const int t = best_index[m]; c += 2 * t * (t + 1); }  // the adjoint re-evaluates t policy solves with i perturbation solves each
-    return c;
-  };
-  if (threadIdx.x == 0) smax = 1;
-  for (int i = threadIdx.x; i < NB; i += blockDim.x) hist[i] = 0;
-  __syncthreads();
-  int mx = 1;
-  for (int m = threadIdx.x; m < M; m += blockDim.x) mx = max(mx, cost(m));
-  atomicMax(&smax, mx);
-  __syncthreads();
-  const double scale = (double)(NB - 1) / (double)smax;
-  for (int m = threadIdx.x; m < M; m += blockDim.x) atomicAdd(&hist[(int)(cost(m) * scale)], 1);
-  __syncthreads();
-  if (threadIdx.x == 0) {  // exclusive offsets in DESCENDING bucket order
-    int run = 0;
-    for (int b = NB - 1; b >= 0; --b) { const int c = hist[b]; hist[b] = run; run += c; }
-  }
-  __syncthreads();
-  for (int m = threadIdx.x; m < M; m += blockDim.x) order[atomicAdd(&hist[(int)(cost(m) * scale)], 1)] = m;
-}
-
-// out = [sums[0 .. need), number of failed trajectories, kernel watchdog flag]: the vector the multi-GPU all-reduce sums
-__global__ void rbo_gather_sums_kernel(const double* __restrict__ sums, int need, int idx_failed, const int* __restrict__ work_counter, double* __restrict__ out) {
-  for (int i = threadIdx.x; i < need; i += blockDim.x) out[i] = sums[i];
-  if (threadIdx.x == 0) { out[need] = sums[idx_failed]; out[need + 1] = (work_counter[1] || work_counter[2]) ? 1.0 : 0.0; }
-}
-
-// FP64 FMA micro-benchmark: the roofline denominator for this path (MEASURED_PEAKS.json has no FP64 figure).
-// Diagnostic (rbo_tr_step_batch): the device code of the per-start trust-region step on B independent subproblems, one warp each,
-// through the same dispatch as slot_logic_warp (registers for 2 <= n <= 16, shared memory otherwise). H: [B][n*n], g: [B][n],
-// p: [B][n], hit: [B].
-__global__ void rbo_tr_step_kernel(const double* H, const double* g, const double* Delta, int n, int B, double* p, int* hit) {
-  extern __shared__ __align__(16) double trs[];
-  const int lane = threadIdx.x & 31, wpb = blockDim.x >> 5, w = threadIdx.x >> 5, b = blockIdx.x * wpb + w;
-  if (b >= B) return;
-  double* base = trs + (size_t)w * (2 * n * n + 4 * n + 32);
-  double* Hs = base; double* A = Hs + n * n; double* gs = A + n * n; double* ta = gs + n; double* te = ta + n; double* yv = te + n;
-  int* fr = reinterpret_cast<int*>(yv + n);
-  for (int i = lane; i < n * n; i += 32) Hs[i] = H[(size_t)b * n * n + i];
-  if (lane < n) { gs[lane] = g[(size_t)b * n + lane]; fr[lane] = lane; }
-  __syncwarp();
-  const bool h_ = (n >= 2 && n <= 16) ? tr_step16(Hs, gs, fr, n, n, Delta[b], ta, te, yv) : tr_step_warp(Hs, gs, fr, n, n, Delta[b], A, yv);
-  if (lane < n) p[(size_t)b * n + lane] = yv[lane];
-  if (lane == 0) hit[b] = h_ ? 1 : 0;
-}
-
-__global__ void rbo_fp64_peak_kernel(double* out, int iters) {
-  double a[16];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) a[i] = 1.0 + 1e-9 * (threadIdx.x + i);
-  const double b = 1.0000001, c = 1e-9;
-  for (int it = 0; it < iters; ++it) {
-#pragma unroll
-    for (int i = 0; i < 16; ++i) a[i] = fma(a[i], b, c);
-  }
-  double s = 0.0;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) s += a[i];
-  out[(size_t)blockIdx.x * blockDim.x + threadIdx.x] = s;
-}
-
-#endif  // !RBO_VGLOB
 
 }  // namespace rbo
 
