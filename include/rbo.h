@@ -227,11 +227,37 @@ void rbo_default_sga_opts(rbo_sga_opts* o);
  * normals or starts; the plan limits of rbo_rollout (RBO_ERR_UNSUPPORTED); RBO_ERR_CUDA with the watchdog message if the rollout
  * kernel reported a stuck pipeline (every restart stops then). Afterwards the handle keeps its surrogate, normals and starts;
  * RBO_FLAG_REPLAY_TAPE and the per-trajectory read-backs are refused until the next rollout, because the last launch did not
- * run every restart. One GPU only: the per-iteration statistics of several would need an all-reduce inside the loop. */
+ * run every restart. Over several GPUs, or several handles that each hold a shard of the samples: rbo_stochastic_solve_batch_sharded. */
 int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
                                const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
                                double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail, double* x_hist,
                                double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist, rbo_summary* summary);
+/* rbo_stochastic_solve_batch over the samples of several handles, e.g. one per GPU. Each handle holds the same surrogate and starts and
+ * one shard [m_begin, m_begin + m_count) of the same M_total normals (rbo_set_normals / rbo_generate_normals); the shards tile
+ * [0, M_total), and the handles may sit on one device or several and come in any order. Per iteration every handle runs the rollouts
+ * of its shard on its own stream; hs[0], the leader, gathers every shard's per-trajectory results (peer copies, peer access enabled
+ * where the devices allow it), computes the statistics and the step over all M_total samples, and the other handles take the new
+ * iterates from it. The host enqueues every iteration and synchronises each handle once at the end.
+ * The statistics and the step run over the shards' results in global sample order, so the result equals, bit for bit,
+ * rbo_stochastic_solve_batch on one handle that holds all M_total samples, whatever the split and the devices, wherever the rollout
+ * kernel's per-trajectory results do not depend on the order it hands trajectories out: when every start has a start slot of its own
+ * (the plan's W >= the number of starts). With more starts than slots a CTA orders the starts by the evaluation counts of its previous
+ * trajectory and its row splits follow the number of active slots, so the last bits of a trajectory follow the CTA's history; two
+ * one-handle calls then differ as much as a split and a one-handle call do. The arguments mean what they mean there, except:
+ *   dual_dirs : d x h x M_total (every handle uploads its own samples' slice), or NULL = zeros
+ *   fail      : fail[0, b] is a global sample index
+ *   summary   : kernel_ms of the loop on the leader's stream, gpu_launches summed over handles, n_traj and n_failed over all samples
+ * Errors, returned before anything is enqueued and reported by rbo_last_error(hs[0]) (rbo_last_error(NULL) for n_handles < 1 or a
+ * NULL hs[0]); every handle is left as it was: RBO_ERR_ARG for n_handles < 1, a NULL or repeated handle, shards that do not tile
+ * [0, M_total), handles that disagree on d, N, the number of starts, hp1 or M_total; RBO_ERR_STATE (naming the handle) for a handle
+ * without surrogate, normals or starts; every error of rbo_stochastic_solve_batch. A watchdog flag on any handle stops every restart
+ * and returns RBO_ERR_CUDA with a message naming the handle (its index in hs). Afterwards every handle refuses RBO_FLAG_REPLAY_TAPE
+ * and the per-trajectory read-backs until its next rollout. With n_handles == 1 the call is rbo_stochastic_solve_batch. */
+int rbo_stochastic_solve_batch_sharded(rbo_handle* const* hs, int n_handles, const rbo_sga_opts* o, const double* x0s, int n_x0,
+                                       const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon, double fmini,
+                                       const double* dual_dirs, double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail,
+                                       double* x_hist, double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist,
+                                       rbo_summary* summary);
 
 /* Per-handle partial statistics of the last rollout, for the multi-GPU all-reduce:
  * sums = [n, n*mean_v, M2_v, n*mean_v^2, (n*mean, M2, n*mean^2) per grad_x row..., per grad_theta row..., n_failed, watchdog]

@@ -58,6 +58,8 @@ SYMBOLS = {
     "rbo_default_sga_opts": (None, [C.POINTER(SgaOpts)]),
     "rbo_stochastic_solve_batch": (C.c_int, [C.c_void_p, C.POINTER(SgaOpts), _dp, C.c_int, _dp, C.c_int, _dp, _dp, C.c_int, C.c_double, _dp,
                                              _dp, _ip, _ip, _ip, _dp, _dp, _dp, _dp, _dp, C.POINTER(Summary)]),
+    "rbo_stochastic_solve_batch_sharded": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(SgaOpts), _dp, C.c_int, _dp, C.c_int, _dp, _dp,
+                                                     C.c_int, C.c_double, _dp, _dp, _ip, _ip, _ip, _dp, _dp, _dp, _dp, _dp, C.POINTER(Summary)]),
     "rbo_partial_sums_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "rbo_partial_sums_host": (C.c_int, [C.c_void_p, _dp, C.c_int]),
     "rbo_get_results": (C.c_int, [C.c_void_p, _dp, _dp, _dp, _ip, _ip, _ip]),

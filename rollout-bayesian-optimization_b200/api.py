@@ -399,6 +399,7 @@ class RolloutEngine:
             self.handle.check(self.lib.rbo_set_stream(self.handle.h, C.c_void_p(stream)))
         self.d = None
         self.m_count = 0
+        self.m_begin, self.M_total = 0, 0  # the shard of the normals: samples [m_begin, m_begin + m_count) of M_total
 
     def close(self):
         self.handle.close()
@@ -457,12 +458,12 @@ class RolloutEngine:
         M = rn.shape[0]
         m_count = M - m_begin if m_count is None else m_count
         self.handle.check(self.lib.rbo_set_normals(self.handle.h, dptr(rn), M, rn.shape[2], m_begin, m_count))
-        self.m_count = m_count
+        self.m_count, self.m_begin, self.M_total = m_count, m_begin, M
 
     def generate_normals(self, M_total, hp1, m_begin=0, m_count=None):
         m_count = M_total - m_begin if m_count is None else m_count
         self.handle.check(self.lib.rbo_generate_normals(self.handle.h, M_total, hp1, m_begin, m_count))
-        self.m_count = m_count
+        self.m_count, self.m_begin, self.M_total = m_count, m_begin, M_total
 
     def get_normals(self, hp1):
         out = np.zeros((self.m_count, self.d + 1, hp1), order="F")
@@ -532,16 +533,10 @@ class RolloutEngine:
         (max_iterations x B), gmean_hist, gstd_hist (d x max_iterations x B; NaN past n_iter) and summary."""
         o = _sga_opts(Adam() if optimizer is None else optimizer, max_iterations, use_eswavs, project)
         x0s, theta, lbs, ubs, dual_dirs = _sga_arrays(x0s, theta, lbs, ubs, horizon, dual_dirs, self.d, self.m_count or None)
-        d, B, T = x0s.shape[0], x0s.shape[1], int(max_iterations)
-        r = dict(x_final=np.zeros((d, B), order="F"), n_iter=np.zeros(B, np.int32), end_status=np.zeros(B, np.int32),
-                 fail=np.zeros((2, B), np.int32, order="F"), x_hist=np.zeros((d, T, B), order="F"), mean_hist=np.zeros((T, B), order="F"),
-                 std_hist=np.zeros((T, B), order="F"), gmean_hist=np.zeros((d, T, B), order="F"), gstd_hist=np.zeros((d, T, B), order="F"))
-        s = Summary()
+        r, s = _sga_results(x0s.shape[0], x0s.shape[1], max_iterations)
         self.handle.check(self.lib.rbo_stochastic_solve_batch(
-            self.handle.h, C.byref(o), dptr(x0s), B, dptr(theta), len(theta), dptr(lbs), dptr(ubs), int(horizon), float(fmini), dptr(dual_dirs),
-            dptr(r["x_final"]), iptr(r["n_iter"]), iptr(r["end_status"]), iptr(r["fail"]), dptr(r["x_hist"]), dptr(r["mean_hist"]),
-            dptr(r["std_hist"]), dptr(r["gmean_hist"]), dptr(r["gstd_hist"]), C.byref(s)))
-        r["summary"] = s
+            self.handle.h, C.byref(o), dptr(x0s), x0s.shape[1], dptr(theta), len(theta), dptr(lbs), dptr(ubs), int(horizon), float(fmini),
+            dptr(dual_dirs), *_sga_result_ptrs(r), C.byref(s)))
         return r
 
     def tape(self, horizon, ntheta=1):
@@ -896,7 +891,60 @@ def _sga_arrays(x0s, theta, lbs, ubs, horizon, dual_dirs, d=None, M=None):
     return x0s, theta, lbs, ubs, dual_dirs
 
 
-def stochastic_solve_batch(optimizer, T, tp, es, starts, max_iterations=50, use_eswavs=True, dual_directions=None, device=0):
+def _sga_results(d, B, T):
+    """The result dict of stochastic_solve_batch (summary included) for d dimensions, B restarts and T iterations, and its Summary."""
+    s = Summary()
+    r = dict(x_final=np.zeros((d, B), order="F"), n_iter=np.zeros(B, np.int32), end_status=np.zeros(B, np.int32),
+             fail=np.zeros((2, B), np.int32, order="F"), x_hist=np.zeros((d, T, B), order="F"), mean_hist=np.zeros((T, B), order="F"),
+             std_hist=np.zeros((T, B), order="F"), gmean_hist=np.zeros((d, T, B), order="F"), gstd_hist=np.zeros((d, T, B), order="F"),
+             summary=s)
+    return r, s
+
+
+def _sga_result_ptrs(r):
+    return (dptr(r["x_final"]), iptr(r["n_iter"]), iptr(r["end_status"]), iptr(r["fail"]), dptr(r["x_hist"]), dptr(r["mean_hist"]),
+            dptr(r["std_hist"]), dptr(r["gmean_hist"]), dptr(r["gstd_hist"]))
+
+
+def _check_shards(engines):
+    """The engines' shards of the normals must tile [0, M_total) of one M_total (rbo_stochastic_solve_batch_sharded's own check, made
+    before any library call)."""
+    if len(engines) < 1:
+        raise ValueError("stochastic_solve_batch_sharded: no engine")
+    M_total = engines[0].M_total
+    shards = sorted((e.m_begin, e.m_count, e.M_total) for e in engines)
+    nxt = 0
+    for m_begin, m_count, M in shards:
+        if M != M_total or m_begin != nxt or m_count < 1:
+            raise ValueError(f"stochastic_solve_batch_sharded: the shards (m_begin, m_count, M_total) {shards} do not tile [0, M_total)")
+        nxt += m_count
+    if nxt != M_total or M_total < 1:
+        raise ValueError(f"stochastic_solve_batch_sharded: the shards (m_begin, m_count, M_total) {shards} do not tile [0, M_total)")
+    return M_total
+
+
+def stochastic_solve_batch_sharded(engines, x0s, theta, lbs, ubs, horizon, fmini, dual_dirs=None, optimizer=None, max_iterations=50,
+                                   use_eswavs=True, project=False):
+    """rbo_stochastic_solve_batch_sharded: RolloutEngine.stochastic_solve_batch over the samples of several engines (e.g. one per GPU),
+    each holding the same surrogate and starts and one shard of the same M_total normals (set_normals(rn, m_begin, m_count) or
+    generate_normals); the shards must tile [0, M_total), in any order. engines[0] leads: it gathers the shards' results every iteration
+    and runs the statistics and the step. dual_dirs is d x h x M_total. Returns the dict of RolloutEngine.stochastic_solve_batch, equal
+    bit for bit to one engine holding all M_total samples wherever that engine's result does not depend on the rollout kernel's hand-out
+    order (see include/rbo.h); fail[0, b] is a global sample index."""
+    engines = list(engines)
+    M_total = _check_shards(engines)
+    o = _sga_opts(Adam() if optimizer is None else optimizer, max_iterations, use_eswavs, project)
+    x0s, theta, lbs, ubs, dual_dirs = _sga_arrays(x0s, theta, lbs, ubs, horizon, dual_dirs, engines[0].d, M_total)
+    r, s = _sga_results(x0s.shape[0], x0s.shape[1], max_iterations)
+    lead = engines[0]
+    hs = (C.c_void_p * len(engines))(*[e.handle.h.value for e in engines])
+    lead.handle.check(lead.lib.rbo_stochastic_solve_batch_sharded(
+        hs, len(engines), C.byref(o), dptr(x0s), x0s.shape[1], dptr(theta), len(theta), dptr(lbs), dptr(ubs), int(horizon), float(fmini),
+        dptr(dual_dirs), *_sga_result_ptrs(r), C.byref(s)))
+    return r
+
+
+def stochastic_solve_batch(optimizer, T, tp, es, starts, max_iterations=50, use_eswavs=True, dual_directions=None, device=0, devices=None):
     """stochastic_solve (utils.jl:235-265) from every column of `starts` (d x B) at once, on the device: one library call, one
     synchronisation. Each restart runs the loop of `stochastic_solve` with its own optimiser state (from `optimizer`'s
     hyper-parameters; an Adam with t > 0 is rejected) and its own ESWAVS stop, on the same normals (common random numbers).
@@ -905,24 +953,38 @@ def stochastic_solve_batch(optimizer, T, tp, es, starts, max_iterations=50, use_
     global RNG and reused, as simulate_trajectory_mc_batch does: this is not the reference's per-iteration rand(dim) consumption (Q5),
     which `stochastic_solve` reproduces through its two-phase call.
 
+    `devices` (a list of device ids) splits the samples evenly over one engine per device (rbo_stochastic_solve_batch_sharded, the
+    same result, bit for bit where the one-device result does not depend on the hand-out order); None runs on `device` alone.
+
     Returns (X_final, histories): X_final is d x B (each restart's iterate after its last step, or the x at which it stopped);
     histories[b] lists the (x, mean, grad) tuples of `stochastic_solve` for restart b. Raises RboError naming the restart and the
     sample when a trajectory failed where the reference would have thrown."""
     d, h, M = len(tp.x0), tp.horizon, tp.mc_iters
     _sga_opts(optimizer, max_iterations, use_eswavs, False)
     starts = _sga_arrays(starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, dual_directions, d, M)[0]
+    devices = [device] if devices is None else list(devices)
+    if not 1 <= len(devices) <= M:
+        raise ValueError(f"stochastic_solve_batch: {len(devices)} devices for {M} samples; every device needs at least one")
     if dual_directions is None and h > 0:
         dual_directions = np.asfortranarray(np.random.rand(d, h, M))
-    eng = RolloutEngine(device)
+    engines = []
     try:
-        eng.set_surrogate(T.fs)
-        eng.set_normals(tp.rnstream_sequence)
-        eng.set_starts(get_starts(es))
+        for i, dev in enumerate(devices):
+            eng = RolloutEngine(dev)
+            engines.append(eng)
+            eng.set_surrogate(T.fs)
+            m0, m1 = M * i // len(devices), M * (i + 1) // len(devices)
+            eng.set_normals(tp.rnstream_sequence, m0, m1 - m0)
+            eng.set_starts(get_starts(es))
         fmini = float(np.min(get_observations(T.s)))  # rollout.jl:109
-        r = eng.stochastic_solve_batch(starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, fmini, dual_dirs=dual_directions, optimizer=optimizer,
-                                       max_iterations=max_iterations, use_eswavs=use_eswavs)
+        kw = dict(dual_dirs=dual_directions, optimizer=optimizer, max_iterations=max_iterations, use_eswavs=use_eswavs)
+        if len(engines) == 1:
+            r = engines[0].stochastic_solve_batch(starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, fmini, **kw)
+        else:
+            r = stochastic_solve_batch_sharded(engines, starts, tp.θ, tp.spatial_lbs, tp.spatial_ubs, h, fmini, **kw)
     finally:
-        eng.close()
+        for eng in engines:
+            eng.close()
     failed = np.nonzero(r["end_status"] == SGA_FAILED)[0]
     if len(failed):
         b = int(failed[0])

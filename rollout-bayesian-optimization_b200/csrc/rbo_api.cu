@@ -77,6 +77,8 @@ struct rbo_handle {
   int device = 0;
   cudaStream_t own_stream = nullptr, stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  // untimed: "rollout k done" on this handle, "step k done" when it leads rbo_stochastic_solve_batch_sharded (each reused every iteration)
+  cudaEvent_t ev_rollout = nullptr, ev_step = nullptr;
   int num_sms = 0, max_smem = 0;
   std::string err;
   rbo_solver_opts so;
@@ -89,6 +91,7 @@ struct rbo_handle {
   DevBuf<double> Xb, yb, c0, u0, Lf, Lb, Lbf, x0_batch;
   // normals / starts
   int M = 0, hp1 = 0;
+  int m_begin = 0, M_total = 0;  // the shard [m_begin, m_begin + M) of M_total samples these normals are
   DevBuf<double> rn;
   int S = 0;
   DevBuf<double> starts;
@@ -123,10 +126,15 @@ struct rbo_handle {
   // rbo_stochastic_solve_batch: optimiser state, bias corrections and history (doubles); per-restart integers; the work list
   DevBuf<double> sga_dbl;
   DevBuf<int> sga_int, worklist;
+  // rbo_stochastic_solve_batch_sharded, on the leader: every shard's values and grad_x; status and the watchdog flag table
+  DevBuf<double> sga_gather;
+  DevBuf<int> sga_igather;
 
   ~rbo_handle() {
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
+    if (ev_rollout) cudaEventDestroy(ev_rollout);
+    if (ev_step) cudaEventDestroy(ev_step);
     if (own_stream) cudaStreamDestroy(own_stream);
   }
 };
@@ -193,6 +201,8 @@ int rbo_create(rbo_handle** out, int device_id) {
   h->stream = h->own_stream;
   CK(nullptr, cudaEventCreate(&h->ev0));
   CK(nullptr, cudaEventCreate(&h->ev1));
+  CK(nullptr, cudaEventCreateWithFlags(&h->ev_rollout, cudaEventDisableTiming));
+  CK(nullptr, cudaEventCreateWithFlags(&h->ev_step, cudaEventDisableTiming));
   CK(nullptr, h->work_counter.reserve(16));  // [0] trajectory scheduler, [1..2] kernel watchdog flags
   CK(nullptr, h->cta_done.reserve(1024));
   CK(nullptr, h->sobol_dirs.reserve(sizeof(rbo_sobol_dirs_host) / sizeof(unsigned)));
@@ -431,6 +441,7 @@ int rbo_set_normals(rbo_handle* h, const double* rn, int M_total, int hp1, int m
   CK(h, cudaMemcpy2DAsync(h->rn, (size_t)m_count * 8, rn + m_begin, (size_t)M_total * 8, (size_t)m_count * 8, (size_t)q1 * hp1, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   h->M = m_count; h->hp1 = hp1; h->order_M = 0;
+  h->m_begin = m_begin; h->M_total = M_total;
   return RBO_SUCCESS;
 }
 
@@ -448,6 +459,7 @@ int rbo_generate_normals(rbo_handle* h, int M_total, int hp1, int m_begin, int m
   rbo_normals_kernel<<<blocks, 256, 0, h->stream>>>(h->sobol_dirs, h->rn, M_total, h->d, hp1, m_begin, m_count);
   CK(h, cudaGetLastError());
   h->M = m_count; h->hp1 = hp1; h->order_M = 0;
+  h->m_begin = m_begin; h->M_total = M_total;
   return RBO_SUCCESS;
 }
 
@@ -648,9 +660,13 @@ static cudaError_t enqueue_rollout(const rbo_handle* h, const DevProblem& P, con
 }
 
 // wd: the work_counter entries the rollout kernel's watchdog writes ([1], [2] flags; [4..8] where it waited)
-static int watchdog_fail(rbo_handle* h, const int* wd) {
-  return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", wd[1] ? "[panel pipeline wait never completed] " : "",
-              wd[2] ? "[inner solve exceeded its evaluation bound]" : "", wd[4], wd[5], wd[6], wd[7], wd[8]);
+// handle >= 0: the index of the flagging handle among the handles of rbo_stochastic_solve_batch_sharded
+static int watchdog_fail(rbo_handle* h, const int* wd, int handle = -1) {
+  char who[32] = "";
+  if (handle >= 0) snprintf(who, sizeof(who), " on handle %d", handle);
+  return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog%s: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", who,
+              wd[1] ? "[panel pipeline wait never completed] " : "", wd[2] ? "[inner solve exceeded its evaluation bound]" : "", wd[4], wd[5],
+              wd[6], wd[7], wd[8]);
 }
 
 static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
@@ -805,50 +821,114 @@ void rbo_default_sga_opts(rbo_sga_opts* o) {
   o->eps = 1e-8;
 }
 
-int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
-                               const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
-                               double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail_out, double* x_hist,
-                               double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist, rbo_summary* summary) {
-  if (!h) return RBO_ERR_ARG;
-  const char* me = "rbo_stochastic_solve_batch";
+}  // extern "C"
+
+// stochastic_solve from a batch of restarts over the n handles hs, each holding one shard of the samples (sharded: the shards of the
+// recorded M_total; otherwise n = 1 and the handle's own samples are the whole set). Per iteration k, every handle runs the work list
+// and the rollout of its shard on its own stream; the leader hs[0] waits for them, gathers every shard's values, grad_x, status and
+// watchdog flags in global sample order (restart-major) and runs the step kernel over them, and every other handle copies the new
+// iterates and live flags from the leader before its next iteration. With one handle nothing is gathered: the step reads the rollout's
+// own buffers. Every iteration is enqueued up front; each handle's stream is synchronised once, at the end.
+static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta,
+                     int ntheta, const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs, double* x_final,
+                     int32_t* n_iter, int32_t* end_status, int32_t* fail_out, double* x_hist, double* mean_hist, double* std_hist,
+                     double* gmean_hist, double* gstd_hist, rbo_summary* summary) {
+  const char* me = sharded ? "rbo_stochastic_solve_batch_sharded" : "rbo_stochastic_solve_batch";
+  rbo_handle* const h = hs[0];  // the leader: errors, optimiser state, statistics, history
+  for (int i = 1; i < n; ++i) {
+    if (!hs[i]) return fail(h, RBO_ERR_ARG, "%s: handle %d is NULL", me, i);
+    for (int j = 0; j < i; ++j)
+      if (hs[j] == hs[i]) return fail(h, RBO_ERR_ARG, "%s: handles %d and %d are the same handle", me, j, i);
+  }
   if (!o || !x0s || !x_final || !n_iter || !end_status) return fail(h, RBO_ERR_ARG, "%s: o, x0s, x_final, n_iter and end_status are required", me);
   if (n_x0 < 1) return fail(h, RBO_ERR_ARG, "%s: n_x0 = %d < 1", me, n_x0);
   if (o->max_iterations < 1) return fail(h, RBO_ERR_ARG, "%s: max_iterations = %d < 1", me, o->max_iterations);
   if (o->optimizer != RBO_OPT_SGA && o->optimizer != RBO_OPT_ADAM) return fail(h, RBO_ERR_ARG, "%s: unknown optimizer %d", me, o->optimizer);
   if (!(o->eta > 0.0)) return fail(h, RBO_ERR_ARG, "%s: eta = %g must be > 0", me, o->eta);
-  if (!h->have_sur) return fail(h, RBO_ERR_STATE, "%s: no surrogate (rbo_set_surrogate)", me);
-  if (!h->rn) return fail(h, RBO_ERR_STATE, "%s: no normals (rbo_set_normals / rbo_generate_normals)", me);
-  if (!h->starts) return fail(h, RBO_ERR_STATE, "%s: no starts (rbo_set_starts)", me);
-  CK(h, cudaSetDevice(h->device));
-  const int B = n_x0, d = h->d, Ms = h->M, maxit = o->max_iterations;
-  CK(h, h->x0_batch.reserve((size_t)B * d));
-  CK(h, cudaMemcpyAsync(h->x0_batch, x0s, (size_t)B * d * 8, cudaMemcpyHostToDevice, h->stream));
-  if (dual_dirs) {
-    const size_t nd = (size_t)Ms * std::max(horizon, 0) * d;
-    CK(h, h->dual_dirs.reserve(nd));
-    CK(h, cudaMemcpyAsync(h->dual_dirs, dual_dirs, nd * 8, cudaMemcpyHostToDevice, h->stream));
+  for (int i = 0; i < n; ++i) {
+    char who[32] = "";
+    if (sharded) snprintf(who, sizeof(who), "handle %d has ", i);
+    if (!hs[i]->have_sur) return fail(h, RBO_ERR_STATE, "%s: %sno surrogate (rbo_set_surrogate)", me, who);
+    if (!hs[i]->rn) return fail(h, RBO_ERR_STATE, "%s: %sno normals (rbo_set_normals / rbo_generate_normals)", me, who);
+    if (!hs[i]->starts) return fail(h, RBO_ERR_STATE, "%s: %sno starts (rbo_set_starts)", me, who);
   }
-  DevProblem P;
-  PlanChoice pc;
-  int grid = 0;
-  int rc = prepare_launch(h, x0s, theta, ntheta, lbs, ubs, horizon, fmini, RBO_MODE_VALUE_GRAD, 0, dual_dirs ? h->dual_dirs.p : nullptr, nullptr,
-                          h->x0_batch.p, B, P, pc, grid);
-  if (rc) return rc;
-  const int M = P.M;
-  // the conditions under which launch_rollout hands out longest-first; the order then follows the previous iteration's costs
-  const bool lpt = h->lpt && horizon > 0 && M > 2 * grid;
-  if (lpt) CK(h, h->order.reserve(M));
-  const int* order = P.order;
+  const int B = n_x0, d = h->d, maxit = o->max_iterations;
+  const int Mt = sharded ? h->M_total : h->M;  // samples over all handles
+  if (sharded) {
+    for (int i = 1; i < n; ++i) {
+      const rbo_handle* g = hs[i];
+      if (g->d != d || g->N != h->N || g->S != h->S || g->hp1 != h->hp1 || g->M_total != Mt)
+        return fail(h, RBO_ERR_ARG, "%s: handle %d holds (d, N, starts, hp1, M_total) = (%d, %d, %d, %d, %d), handle 0 (%d, %d, %d, %d, %d)", me,
+                    i, g->d, g->N, g->S, g->hp1, g->M_total, d, h->N, h->S, h->hp1, Mt);
+    }
+    std::vector<std::pair<int, int>> shards(n);  // (m_begin, handle)
+    for (int i = 0; i < n; ++i) shards[i] = {hs[i]->m_begin, i};
+    std::sort(shards.begin(), shards.end());
+    int next = 0;
+    for (const auto& sh : shards) {
+      if (sh.first != next)
+        return fail(h, RBO_ERR_ARG, "%s: the shards do not tile [0, %d): handle %d begins at sample %d, %d expected", me, Mt, sh.second, sh.first, next);
+      next += hs[sh.second]->M;
+    }
+    if (next != Mt) return fail(h, RBO_ERR_ARG, "%s: the shards do not tile [0, %d): they cover [0, %d)", me, Mt, next);
+  }
 
-  // device state: doubles [m | v | bias | x_hist | gmean_hist | gstd_hist | mean_hist | std_hist], ints [live | n_iter | end_status |
+  // every handle's launch is prepared before anything is enqueued: an error leaves every handle as it was
+  struct Shard {
+    DevProblem P;
+    PlanChoice pc;
+    int grid = 0, Ms = 0, m_begin = 0;
+    bool lpt = false;
+    const int* order = nullptr;
+  };
+  std::vector<Shard> sh(n);
+  for (int i = 0; i < n; ++i) {
+    rbo_handle* g = hs[i];
+    Shard& s = sh[i];
+    s.Ms = g->M;
+    s.m_begin = sharded ? g->m_begin : 0;
+    CK(h, cudaSetDevice(g->device));
+    CK(h, g->x0_batch.reserve((size_t)B * d));
+    if (dual_dirs) CK(h, g->dual_dirs.reserve((size_t)s.Ms * std::max(horizon, 0) * d));
+    int rc = prepare_launch(g, x0s, theta, ntheta, lbs, ubs, horizon, fmini, RBO_MODE_VALUE_GRAD, 0, dual_dirs ? g->dual_dirs.p : nullptr, nullptr,
+                            g->x0_batch.p, B, s.P, s.pc, s.grid);
+    if (rc) {
+      if (i > 0) h->err = std::string(me) + ": handle " + std::to_string(i) + ": " + g->err;
+      return rc;
+    }
+    // the conditions under which launch_rollout hands out longest-first; the order then follows the previous iteration's costs
+    s.lpt = g->lpt && horizon > 0 && s.P.M > 2 * s.grid;
+    if (s.lpt) CK(h, g->order.reserve(s.P.M));
+    s.order = s.P.order;
+    CK(h, g->worklist.reserve(s.P.M));
+    if (i > 0) CK(h, g->sga_int.reserve(B));  // live
+    s.P.order = g->worklist;
+  }
+  if (sharded)  // peer access where the devices allow it (the copies below work without it, through the host)
+    for (int i = 0; i < n; ++i)
+      for (int j = 0; j < n; ++j) {
+        const int di = hs[i]->device, dj = hs[j]->device;
+        int can = 0;
+        if (di == dj || cudaDeviceCanAccessPeer(&can, di, dj) != cudaSuccess || !can) continue;
+        CK(h, cudaSetDevice(di));
+        const cudaError_t e = cudaDeviceEnablePeerAccess(dj, 0);
+        if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+        else CK(h, e);
+      }
+
+  // leader state: doubles [m | v | bias | x_hist | gmean_hist | gstd_hist | mean_hist | std_hist], ints [live | n_iter | end_status |
   // fail (2 per restart) | nfail | sticky watchdog record (16)]
-  const size_t nx = (size_t)d * B, nh = (size_t)maxit * B;
+  CK(h, cudaSetDevice(h->device));
+  const size_t nx = (size_t)d * B, nh = (size_t)maxit * B, nt = (size_t)B * Mt;
   const size_t o_bias = 2 * nx, o_xh = o_bias + 2 * (size_t)maxit, o_gmh = o_xh + nh * d, o_gsh = o_gmh + nh * d, o_mh = o_gsh + nh * d,
                o_sh = o_mh + nh, n_dbl = o_sh + nh;
   const size_t i_iter = B, i_end = 2 * (size_t)B, i_fail = 3 * (size_t)B, i_nfail = 5 * (size_t)B, i_sticky = 6 * (size_t)B, n_int = i_sticky + 16;
   CK(h, h->sga_dbl.reserve(n_dbl));
   CK(h, h->sga_int.reserve(n_int));
-  CK(h, h->worklist.reserve(M));
+  if (n > 1) {
+    CK(h, h->sga_gather.reserve(nt * (1 + d)));  // values [B][Mt] | grad_x [B][Mt][d]
+    CK(h, h->sga_igather.reserve(nt + 16 * (size_t)n));  // status [B][Mt] | watchdog table [n][16]
+  }
   double* D = h->sga_dbl;
   int* I = h->sga_int;
   std::vector<double> bias(2 * (size_t)maxit);
@@ -862,44 +942,95 @@ int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const doubl
   CK(h, cudaMemcpyAsync(D + o_bias, bias.data(), bias.size() * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemsetAsync(D + o_xh, 0xff, (n_dbl - o_xh) * 8, h->stream));  // all-ones bytes: NaN past n_iter
   CK(h, cudaMemcpyAsync(I, ist.data(), n_int * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+  for (int i = 0; i < n; ++i) {  // every handle: the starting points, its slice of the dual directions, and (other handles) live = 1
+    rbo_handle* g = hs[i];
+    CK(h, cudaSetDevice(g->device));
+    CK(h, cudaMemcpyAsync(g->x0_batch, x0s, nx * 8, cudaMemcpyHostToDevice, g->stream));
+    if (dual_dirs) {
+      const size_t per = (size_t)std::max(horizon, 0) * d;  // dual_dirs[:, :, m] is contiguous: the shard is one block
+      CK(h, cudaMemcpyAsync(g->dual_dirs, dual_dirs + (size_t)sh[i].m_begin * per, (size_t)sh[i].Ms * per * 8, cudaMemcpyHostToDevice, g->stream));
+    }
+    if (i > 0) CK(h, cudaMemcpyAsync(g->sga_int, ist.data(), (size_t)B * sizeof(int), cudaMemcpyHostToDevice, g->stream));
+  }
+  CK(h, cudaSetDevice(h->device));
 
   SgaProblem S;
   memset(&S, 0, sizeof(S));
-  S.B = B; S.Ms = Ms; S.d = d; S.maxit = maxit;
+  S.B = B; S.Ms = Mt; S.d = d; S.maxit = maxit;
   S.optimizer = o->optimizer; S.use_eswavs = o->use_eswavs != 0; S.project = o->project != 0;
   S.eta = o->eta; S.beta1 = o->beta1; S.beta2 = o->beta2; S.eps = o->eps;
   S.omb1 = 1.0 - o->beta1; S.omb2 = 1.0 - o->beta2;
   for (int a = 0; a < d; ++a) { S.lbs[a] = lbs[a]; S.ubs[a] = ubs[a]; }
   S.bias = D + o_bias;
-  S.values = h->values; S.grad_x = h->grad_x; S.status = h->status; S.work_counter = h->work_counter;
+  if (n > 1) {
+    S.values = h->sga_gather; S.grad_x = h->sga_gather + nt; S.status = h->sga_igather; S.watchdog = h->sga_igather + nt;
+  } else {
+    S.values = h->values; S.grad_x = h->grad_x; S.status = h->status; S.watchdog = h->work_counter;
+  }
+  S.n_watchdog = n;
   S.x = h->x0_batch; S.m = D; S.v = D + nx;
   S.xh = D + o_xh; S.gmh = D + o_gmh; S.gsh = D + o_gsh; S.mh = D + o_mh; S.sh = D + o_sh;
   S.live = I; S.n_iter = I + i_iter; S.end_status = I + i_end; S.fail = I + i_fail; S.nfail = I + i_nfail; S.sticky = I + i_sticky;
 
   // every iteration enqueued at once: a launch after the last restart stopped hands out nothing
-  P.order = h->worklist;
   int launches = 0;
   CK(h, cudaEventRecord(h->ev0, h->stream));
   for (int k = 0; k < maxit; ++k) {
-    rbo_sga_worklist_kernel<<<1, 1024, 0, h->stream>>>(order, S.live, Ms, M, h->worklist);
-    CK(h, cudaGetLastError());
-    CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
-    CK(h, enqueue_rollout(h, P, pc, grid));
+    for (int i = 0; i < n; ++i) {
+      rbo_handle* g = hs[i];
+      Shard& s = sh[i];
+      CK(h, cudaSetDevice(g->device));
+      if (i > 0 && k > 0) {  // the iterates and live flags the leader's step k-1 left
+        CK(h, cudaStreamWaitEvent(g->stream, h->ev_step, 0));
+        CK(h, cudaMemcpyAsync(g->x0_batch, h->x0_batch, nx * 8, cudaMemcpyDefault, g->stream));
+        CK(h, cudaMemcpyAsync(g->sga_int, h->sga_int, (size_t)B * sizeof(int), cudaMemcpyDefault, g->stream));
+      }
+      rbo_sga_worklist_kernel<<<1, 1024, 0, g->stream>>>(s.order, g->sga_int, s.Ms, s.P.M, g->worklist);
+      CK(h, cudaGetLastError());
+      CK(h, cudaMemsetAsync(g->work_counter, 0, 16 * sizeof(int), g->stream));
+      CK(h, enqueue_rollout(g, s.P, s.pc, s.grid));
+      launches += 2;
+      if (n > 1) CK(h, cudaEventRecord(g->ev_rollout, g->stream));
+    }
+    CK(h, cudaSetDevice(h->device));
+    if (n > 1) {
+      double* gv = h->sga_gather;
+      double* gg = gv + nt;
+      int* gs = h->sga_igather;
+      for (int i = 0; i < n; ++i) {  // shard i at global sample m_begin of every restart
+        const rbo_handle* g = hs[i];
+        const size_t Ms = sh[i].Ms, m0 = sh[i].m_begin;
+        if (i > 0) CK(h, cudaStreamWaitEvent(h->stream, g->ev_rollout, 0));
+        CK(h, cudaMemcpy2DAsync(gv + m0, Mt * 8, g->values, Ms * 8, Ms * 8, B, cudaMemcpyDefault, h->stream));
+        CK(h, cudaMemcpy2DAsync(gg + m0 * d, Mt * d * 8, g->grad_x, Ms * d * 8, Ms * d * 8, B, cudaMemcpyDefault, h->stream));
+        CK(h, cudaMemcpy2DAsync(gs + m0, Mt * sizeof(int), g->status, Ms * sizeof(int), Ms * sizeof(int), B, cudaMemcpyDefault, h->stream));
+        CK(h, cudaMemcpyAsync(gs + nt + 16 * i, g->work_counter, 16 * sizeof(int), cudaMemcpyDefault, h->stream));
+      }
+    }
     rbo_sga_step_kernel<<<B, 256, 0, h->stream>>>(S, k);
     CK(h, cudaGetLastError());
-    launches += 3;
-    if (lpt) {
-      rbo_lpt_order_kernel<<<1, 1024, 0, h->stream>>>(h->n_evals, h->grad_case, h->best_index, M, horizon, h->order);
+    ++launches;
+    if (n > 1) CK(h, cudaEventRecord(h->ev_step, h->stream));
+    for (int i = 0; i < n; ++i) {
+      rbo_handle* g = hs[i];
+      Shard& s = sh[i];
+      if (!s.lpt) continue;
+      CK(h, cudaSetDevice(g->device));
+      rbo_lpt_order_kernel<<<1, 1024, 0, g->stream>>>(g->n_evals, g->grad_case, g->best_index, s.P.M, horizon, g->order);
       CK(h, cudaGetLastError());
-      order = h->order;
+      s.order = g->order;
       ++launches;
     }
   }
+  CK(h, cudaSetDevice(h->device));
   CK(h, cudaEventRecord(h->ev1, h->stream));
-  h->order_M = lpt ? M : 0;
-  h->last_mode = RBO_MODE_VALUE_GRAD;
-  // the per-trajectory buffers now hold each restart's last iteration: no read-back and no replay until the next rollout
-  h->outM = 0; h->outh = -1; h->xs_valid = false;
+  for (int i = 0; i < n; ++i) {
+    rbo_handle* g = hs[i];
+    g->order_M = sh[i].lpt ? sh[i].P.M : 0;
+    g->last_mode = RBO_MODE_VALUE_GRAD;
+    // the per-trajectory buffers now hold each restart's last iteration: no read-back and no replay until the next rollout
+    g->outM = 0; g->outh = -1; g->xs_valid = false;
+  }
 
   std::vector<int> ires(n_int);
   CK(h, cudaMemcpyAsync(x_final, h->x0_batch, nx * 8, cudaMemcpyDeviceToHost, h->stream));
@@ -909,11 +1040,14 @@ int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const doubl
   if (gstd_hist) CK(h, cudaMemcpyAsync(gstd_hist, D + o_gsh, nh * d * 8, cudaMemcpyDeviceToHost, h->stream));
   if (mean_hist) CK(h, cudaMemcpyAsync(mean_hist, D + o_mh, nh * 8, cudaMemcpyDeviceToHost, h->stream));
   if (std_hist) CK(h, cudaMemcpyAsync(std_hist, D + o_sh, nh * 8, cudaMemcpyDeviceToHost, h->stream));
-  CK(h, cudaStreamSynchronize(h->stream));
+  for (int i = n - 1; i >= 0; --i) {
+    CK(h, cudaSetDevice(hs[i]->device));
+    CK(h, cudaStreamSynchronize(hs[i]->stream));
+  }
   std::memcpy(n_iter, ires.data() + i_iter, (size_t)B * sizeof(int));
   std::memcpy(end_status, ires.data() + i_end, (size_t)B * sizeof(int));
   if (fail_out) std::memcpy(fail_out, ires.data() + i_fail, 2 * (size_t)B * sizeof(int));
-  if (ires[i_sticky]) return watchdog_fail(h, ires.data() + i_sticky);
+  if (ires[i_sticky]) return watchdog_fail(h, ires.data() + i_sticky, sharded ? ires[i_sticky + 9] : -1);
   if (summary) {
     float ms = 0;
     CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -923,11 +1057,33 @@ int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const doubl
     summary->kernel_ms = ms;
     summary->gpu_launches = launches;
     long long ntraj = 0, nfailed = 0;
-    for (int b = 0; b < B; ++b) { ntraj += (long long)ires[i_iter + b] * Ms; nfailed += ires[i_nfail + b]; }
+    for (int b = 0; b < B; ++b) { ntraj += (long long)ires[i_iter + b] * Mt; nfailed += ires[i_nfail + b]; }
     summary->n_traj = (int)ntraj;
     summary->n_failed = (int)nfailed;
   }
   return RBO_SUCCESS;
+}
+
+extern "C" {
+
+int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
+                               const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
+                               double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail_out, double* x_hist,
+                               double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist, rbo_summary* summary) {
+  if (!h) return RBO_ERR_ARG;
+  return sga_solve(&h, 1, false, o, x0s, n_x0, theta, ntheta, lbs, ubs, horizon, fmini, dual_dirs, x_final, n_iter, end_status, fail_out,
+                   x_hist, mean_hist, std_hist, gmean_hist, gstd_hist, summary);
+}
+
+int rbo_stochastic_solve_batch_sharded(rbo_handle* const* hs, int n_handles, const rbo_sga_opts* o, const double* x0s, int n_x0,
+                                       const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon, double fmini,
+                                       const double* dual_dirs, double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail_out,
+                                       double* x_hist, double* mean_hist, double* std_hist, double* gmean_hist, double* gstd_hist,
+                                       rbo_summary* summary) {
+  if (!hs || n_handles < 1) return fail(nullptr, RBO_ERR_ARG, "rbo_stochastic_solve_batch_sharded: n_handles = %d < 1", n_handles);
+  if (!hs[0]) return fail(nullptr, RBO_ERR_ARG, "rbo_stochastic_solve_batch_sharded: handle 0 is NULL");
+  return sga_solve(hs, n_handles, true, o, x0s, n_x0, theta, ntheta, lbs, ubs, horizon, fmini, dual_dirs, x_final, n_iter, end_status, fail_out,
+                   x_hist, mean_hist, std_hist, gmean_hist, gstd_hist, summary);
 }
 
 int rbo_partial_sums_device(rbo_handle* h, double* sums_device, int len) {

@@ -1,6 +1,8 @@
 // sga_kernels.cu -- the per-iteration kernels of rbo_stochastic_solve_batch (include/rbo.h): stochastic_solve (utils.jl:235-265)
 // from a batch of restarts with no host round trip. One iteration is
 //   rbo_sga_worklist_kernel -> the rollout kernel (unchanged) -> rbo_sga_step_kernel [-> rbo_lpt_order_kernel].
+// Over several handles (rbo_stochastic_solve_batch_sharded) each runs the work list, rollout and order kernels on its own shard of
+// the samples; the step kernel runs once, on the leader, over the shards' outputs gathered in global sample order.
 // The rollout kernel hands out P.order[i] and ends a CTA at the first entry >= P.M, so the work list below (the live restarts'
 // trajectories, then the sentinel M) is all it takes to stop restarts on the device.
 #include "sga_kernels.cuh"
@@ -68,12 +70,16 @@ __global__ void __launch_bounds__(SGA_THREADS) rbo_sga_step_kernel(const __grid_
   __shared__ double s_mean[RBO_MAXD + 1], s_std[RBO_MAXD + 1];
   __shared__ double s_bc;
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  const int* wc = S.work_counter;
-  // kernel watchdog: the memset before each rollout launch clears work_counter[1..2]; a flag seen once stops every restart
-  if (S.sticky[0] != 0 || wc[1] != 0 || wc[2] != 0) {
+  // kernel watchdog: the memset before each rollout launch clears work_counter[1..2]; a flag seen once, on any handle, stops every restart
+  int flagged = -1;
+  for (int i = 0; i < S.n_watchdog && flagged < 0; ++i)
+    if (S.watchdog[16 * i + 1] != 0 || S.watchdog[16 * i + 2] != 0) flagged = i;
+  if (S.sticky[0] != 0 || flagged >= 0) {
     if (tid == 0) {
       if (b == 0 && S.sticky[0] == 0) {
+        const int* wc = S.watchdog + 16 * flagged;
         for (int i = 1; i <= 8; ++i) S.sticky[i] = wc[i];
+        S.sticky[9] = flagged;
         S.sticky[0] = 1;
       }
       S.live[b] = 0;

@@ -470,3 +470,41 @@ function simulate_trajectory_mc_multigpu(T::Trajectory, tp::TrajectoryParameters
     return ExpectedTrajectoryOutput(μxθ = μxθ, σ_μxθ = σ_μxθ, ∇μx = ∇μx, σ_∇μx = vec(Distributions.std(spatial_gradients_container, dims = 2, mean = ∇μx)),
                                     ∇μθ = ∇μθ, σ_∇μθ = vec(Distributions.std(hyperparameter_gradients_container, dims = 2, mean = ∇μθ)))
 end
+
+# stochastic_solve_batch with the samples split evenly over one handle per entry of `devices` (rbo_stochastic_solve_batch_sharded):
+# every handle runs the rollouts of its shard, the first gathers the shards' results every iteration and takes the step. The final
+# iterates equal those of one handle holding every sample (bit for bit where that handle's do not depend on the hand-out order,
+# include/rbo.h). Fresh handles: the resident inputs of _rbo_handle stay as
+# they were.
+function stochastic_solve_batch_multigpu(; optimizer::StochasticGradientAscent, surrogate::Surrogate, tp::TrajectoryParameters,
+                                         es::ExperimentSetup, starts::Matrix{Float64}, devices::Vector{Int})
+    T = _rbo_trajectory(surrogate, tp)
+    fs = get_fantasy_surrogate(T)
+    N = get_known_observations(fs)
+    rn = tp.rnstream_sequence
+    M, d, hor, B, n = tp.mc_iters, length(tp.x0), tp.horizon, size(starts, 2), length(devices)
+    1 <= n <= M || error("stochastic_solve_batch_multigpu: $n devices for $M samples")
+    xs = get_starts(es)
+    bounds = [div(M * g, n) for g in 0:n]
+    hs = [RboHandle(dev) for dev in devices]
+    for (g, h) in enumerate(hs)
+        _rbo_set_surrogate!(h, fs.X, fs.L.data, fs.y, fs.cs[1], N, fs.ψ, fs.g, fs.σn2)
+        _rbo_check(h, ccall((:rbo_set_normals, librbo), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Cint, Cint, Cint), h.ptr, rn, M, size(rn, 3), bounds[g], bounds[g+1] - bounds[g]))
+        _rbo_check(h, ccall((:rbo_set_starts, librbo), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint), h.ptr, xs, size(xs, 2)))
+    end
+    θ = Vector{Float64}(tp.θ)
+    dual = rand(d, max(hor, 1), M)
+    opts = Ref(_rbo_sga_opts(optimizer))
+    xfinal = zeros(d, B); n_iter = zeros(Int32, B); end_status = zeros(Int32, B); fail = zeros(Int32, 2, B)
+    ptrs = [h.ptr for h in hs]
+    GC.@preserve hs _rbo_check(hs[1], ccall((:rbo_stochastic_solve_batch_sharded, librbo), Cint,
+        (Ptr{Ptr{Cvoid}}, Cint, Ref{RboSgaOpts}, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64},
+         Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cvoid}),
+        ptrs, n, opts, starts, B, θ, length(θ), tp.spatial_lbs, tp.spatial_ubs, hor, minimum(get_observations(surrogate)), dual,
+        xfinal, n_iter, end_status, fail, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL))
+    for b in 1:B
+        end_status[b] == 2 || continue                                                      # RBO_SGA_FAILED: the serial loop would throw
+        error("restart $b, sample $(fail[1, b] + 1): " * get(_RBO_STATUS, Int(fail[2, b]), "error"))
+    end
+    return xfinal
+end
