@@ -226,8 +226,9 @@ void rbo_default_sga_opts(rbo_sga_opts* o);
  * Errors: RBO_ERR_ARG for n_x0 < 1, max_iterations < 1, an unknown optimiser or eta <= 0; RBO_ERR_STATE without surrogate,
  * normals or starts; the plan limits of rbo_rollout (RBO_ERR_UNSUPPORTED); RBO_ERR_CUDA with the watchdog message if the rollout
  * kernel reported a stuck pipeline (every restart stops then). Afterwards the handle keeps its surrogate, normals and starts;
- * RBO_FLAG_REPLAY_TAPE and the per-trajectory read-backs are refused until the next rollout, because the last launch did not
- * run every restart. Over several GPUs, or several handles that each hold a shard of the samples: rbo_stochastic_solve_batch_sharded. */
+ * RBO_FLAG_REPLAY_TAPE, the per-trajectory read-backs and the partial sums (rbo_partial_sums_*) are refused with RBO_ERR_STATE
+ * until the next rollout, because the last launch did not run every restart and computed no statistics. Over several GPUs, or
+ * several handles that each hold a shard of the samples: rbo_stochastic_solve_batch_sharded. */
 int rbo_stochastic_solve_batch(rbo_handle* h, const rbo_sga_opts* o, const double* x0s, int n_x0, const double* theta, int ntheta,
                                const double* lbs, const double* ubs, int horizon, double fmini, const double* dual_dirs,
                                double* x_final, int32_t* n_iter, int32_t* end_status, int32_t* fail, double* x_hist,
@@ -264,7 +265,8 @@ int rbo_stochastic_solve_batch_sharded(rbo_handle* const* hs, int n_handles, con
  * length 1 + 3*(1 + d + ntheta) + 2. Written to a DEVICE buffer (e.g. a torch tensor handed to NCCL), stream-ordered.
  * n counts the trajectories with status RBO_TRAJ_OK only -- failed ones are excluded from every sum and counted in n_failed;
  * watchdog != 0 if the kernel reported a stuck pipeline or an inner solve beyond its evaluation bound.
- * M2 is the centred sum of squares around this handle's own mean (two-pass, as rollout.jl:328-337). */
+ * M2 is the centred sum of squares around this handle's own mean (two-pass, as rollout.jl:328-337).
+ * RBO_ERR_STATE before the first rollout of the handle and after an SGA loop until the next rollout; RBO_ERR_ARG if len is short. */
 int rbo_partial_sums_device(rbo_handle* h, double* sums_device, int len);
 /* The same vector on the HOST, for a single-process multi-GPU host (e.g. Julia: one handle per device, rbo_rollout_device on each --
  * the launches are asynchronous --, then this call per handle, an element-wise sum, rbo_finalize_sums): waits for this handle's launch. */

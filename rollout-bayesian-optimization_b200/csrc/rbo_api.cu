@@ -73,6 +73,14 @@ struct DevBuf {
   operator T*() const { return p; }
 };
 
+// The launch the outputs hold; every read-back checks valid(): a rollout's results and statistics, not after an SGA loop until the next.
+struct LastLaunch {
+  int M = 0, h = -1, S = 0, d = 0, nth = 0, mode = 0;
+  bool xs = false, tape_ex = false;  // its x-path is on the device (RBO_FLAG_REPLAY_TAPE); it ran with RBO_FLAG_TAPE_EX
+  bool valid() const { return h >= 0; }
+  void reset() { *this = LastLaunch(); }
+};
+
 struct rbo_handle {
   int device = 0;
   cudaStream_t own_stream = nullptr, stream = nullptr;
@@ -96,24 +104,19 @@ struct rbo_handle {
   int S = 0;
   DevBuf<double> starts;
   DevBuf<unsigned> sobol_dirs;
-  // outputs, and the shape of the last launch they hold (what the read-back calls and RBO_FLAG_REPLAY_TAPE go by)
-  int outM = 0, outh = -1, outS = 0, outd = 0, outnth = 0;
+  LastLaunch last;  // the launch the outputs below hold
   DevBuf<double> values, grad_x, grad_theta, xs, ys, gys, alphas;
   DevBuf<int> best_index, grad_case, status, n_evals, start_status, start_iters;
   DevBuf<int> work_counter;
-  DevBuf<double> sums;
-  int sums_len = 0;
+  DevBuf<double> sums;  // StatsLayout::len, then room for the gathered vector (rbo_partial_sums_host)
   DevBuf<double> dual_dirs, x_forced, cs_tape, gh_nodes, gh_weights;
   int gh_depth = 0, gh_M = 0;
-  int last_mode = 0;
   double htol = 1e-4;
   int rs_cap = 0;           // development knob: cap on the row splits of the Gram reductions (0 = default)
   int vglob_wmax = 0;       // development knob: cap on the start slots of the large-n variant (0 = default)
   int force_vglob = 0;      // development / test knob: use the large-n variant even when shared memory would do
   DevBuf<double> Vscratch, Bscratch;
   DevBuf<double> t_mu, t_sigma, t_dmu, t_dsigma, t_Halpha;
-  bool tex_valid = false;
-  bool xs_valid = false;    // the x-path of the last rollout is on the device (RBO_FLAG_REPLAY_TAPE)
   DevBuf<int> order;        // longest-first order of the trajectories of the last launch (scheduling hint for the next one)
   int order_M = 0;          // 0: no valid order
   int lpt = 1;              // RBO_TUNE_LPT
@@ -160,6 +163,12 @@ template <class T>
 static cudaError_t copy_out(T* dst, const DevBuf<T>& src, size_t n, cudaStream_t stream) {
   return dst ? cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, stream) : cudaSuccess;
 }
+// H2D of n elements of src into dst, grown to hold them (stream-ordered).
+template <class T>
+static cudaError_t copy_in(DevBuf<T>& dst, const T* src, size_t n, cudaStream_t stream) {
+  const cudaError_t e = dst.reserve(n);
+  return e != cudaSuccess ? e : cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyHostToDevice, stream);
+}
 
 extern "C" {
 
@@ -203,7 +212,7 @@ int rbo_create(rbo_handle** out, int device_id) {
   CK(nullptr, cudaEventCreate(&h->ev1));
   CK(nullptr, cudaEventCreateWithFlags(&h->ev_rollout, cudaEventDisableTiming));
   CK(nullptr, cudaEventCreateWithFlags(&h->ev_step, cudaEventDisableTiming));
-  CK(nullptr, h->work_counter.reserve(16));  // [0] trajectory scheduler, [1..2] kernel watchdog flags
+  CK(nullptr, h->work_counter.reserve(WC_LEN));
   CK(nullptr, h->cta_done.reserve(1024));
   CK(nullptr, h->sobol_dirs.reserve(sizeof(rbo_sobol_dirs_host) / sizeof(unsigned)));
   CK(nullptr, cudaMemcpyAsync(h->sobol_dirs, rbo_sobol_dirs_host, sizeof(rbo_sobol_dirs_host), cudaMemcpyHostToDevice, h->stream));
@@ -477,10 +486,8 @@ int rbo_set_quadrature(rbo_handle* h, const double* nodes, const double* weights
   if (!nodes || !weights || depth < 1 || m_count < 1) return fail(h, RBO_ERR_ARG, "rbo_set_quadrature: bad arguments");
   CK(h, cudaSetDevice(h->device));
   const size_t n = (size_t)depth * m_count;
-  CK(h, h->gh_nodes.reserve(n));
-  CK(h, h->gh_weights.reserve(n));
-  CK(h, cudaMemcpyAsync(h->gh_nodes, nodes, n * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(h, cudaMemcpyAsync(h->gh_weights, weights, n * 8, cudaMemcpyHostToDevice, h->stream));
+  CK(h, copy_in(h->gh_nodes, nodes, n, h->stream));
+  CK(h, copy_in(h->gh_weights, weights, n, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   h->gh_depth = depth; h->gh_M = m_count;
   return RBO_SUCCESS;
@@ -492,8 +499,7 @@ int rbo_set_starts(rbo_handle* h, const double* starts, int S) {
   if (!starts || S < 1) return fail(h, RBO_ERR_ARG, "rbo_set_starts: bad arguments");
   if (S > 65535) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_set_starts: %d starts (the kernel keeps per-start counters and the hand-out order as 16-bit values: at most 65535)", S);
   CK(h, cudaSetDevice(h->device));
-  CK(h, h->starts.reserve((size_t)S * h->d));
-  CK(h, cudaMemcpyAsync(h->starts, starts, (size_t)S * h->d * 8, cudaMemcpyHostToDevice, h->stream));
+  CK(h, copy_in(h->starts, starts, (size_t)S * h->d, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
   h->S = S;
   return RBO_SUCCESS;
@@ -504,9 +510,10 @@ int rbo_set_starts(rbo_handle* h, const double* starts, int S) {
 // ---------------------------------------------------------------------------------------------------------
 // Makes the output buffers hold a launch of M trajectories (horizon hor, S starts) and records that shape.
 static int ensure_outputs(rbo_handle* h, int M, int hor, int S, int d, int nth) {
-  if (h->outM == M && h->outh == hor && h->outS == S && h->outd == d && h->outnth == nth) return RBO_SUCCESS;
+  LastLaunch& o = h->last;
+  if (o.M == M && o.h == hor && o.S == S && o.d == d && o.nth == nth) return RBO_SUCCESS;
   const int hh = std::max(hor, 1);
-  h->outM = 0; h->outh = -1; h->xs_valid = false;  // the record is only valid once every buffer below holds its shape
+  o.reset();  // the record is only valid once every buffer below holds its shape
   CK(h, h->values.reserve((size_t)M));
   CK(h, h->grad_x.reserve((size_t)M * d));
   CK(h, h->grad_theta.reserve((size_t)M * nth));
@@ -520,9 +527,9 @@ static int ensure_outputs(rbo_handle* h, int M, int hor, int S, int d, int nth) 
   CK(h, h->n_evals.reserve((size_t)M * hh));
   CK(h, h->start_status.reserve((size_t)M * hh * S));
   CK(h, h->start_iters.reserve((size_t)M * hh * S));
-  h->sums_len = 1 + 3 * (1 + d + nth) + hh + (hor + 2) + 2;
-  CK(h, h->sums.reserve((size_t)h->sums_len + 1 + 3 * (1 + d + nth) + 2));  // + the gathered partial-sums vector (rbo_partial_sums_host)
-  h->outM = M; h->outh = hor; h->outS = S; h->outd = d; h->outnth = nth;
+  const StatsLayout L(d, nth, hor);
+  CK(h, h->sums.reserve((size_t)L.len + L.gathered));
+  o.M = M; o.h = hor; o.S = S; o.d = d; o.nth = nth;
   return RBO_SUCCESS;
 }
 
@@ -576,55 +583,65 @@ static double f_step(double n, double d) { return 2 * n * n * (d + 1) + 2 * n * 
 // what this implementation executes per evaluation: (d+1) forward + 1 backward substitutions, Gram + two Hessian sums
 static double f_eval_exec(double n, double d) { return n * n * (d + 2) + n * (3 * d * (d + 1) + 4 * d + 40); }
 
+// The inputs of one rollout launch; dual_dirs, x_forced and x0_batch (d x B starting points) are device arrays or NULL.
+struct RolloutArgs {
+  const double *x0, *theta; int ntheta; const double *lbs, *ubs; int horizon; double fmini; int mode, flags;
+  const double *dual_dirs = nullptr, *x_forced = nullptr, *x0_batch = nullptr; int B = 1;
+};
+// A prepared launch: the rollout kernel's parameter block, its plan and grid, and whether it hands out longest-first.
+struct Launch { DevProblem P; PlanChoice pc; int grid = 0; bool lpt = false; };
+
 // Validates a launch, chooses its plan, makes the output and scratch buffers hold it and fills the rollout kernel's parameter block
-// P (P.order: the longest-first order of the previous launch when it applies) and its grid. Enqueues no kernel.
-static int prepare_launch(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
-                          double fmini, int mode, int flags, const double* dual_dirs_dev, const double* x_forced_dev,
-                          const double* x0_batch_dev, int B, DevProblem& P, PlanChoice& pc, int& grid) {
+// (P.order: the recorded longest-first order when it applies) and its grid. Enqueues no kernel.
+static int prepare_launch(rbo_handle* h, const RolloutArgs& a, Launch& L) {
+  int flags = a.flags, horizon = a.horizon;
   const bool myopic = (flags & RBO_FLAG_MYOPIC_INTERNAL) != 0, ghq = (flags & RBO_FLAG_GAUSS_HERMITE) != 0;
   if (!h->have_sur) return fail(h, RBO_ERR_STATE, "rbo_rollout: no surrogate (rbo_set_surrogate)");
   if (ghq && !h->gh_nodes) return fail(h, RBO_ERR_STATE, "rbo_rollout: no quadrature data (rbo_set_quadrature)");
   if (!h->rn && !myopic && !ghq) return fail(h, RBO_ERR_STATE, "rbo_rollout: no normals (rbo_set_normals / rbo_generate_normals)");
   if (!h->starts && !(flags & RBO_FLAG_TEACHER_FORCED)) return fail(h, RBO_ERR_STATE, "rbo_rollout: no starts (rbo_set_starts)");
-  if (!x0 || !theta || !lbs || !ubs || ntheta < 1) return fail(h, RBO_ERR_ARG, "rbo_rollout: bad arguments");
+  if (!a.x0 || !a.theta || !a.lbs || !a.ubs || a.ntheta < 1) return fail(h, RBO_ERR_ARG, "rbo_rollout: bad arguments");
   if (horizon < 0 || horizon + 1 > RBO_MAXFAN) return fail(h, RBO_ERR_UNSUPPORTED, "rbo_rollout: horizon %d not in [0, %d]", horizon, RBO_MAXFAN - 1);
   if (!myopic && !ghq && horizon + 1 > h->hp1) return fail(h, RBO_ERR_ARG, "rbo_rollout: normals hold %d steps, horizon + 1 = %d needed", h->hp1, horizon + 1);
   if (ghq && horizon + 1 > h->gh_depth) return fail(h, RBO_ERR_ARG, "rbo_rollout: quadrature depth %d < horizon + 1 = %d", h->gh_depth, horizon + 1);
   const int Ms = myopic ? 1 : (ghq ? h->gh_M : h->M);  // sample indices
-  const int M = Ms * std::max(B, 1);                    // trajectories of this launch
+  const int B = std::max(a.B, 1), M = Ms * B;          // trajectories of this launch
   if (flags & RBO_FLAG_REPLAY_TAPE) {
     // second phase of the two-phase call: replay the x-path of the previous rollout of this handle (still on the device)
-    if (myopic || h->outh != horizon || h->outM != M || !h->xs_valid) return fail(h, RBO_ERR_STATE, "rbo_rollout: RBO_FLAG_REPLAY_TAPE needs a preceding rollout with the same samples and horizon on this handle");
+    const LastLaunch& o = h->last;
+    if (myopic || !o.valid() || o.h != horizon || o.M != M || !o.xs) return fail(h, RBO_ERR_STATE, "rbo_rollout: RBO_FLAG_REPLAY_TAPE needs a preceding rollout with the same samples and horizon on this handle");
     flags |= RBO_FLAG_TEACHER_FORCED;
-  } else if ((flags & RBO_FLAG_TEACHER_FORCED) && !x_forced_dev) return fail(h, RBO_ERR_ARG, "rbo_rollout: teacher forcing without x_forced");
-  if (mode != RBO_MODE_VALUE && mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_ARG, "rbo_rollout: bad mode");
-  for (int a = 0; a < h->d; ++a)
-    if (!(lbs[a] <= ubs[a])) return fail(h, RBO_ERR_ARG, "rbo_rollout: lower bound above upper bound in dimension %d", a);
+  } else if ((flags & RBO_FLAG_TEACHER_FORCED) && !a.x_forced) return fail(h, RBO_ERR_ARG, "rbo_rollout: teacher forcing without x_forced");
+  if (a.mode != RBO_MODE_VALUE && a.mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_ARG, "rbo_rollout: bad mode");
+  for (int k = 0; k < h->d; ++k)
+    if (!(a.lbs[k] <= a.ubs[k])) return fail(h, RBO_ERR_ARG, "rbo_rollout: lower bound above upper bound in dimension %d", k);
   CK(h, cudaSetDevice(h->device));
   const int S = std::max(h->S, 1);
-  if (!choose_plan(h, horizon, S, mode, &pc))
+  PlanChoice& pc = L.pc;
+  if (!choose_plan(h, horizon, S, a.mode, &pc))
     return fail(h, RBO_ERR_UNSUPPORTED, "rbo_rollout: problem (d=%d, N=%d, h=%d) needs more than %d bytes of shared memory per CTA", h->d, h->N, horizon, h->max_smem);
   if (getenv("RBO_DEBUG")) fprintf(stderr, "[rbo] plan: W=%d RP=%d NR=%d RSmax=%d NPmax=%d xsm=%d smem=%zu B (limit %d)\n", pc.W, pc.RP, pc.NR, pc.RSmax, pc.NPmax, pc.xsm, pc.bytes, h->max_smem);
   if (getenv("RBO_DEBUG")) fprintf(stderr, "[rbo] plan: RSh=%d vglob=%d\n", pc.RSh, pc.vglob);
-  int rc = ensure_outputs(h, M, horizon, S, h->d, ntheta);
+  int rc = ensure_outputs(h, M, horizon, S, h->d, a.ntheta);
   if (rc) return rc;
+  DevProblem& P = L.P;
   memset(&P, 0, sizeof(P));
   P.d = h->d; P.N = h->N; P.N8 = h->N8; P.nb8 = h->nb8; P.nb32 = h->nb32; P.h = horizon; P.S = S; P.W = pc.W; P.RSmax = pc.RSmax; P.NPmax = pc.NPmax; P.xsm = pc.xsm; P.XP = h->N8 + 1;
   P.RSh = pc.RSh;
   P.pl = make_plan(P.d, P.N8, horizon, pc.W, pc.RP, pc.NR, pc.RSmax, pc.NPmax, pc.xsm, pc.RSh, pc.vglob, S);
   P.vglob = pc.vglob;
-  P.CS = h->d + 3; P.RP = pc.RP; P.NR = pc.NR; P.M = M; P.Ms = Ms; P.B = std::max(B, 1); P.x0_batch = (B > 1 || x0_batch_dev) ? x0_batch_dev : nullptr; P.hp1 = h->hp1; P.mode = mode; P.flags = flags; P.ntheta = ntheta;
+  P.CS = h->d + 3; P.RP = pc.RP; P.NR = pc.NR; P.M = M; P.Ms = Ms; P.B = B; P.x0_batch = a.x0_batch; P.hp1 = h->hp1; P.mode = a.mode; P.flags = flags; P.ntheta = a.ntheta;
   P.kern = h->kern; P.rule_id = h->rule_id; P.sigma_tol = h->sigma_tol; P.sigma_n2 = h->sigma_n2; P.k0 = h->k0; P.d2k0 = h->d2k0;
-  P.ymin_base = h->ymin_base; P.m52_c = std::sqrt(5.0) / h->kern.th[0]; P.fmini = fmini; P.theta1 = theta[0]; P.htol = h->htol; P.so = h->so;
-  for (int a = 0; a < h->d; ++a) { P.x0[a] = x0[a]; P.lbs[a] = lbs[a]; P.ubs[a] = ubs[a]; }
+  P.ymin_base = h->ymin_base; P.m52_c = std::sqrt(5.0) / h->kern.th[0]; P.fmini = a.fmini; P.theta1 = a.theta[0]; P.htol = h->htol; P.so = h->so;
+  for (int k = 0; k < h->d; ++k) { P.x0[k] = a.x0[k]; P.lbs[k] = a.lbs[k]; P.ubs[k] = a.ubs[k]; }
   P.Xb = h->Xb; P.yb = h->yb; P.c0 = h->c0; P.u0 = h->u0; P.Lf = h->Lf; P.Lb = h->Lb; P.Lbf = h->Lbf; P.rn = h->rn; P.starts = h->starts;
-  P.dual_dirs = dual_dirs_dev; P.x_forced = x_forced_dev;
+  P.dual_dirs = a.dual_dirs; P.x_forced = a.x_forced;
   P.gh_nodes = h->gh_nodes; P.gh_weights = h->gh_weights; P.gh_depth = h->gh_depth;
   P.values = h->values; P.grad_x = h->grad_x; P.grad_theta = h->grad_theta; P.best_index = h->best_index; P.grad_case = h->grad_case;
   P.status = h->status; P.xs = h->xs; P.ys = h->ys; P.gys = h->gys; P.alphas = h->alphas; P.n_evals = h->n_evals;
   P.start_status = h->start_status; P.start_iters = h->start_iters;
   P.work_counter = h->work_counter;
-  h->tex_valid = false;
+  h->last.tape_ex = false;
   if (flags & RBO_FLAG_TAPE_EX) {
     if (myopic) return fail(h, RBO_ERR_ARG, "rbo_rollout: RBO_FLAG_TAPE_EX does not apply to the myopic solve");
     const size_t n = (size_t)M * std::max(horizon, 1), d = h->d;
@@ -634,11 +651,14 @@ static int prepare_launch(rbo_handle* h, const double* x0, const double* theta, 
     CK(h, h->t_dsigma.reserve(n * d));
     CK(h, h->t_Halpha.reserve(n * d * d));
     P.t_mu = h->t_mu; P.t_sigma = h->t_sigma; P.t_dmu = h->t_dmu; P.t_dsigma = h->t_dsigma; P.t_Halpha = h->t_Halpha;
-    h->tex_valid = true;
+    h->last.tape_ex = true;
   }
-  grid = std::min(M, h->num_sms);
-  // longest-first hand-out when the previous launch ran the same trajectories (same normals, nearby x0): only worth it beyond two waves
-  P.order = (h->lpt && !myopic && h->order_M == M && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) ? h->order.p : nullptr;
+  const int grid = L.grid = std::min(M, h->num_sms);
+  // Longest-first (RBO_TUNE_LPT): a launch's evaluation counts order the next launch on the same trajectories (not myopic, not forced),
+  // beyond two waves. Such a launch records the order for the next one and uses the recorded one if that covers the same M.
+  L.lpt = h->lpt && !myopic && !(flags & RBO_FLAG_TEACHER_FORCED) && horizon > 0 && M > 2 * grid;
+  if (L.lpt) CK(h, h->order.reserve(M));
+  P.order = L.lpt && h->order_M == M ? h->order.p : nullptr;
   P.cta_done = grid <= 1024 ? h->cta_done.p : nullptr;
   CK(h, h->cs_tape.reserve((size_t)grid * (horizon + 2) * pc.NR));
   P.cs_tape = h->cs_tape;
@@ -652,131 +672,117 @@ static int prepare_launch(rbo_handle* h, const double* x0, const double* theta, 
   return RBO_SUCCESS;
 }
 
-// The rollout kernel of a prepared problem (the caller has cleared work_counter: the scheduler counter and the watchdog flags).
-static cudaError_t enqueue_rollout(const rbo_handle* h, const DevProblem& P, const PlanChoice& pc, int grid) {
-  if (pc.vglob) rbo_rollout_kernel_largen<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
-  else rbo_rollout_kernel<<<grid, RBO_THREADS, pc.bytes, h->stream>>>(P);
+// The rollout kernel of a prepared launch (the caller has cleared work_counter: the scheduler counter and the watchdog flags).
+static cudaError_t enqueue_rollout(const rbo_handle* h, const Launch& L) {
+  if (L.pc.vglob) rbo_rollout_kernel_largen<<<L.grid, RBO_THREADS, L.pc.bytes, h->stream>>>(L.P);
+  else rbo_rollout_kernel<<<L.grid, RBO_THREADS, L.pc.bytes, h->stream>>>(L.P);
   return cudaGetLastError();
 }
 
-// wd: the work_counter entries the rollout kernel's watchdog writes ([1], [2] flags; [4..8] where it waited)
-// handle >= 0: the index of the flagging handle among the handles of rbo_stochastic_solve_batch_sharded
+// wd: a work counter record or the SGA loop's sticky record; handle >= 0: the flagging handle's index in rbo_stochastic_solve_batch_sharded
 static int watchdog_fail(rbo_handle* h, const int* wd, int handle = -1) {
   char who[32] = "";
   if (handle >= 0) snprintf(who, sizeof(who), " on handle %d", handle);
   return fail(h, RBO_ERR_CUDA, "rollout kernel watchdog%s: %s%s (wait kind %d, chunk %d, warp %d, consumers %d, block %d)", who,
-              wd[1] ? "[panel pipeline wait never completed] " : "", wd[2] ? "[inner solve exceeded its evaluation bound]" : "", wd[4], wd[5],
-              wd[6], wd[7], wd[8]);
+              wd[WC_STALL] ? "[panel pipeline wait never completed] " : "", wd[WC_EVAL_CAP] ? "[inner solve exceeded its evaluation bound]" : "",
+              wd[WC_WAIT_KIND], wd[WC_WAIT_CHUNK], wd[WC_WAIT_WARP], wd[WC_WAIT_CONSUMERS], wd[WC_WAIT_BLOCK]);
 }
 
-static int launch_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
-                          double fmini, int mode, int flags, const double* dual_dirs_dev, const double* x_forced_dev, bool want_summary,
-                          rbo_summary* summary, const double* x0_batch_dev = nullptr, int B = 1) {
-  DevProblem P;
-  PlanChoice pc;
-  int grid = 0;
-  int rc = prepare_launch(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs_dev, x_forced_dev, x0_batch_dev, B, P, pc, grid);
-  if (rc) return rc;
-  flags = P.flags;
-  const bool myopic = (flags & RBO_FLAG_MYOPIC_INTERNAL) != 0;
-  const int M = P.M;
-  CK(h, cudaMemsetAsync(h->work_counter, 0, 16 * sizeof(int), h->stream));
-  CK(h, cudaEventRecord(h->ev0, h->stream));
-  CK(h, enqueue_rollout(h, P, pc, grid));
-  rbo_stats_kernel<<<1, 1024, 0, h->stream>>>(h->values, mode == RBO_MODE_VALUE_GRAD ? h->grad_x.p : nullptr, mode == RBO_MODE_VALUE_GRAD ? h->grad_theta.p : nullptr,
-                                              h->n_evals, h->best_index, h->grad_case, h->status, M, h->d, ntheta, horizon, h->sums);
-  CK(h, cudaGetLastError());
-  CK(h, cudaEventRecord(h->ev1, h->stream));
-  if (h->lpt && !myopic && horizon > 0 && M > 2 * grid && !(flags & RBO_FLAG_TEACHER_FORCED)) {
-    CK(h, h->order.reserve(M));
-    rbo_lpt_order_kernel<<<1, 1024, 0, h->stream>>>(h->n_evals, h->grad_case, h->best_index, M, std::max(horizon, 1), h->order);
-    CK(h, cudaGetLastError());
-    h->order_M = M;
-  } else if (!(flags & RBO_FLAG_TEACHER_FORCED)) h->order_M = 0;
-  h->last_mode = mode;
-  h->xs_valid = !myopic;
-  if (want_summary && summary) {
-    std::vector<double> sums(h->sums_len);
-    int wd[16] = {0};
-    std::vector<unsigned long long> td(grid);
-    CK(h, cudaMemcpyAsync(sums.data(), h->sums, (size_t)h->sums_len * 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(wd, h->work_counter, sizeof(wd), cudaMemcpyDeviceToHost, h->stream));
-    if (P.cta_done) CK(h, cudaMemcpyAsync(td.data(), h->cta_done, (size_t)grid * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaStreamSynchronize(h->stream));
-    if (wd[1] || wd[2]) return watchdog_fail(h, wd);
-    float ms = 0;
-    CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-    const int d = h->d, hh = std::max(horizon, 1), nrows = 1 + d + ntheta;
-    const double n = sums[0];
-    summary->n_traj = M;
-    summary->mean = n > 0 ? sums[1] / n : NAN;
-    summary->std = n > 1 ? std::sqrt(sums[2] / (n - 1)) : NAN;
-    summary->kernel_ms = ms;
-    summary->gpu_launches = 2 + (h->order_M == M ? 1 : 0);
-    summary->tail_ms = 0.0;
-    if (P.cta_done) {
-      std::sort(td.begin(), td.end());
-      summary->tail_ms = (double)(td.back() - td[grid / 2]) * 1e-6;  // last CTA to finish minus the median CTA
-    }
-    const double* ev = sums.data() + 1 + 3 * nrows;
-    const double* hist = ev + hh;
-    summary->n_failed = (int)hist[horizon + 2];
-    double fl = 0, fx = 0;
-    long long ne = 0;
-    if (myopic) {
-      ne = (long long)ev[0];
-      fl = ev[0] * f_eval(h->N, d);
-      fx = ev[0] * f_eval_exec(h->N, d);
-    } else {
-      fl = M * f_step(h->N, d); fx = M * f_step(h->N, d) * 0.5;
-      for (int j = 1; j <= horizon; ++j) {
-        double nj = h->N + j, e = ev[j - 1];
-        ne += (long long)e;
-        fl += e * f_eval(nj, d) + M * f_step(nj, d);
-        fx += e * f_eval_exec(nj, d) + M * f_step(nj, d) * 0.5;
-      }
-    }
-    if (mode == RBO_MODE_VALUE_GRAD)
-      for (int t = 1; t <= horizon; ++t) {  // F_adj(t) for the hist[t] trajectories whose best step is t (case 3)
-        double fa = t * (2.0 / 3.0) * d * d * d;
-        for (int i = 1; i <= t; ++i) { double ni = h->N + i; fa += f_eval(ni, d) + i * (d + 1) * (2 * ni * ni + 6 * ni * d); }
-        fl += hist[t] * fa;
-        fx += hist[t] * fa;
-      }
-    summary->flops = fl;
-    summary->flops_executed = fx;
-    summary->n_evals = ne;
+// Waits for a launch, checks the watchdog and fills the summary; flops: what the reference performs, flops_executed: what this does.
+static int fill_summary(rbo_handle* h, const Launch& L, rbo_summary* summary) {
+  const DevProblem& P = L.P;
+  const int d = h->d, M = P.M, horizon = P.h;
+  const StatsLayout SL(d, P.ntheta, horizon);
+  std::vector<double> sums(SL.len);
+  int wd[WC_LEN] = {0};
+  std::vector<unsigned long long> td(P.cta_done ? L.grid : 0);
+  CK(h, cudaMemcpyAsync(sums.data(), h->sums, sums.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaMemcpyAsync(wd, h->work_counter, sizeof(wd), cudaMemcpyDeviceToHost, h->stream));
+  if (P.cta_done) CK(h, cudaMemcpyAsync(td.data(), h->cta_done, td.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  if (wd[WC_STALL] || wd[WC_EVAL_CAP]) return watchdog_fail(h, wd);
+  float ms = 0;
+  CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  const double n = sums[0];
+  summary->n_traj = M;
+  summary->mean = n > 0 ? sums[1] / n : NAN;
+  summary->std = n > 1 ? std::sqrt(sums[2] / (n - 1)) : NAN;
+  summary->kernel_ms = ms;
+  summary->gpu_launches = 2 + L.lpt;  // rollout, statistics[, longest-first order]
+  summary->tail_ms = 0.0;
+  if (!td.empty()) {
+    std::sort(td.begin(), td.end());
+    summary->tail_ms = (double)(td.back() - td[td.size() / 2]) * 1e-6;  // last CTA to finish minus the median CTA
   }
+  const double *ev = sums.data() + SL.evals, *hist = sums.data() + SL.hist;
+  summary->n_failed = (int)sums[SL.failed];
+  double fl = 0, fx = 0;
+  long long ne = 0;
+  if (P.flags & RBO_FLAG_MYOPIC_INTERNAL) {
+    ne = (long long)ev[0];
+    fl = ev[0] * f_eval(h->N, d);
+    fx = ev[0] * f_eval_exec(h->N, d);
+  } else {
+    fl = M * f_step(h->N, d); fx = M * f_step(h->N, d) * 0.5;
+    for (int j = 1; j <= horizon; ++j) {
+      double nj = h->N + j, e = ev[j - 1];
+      ne += (long long)e;
+      fl += e * f_eval(nj, d) + M * f_step(nj, d);
+      fx += e * f_eval_exec(nj, d) + M * f_step(nj, d) * 0.5;
+    }
+  }
+  if (P.mode == RBO_MODE_VALUE_GRAD)
+    for (int t = 1; t <= horizon; ++t) {  // F_adj(t) for the hist[t] trajectories whose best step is t (case 3)
+      double fa = t * (2.0 / 3.0) * d * d * d;
+      for (int i = 1; i <= t; ++i) { double ni = h->N + i; fa += f_eval(ni, d) + i * (d + 1) * (2 * ni * ni + 6 * ni * d); }
+      fl += hist[t] * fa;
+      fx += hist[t] * fa;
+    }
+  summary->flops = fl;
+  summary->flops_executed = fx;
+  summary->n_evals = ne;
   return RBO_SUCCESS;
 }
 
-// rbo_rollout and rbo_rollout_batch: the launch on host inputs -- the dual directions (VALUE_GRAD), the forced x-path and, for a
-// batch, the B starting points x0_batch (d x B) are uploaded first -- and the per-trajectory results back to the host.
-static int rollout_host(rbo_handle* h, const double* x0, const double* x0_batch, int B, const double* theta, int ntheta, const double* lbs,
-                        const double* ubs, int horizon, double fmini, int mode, int flags, const double* dual_dirs, const double* x_forced,
-                        double* values, double* grad_x, double* grad_theta, int32_t* best_index, int32_t* grad_case, int32_t* status,
-                        rbo_summary* summary) {
-  const bool grad = mode == RBO_MODE_VALUE_GRAD;
-  const bool forced = (flags & RBO_FLAG_TEACHER_FORCED) && !(flags & RBO_FLAG_REPLAY_TAPE);
+// One rollout launch, its statistics and the longest-first order for the next launch; with a summary it also waits for them.
+static int launch_rollout(rbo_handle* h, const RolloutArgs& a, rbo_summary* summary) {
+  Launch L;
+  if (int rc = prepare_launch(h, a, L)) return rc;
+  const DevProblem& P = L.P;
+  const bool grad = a.mode == RBO_MODE_VALUE_GRAD;
+  CK(h, cudaMemsetAsync(h->work_counter, 0, WC_LEN * sizeof(int), h->stream));
+  CK(h, cudaEventRecord(h->ev0, h->stream));
+  CK(h, enqueue_rollout(h, L));
+  rbo_stats_kernel<<<1, 1024, 0, h->stream>>>(h->values, grad ? h->grad_x.p : nullptr, grad ? h->grad_theta.p : nullptr, h->n_evals, h->best_index,
+                                              h->grad_case, h->status, P.M, h->d, a.ntheta, P.h, h->sums);
+  CK(h, cudaGetLastError());
+  CK(h, cudaEventRecord(h->ev1, h->stream));
+  if (L.lpt) {
+    rbo_lpt_order_kernel<<<1, 1024, 0, h->stream>>>(h->n_evals, h->grad_case, h->best_index, P.M, P.h, h->order);
+    CK(h, cudaGetLastError());
+    h->order_M = P.M;
+  } else if (!(P.flags & RBO_FLAG_TEACHER_FORCED)) h->order_M = 0;  // a teacher-forced launch keeps the order of the free one
+  h->last.mode = a.mode;
+  h->last.xs = !(P.flags & RBO_FLAG_MYOPIC_INTERNAL);
+  return summary ? fill_summary(h, L, summary) : RBO_SUCCESS;
+}
+
+// rbo_rollout and rbo_rollout_batch: uploads a.dual_dirs, a.x_forced and a.x0_batch (host arrays here), launches, reads results back.
+static int rollout_host(rbo_handle* h, RolloutArgs a, double* values, double* grad_x, double* grad_theta, int32_t* best_index,
+                        int32_t* grad_case, int32_t* status, rbo_summary* summary) {
+  const bool grad = a.mode == RBO_MODE_VALUE_GRAD;
+  const bool forced = (a.flags & RBO_FLAG_TEACHER_FORCED) && !(a.flags & RBO_FLAG_REPLAY_TAPE);
   CK(h, cudaSetDevice(h->device));
-  const size_t Ms = (flags & RBO_FLAG_GAUSS_HERMITE) ? (size_t)h->gh_M : (size_t)h->M;
-  const size_t nd = Ms * std::max(horizon, 0) * h->d;
-  if (grad && dual_dirs) {
-    CK(h, h->dual_dirs.reserve(nd));
-    CK(h, cudaMemcpyAsync(h->dual_dirs, dual_dirs, nd * 8, cudaMemcpyHostToDevice, h->stream));
-  }
-  if (forced && x_forced) {
-    CK(h, h->x_forced.reserve(nd));
-    CK(h, cudaMemcpyAsync(h->x_forced, x_forced, nd * 8, cudaMemcpyHostToDevice, h->stream));
-  }
-  if (x0_batch) {
-    CK(h, h->x0_batch.reserve((size_t)B * h->d));
-    CK(h, cudaMemcpyAsync(h->x0_batch, x0_batch, (size_t)B * h->d * 8, cudaMemcpyHostToDevice, h->stream));
-  }
+  const size_t Ms = (a.flags & RBO_FLAG_GAUSS_HERMITE) ? (size_t)h->gh_M : (size_t)h->M;
+  const size_t nd = Ms * std::max(a.horizon, 0) * h->d;
+  if (grad && a.dual_dirs) CK(h, copy_in(h->dual_dirs, a.dual_dirs, nd, h->stream));
+  if (forced && a.x_forced) CK(h, copy_in(h->x_forced, a.x_forced, nd, h->stream));
+  if (a.x0_batch) CK(h, copy_in(h->x0_batch, a.x0_batch, (size_t)a.B * h->d, h->stream));
+  a.dual_dirs = (grad && a.dual_dirs) ? h->dual_dirs.p : nullptr;
+  a.x_forced = forced ? h->x_forced.p : nullptr;
+  a.x0_batch = a.x0_batch ? h->x0_batch.p : nullptr;
   rbo_summary local;
-  int rc = launch_rollout(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, (grad && dual_dirs) ? h->dual_dirs.p : nullptr,
-                          forced ? h->x_forced.p : nullptr, true, summary ? summary : &local, x0_batch ? h->x0_batch.p : nullptr, B);
-  if (rc) return rc;
+  if (int rc = launch_rollout(h, a, summary ? summary : &local)) return rc;
   return rbo_get_results(h, values, grad ? grad_x : nullptr, grad ? grad_theta : nullptr, best_index, grad_case, status);
 }
 
@@ -788,14 +794,14 @@ int rbo_rollout(rbo_handle* h, const double* x0, const double* theta, int ntheta
   if (!h) return RBO_ERR_ARG;
   if (!values) return fail(h, RBO_ERR_ARG, "rbo_rollout: values is NULL");
   if (mode == RBO_MODE_VALUE_GRAD && (!grad_x || !grad_theta)) return fail(h, RBO_ERR_ARG, "rbo_rollout: gradient containers missing in VALUE_GRAD mode");
-  return rollout_host(h, x0, nullptr, 1, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs, x_forced, values, grad_x, grad_theta,
-                      best_index, grad_case, status, summary);
+  return rollout_host(h, {x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs, x_forced}, values, grad_x, grad_theta, best_index,
+                      grad_case, status, summary);
 }
 
 int rbo_rollout_device(rbo_handle* h, const double* x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
                        double fmini, int mode, int flags, const double* dual_dirs_device, const double* x_forced_device, rbo_summary* summary) {
   if (!h) return RBO_ERR_ARG;
-  return launch_rollout(h, x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs_device, x_forced_device, summary != nullptr, summary);
+  return launch_rollout(h, {x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, flags, dual_dirs_device, x_forced_device}, summary);
 }
 
 int rbo_rollout_batch(rbo_handle* h, const double* x0s, int n_x0, const double* theta, int ntheta, const double* lbs, const double* ubs, int horizon,
@@ -805,7 +811,7 @@ int rbo_rollout_batch(rbo_handle* h, const double* x0s, int n_x0, const double* 
   if (!x0s || n_x0 < 1 || !values) return fail(h, RBO_ERR_ARG, "rbo_rollout_batch: bad arguments");
   if (mode == RBO_MODE_VALUE_GRAD && (!grad_x || !grad_theta)) return fail(h, RBO_ERR_ARG, "rbo_rollout_batch: gradient containers missing in VALUE_GRAD mode");
   if (!h->rn) return fail(h, RBO_ERR_STATE, "rbo_rollout_batch: no normals (rbo_set_normals / rbo_generate_normals)");
-  return rollout_host(h, x0s, x0s, n_x0, theta, ntheta, lbs, ubs, horizon, fmini, mode, 0, dual_dirs, nullptr, values, grad_x, grad_theta,
+  return rollout_host(h, {x0s, theta, ntheta, lbs, ubs, horizon, fmini, mode, 0, dual_dirs, nullptr, x0s, n_x0}, values, grad_x, grad_theta,
                       nullptr, nullptr, status, summary);
 }
 
@@ -874,35 +880,24 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
   }
 
   // every handle's launch is prepared before anything is enqueued: an error leaves every handle as it was
-  struct Shard {
-    DevProblem P;
-    PlanChoice pc;
-    int grid = 0, Ms = 0, m_begin = 0;
-    bool lpt = false;
-    const int* order = nullptr;
-  };
+  struct Shard { Launch L; int m_begin = 0; const int* order = nullptr; };  // order: what the next work list follows
   std::vector<Shard> sh(n);
   for (int i = 0; i < n; ++i) {
     rbo_handle* g = hs[i];
     Shard& s = sh[i];
-    s.Ms = g->M;
     s.m_begin = sharded ? g->m_begin : 0;
     CK(h, cudaSetDevice(g->device));
     CK(h, g->x0_batch.reserve((size_t)B * d));
-    if (dual_dirs) CK(h, g->dual_dirs.reserve((size_t)s.Ms * std::max(horizon, 0) * d));
-    int rc = prepare_launch(g, x0s, theta, ntheta, lbs, ubs, horizon, fmini, RBO_MODE_VALUE_GRAD, 0, dual_dirs ? g->dual_dirs.p : nullptr, nullptr,
-                            g->x0_batch.p, B, s.P, s.pc, s.grid);
-    if (rc) {
+    if (dual_dirs) CK(h, g->dual_dirs.reserve((size_t)g->M * std::max(horizon, 0) * d));
+    if (int rc = prepare_launch(g, {x0s, theta, ntheta, lbs, ubs, horizon, fmini, RBO_MODE_VALUE_GRAD, 0, dual_dirs ? g->dual_dirs.p : nullptr,
+                                    nullptr, g->x0_batch.p, B}, s.L)) {
       if (i > 0) h->err = std::string(me) + ": handle " + std::to_string(i) + ": " + g->err;
       return rc;
     }
-    // the conditions under which launch_rollout hands out longest-first; the order then follows the previous iteration's costs
-    s.lpt = g->lpt && horizon > 0 && s.P.M > 2 * s.grid;
-    if (s.lpt) CK(h, g->order.reserve(s.P.M));
-    s.order = s.P.order;
-    CK(h, g->worklist.reserve(s.P.M));
+    s.order = s.L.P.order;
+    CK(h, g->worklist.reserve(s.L.P.M));
     if (i > 0) CK(h, g->sga_int.reserve(B));  // live
-    s.P.order = g->worklist;
+    s.L.P.order = g->worklist;
   }
   if (sharded)  // peer access where the devices allow it (the copies below work without it, through the host)
     for (int i = 0; i < n; ++i)
@@ -917,17 +912,17 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
       }
 
   // leader state: doubles [m | v | bias | x_hist | gmean_hist | gstd_hist | mean_hist | std_hist], ints [live | n_iter | end_status |
-  // fail (2 per restart) | nfail | sticky watchdog record (16)]
+  // fail (2 per restart) | nfail | sticky watchdog record]
   CK(h, cudaSetDevice(h->device));
   const size_t nx = (size_t)d * B, nh = (size_t)maxit * B, nt = (size_t)B * Mt;
   const size_t o_bias = 2 * nx, o_xh = o_bias + 2 * (size_t)maxit, o_gmh = o_xh + nh * d, o_gsh = o_gmh + nh * d, o_mh = o_gsh + nh * d,
                o_sh = o_mh + nh, n_dbl = o_sh + nh;
-  const size_t i_iter = B, i_end = 2 * (size_t)B, i_fail = 3 * (size_t)B, i_nfail = 5 * (size_t)B, i_sticky = 6 * (size_t)B, n_int = i_sticky + 16;
+  const size_t i_iter = B, i_end = 2 * (size_t)B, i_fail = 3 * (size_t)B, i_nfail = 5 * (size_t)B, i_sticky = 6 * (size_t)B, n_int = i_sticky + WC_LEN;
   CK(h, h->sga_dbl.reserve(n_dbl));
   CK(h, h->sga_int.reserve(n_int));
   if (n > 1) {
     CK(h, h->sga_gather.reserve(nt * (1 + d)));  // values [B][Mt] | grad_x [B][Mt][d]
-    CK(h, h->sga_igather.reserve(nt + 16 * (size_t)n));  // status [B][Mt] | watchdog table [n][16]
+    CK(h, h->sga_igather.reserve(nt + WC_LEN * (size_t)n));  // status [B][Mt] | watchdog table [n][WC_LEN]
   }
   double* D = h->sga_dbl;
   int* I = h->sga_int;
@@ -948,7 +943,7 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
     CK(h, cudaMemcpyAsync(g->x0_batch, x0s, nx * 8, cudaMemcpyHostToDevice, g->stream));
     if (dual_dirs) {
       const size_t per = (size_t)std::max(horizon, 0) * d;  // dual_dirs[:, :, m] is contiguous: the shard is one block
-      CK(h, cudaMemcpyAsync(g->dual_dirs, dual_dirs + (size_t)sh[i].m_begin * per, (size_t)sh[i].Ms * per * 8, cudaMemcpyHostToDevice, g->stream));
+      CK(h, cudaMemcpyAsync(g->dual_dirs, dual_dirs + (size_t)sh[i].m_begin * per, (size_t)g->M * per * 8, cudaMemcpyHostToDevice, g->stream));
     }
     if (i > 0) CK(h, cudaMemcpyAsync(g->sga_int, ist.data(), (size_t)B * sizeof(int), cudaMemcpyHostToDevice, g->stream));
   }
@@ -985,10 +980,10 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
         CK(h, cudaMemcpyAsync(g->x0_batch, h->x0_batch, nx * 8, cudaMemcpyDefault, g->stream));
         CK(h, cudaMemcpyAsync(g->sga_int, h->sga_int, (size_t)B * sizeof(int), cudaMemcpyDefault, g->stream));
       }
-      rbo_sga_worklist_kernel<<<1, 1024, 0, g->stream>>>(s.order, g->sga_int, s.Ms, s.P.M, g->worklist);
+      rbo_sga_worklist_kernel<<<1, 1024, 0, g->stream>>>(s.order, g->sga_int, s.L.P.Ms, s.L.P.M, g->worklist);
       CK(h, cudaGetLastError());
-      CK(h, cudaMemsetAsync(g->work_counter, 0, 16 * sizeof(int), g->stream));
-      CK(h, enqueue_rollout(g, s.P, s.pc, s.grid));
+      CK(h, cudaMemsetAsync(g->work_counter, 0, WC_LEN * sizeof(int), g->stream));
+      CK(h, enqueue_rollout(g, s.L));
       launches += 2;
       if (n > 1) CK(h, cudaEventRecord(g->ev_rollout, g->stream));
     }
@@ -999,12 +994,12 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
       int* gs = h->sga_igather;
       for (int i = 0; i < n; ++i) {  // shard i at global sample m_begin of every restart
         const rbo_handle* g = hs[i];
-        const size_t Ms = sh[i].Ms, m0 = sh[i].m_begin;
+        const size_t Ms = sh[i].L.P.Ms, m0 = sh[i].m_begin;
         if (i > 0) CK(h, cudaStreamWaitEvent(h->stream, g->ev_rollout, 0));
         CK(h, cudaMemcpy2DAsync(gv + m0, Mt * 8, g->values, Ms * 8, Ms * 8, B, cudaMemcpyDefault, h->stream));
         CK(h, cudaMemcpy2DAsync(gg + m0 * d, Mt * d * 8, g->grad_x, Ms * d * 8, Ms * d * 8, B, cudaMemcpyDefault, h->stream));
         CK(h, cudaMemcpy2DAsync(gs + m0, Mt * sizeof(int), g->status, Ms * sizeof(int), Ms * sizeof(int), B, cudaMemcpyDefault, h->stream));
-        CK(h, cudaMemcpyAsync(gs + nt + 16 * i, g->work_counter, 16 * sizeof(int), cudaMemcpyDefault, h->stream));
+        CK(h, cudaMemcpyAsync(gs + nt + WC_LEN * i, g->work_counter, WC_LEN * sizeof(int), cudaMemcpyDefault, h->stream));
       }
     }
     rbo_sga_step_kernel<<<B, 256, 0, h->stream>>>(S, k);
@@ -1014,9 +1009,9 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
     for (int i = 0; i < n; ++i) {
       rbo_handle* g = hs[i];
       Shard& s = sh[i];
-      if (!s.lpt) continue;
+      if (!s.L.lpt) continue;
       CK(h, cudaSetDevice(g->device));
-      rbo_lpt_order_kernel<<<1, 1024, 0, g->stream>>>(g->n_evals, g->grad_case, g->best_index, s.P.M, horizon, g->order);
+      rbo_lpt_order_kernel<<<1, 1024, 0, g->stream>>>(g->n_evals, g->grad_case, g->best_index, s.L.P.M, horizon, g->order);
       CK(h, cudaGetLastError());
       s.order = g->order;
       ++launches;
@@ -1024,12 +1019,9 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
   }
   CK(h, cudaSetDevice(h->device));
   CK(h, cudaEventRecord(h->ev1, h->stream));
-  for (int i = 0; i < n; ++i) {
-    rbo_handle* g = hs[i];
-    g->order_M = sh[i].lpt ? sh[i].P.M : 0;
-    g->last_mode = RBO_MODE_VALUE_GRAD;
-    // the per-trajectory buffers now hold each restart's last iteration: no read-back and no replay until the next rollout
-    g->outM = 0; g->outh = -1; g->xs_valid = false;
+  for (int i = 0; i < n; ++i) {  // the outputs hold each restart's last iteration: no read-back and no replay until the next rollout
+    hs[i]->order_M = sh[i].L.lpt ? sh[i].L.P.M : 0;
+    hs[i]->last.reset();
   }
 
   std::vector<int> ires(n_int);
@@ -1047,7 +1039,8 @@ static int sga_solve(rbo_handle* const* hs, int n, bool sharded, const rbo_sga_o
   std::memcpy(n_iter, ires.data() + i_iter, (size_t)B * sizeof(int));
   std::memcpy(end_status, ires.data() + i_end, (size_t)B * sizeof(int));
   if (fail_out) std::memcpy(fail_out, ires.data() + i_fail, 2 * (size_t)B * sizeof(int));
-  if (ires[i_sticky]) return watchdog_fail(h, ires.data() + i_sticky, sharded ? ires[i_sticky + 9] : -1);
+  const int* sticky = ires.data() + i_sticky;
+  if (sticky[WC_STICKY_SEEN]) return watchdog_fail(h, sticky, sharded ? sticky[WC_STICKY_HANDLE] : -1);
   if (summary) {
     float ms = 0;
     CK(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1088,38 +1081,38 @@ int rbo_stochastic_solve_batch_sharded(rbo_handle* const* hs, int n_handles, con
 
 int rbo_partial_sums_device(rbo_handle* h, double* sums_device, int len) {
   if (!h || !sums_device) return RBO_ERR_ARG;
-  const int need = 1 + 3 * (1 + h->outd + h->outnth);
-  if (!h->sums || len < need + 2) return fail(h, RBO_ERR_ARG, "rbo_partial_sums_device: need %d doubles (1 + 3 (1 + d + ntheta) + 2)", need + 2);
+  const LastLaunch& o = h->last;
+  if (!o.valid()) return fail(h, RBO_ERR_STATE, "rbo_partial_sums: no rollout since the handle was created or its last SGA loop");
+  const StatsLayout L(o.d, o.nth, o.h);
+  if (len < L.gathered) return fail(h, RBO_ERR_ARG, "rbo_partial_sums: need %d doubles (1 + 3 (1 + d + ntheta) + 2)", L.gathered);
   CK(h, cudaSetDevice(h->device));
-  const int hh = std::max(h->outh, 1);
-  const int idx_failed = need + hh + (h->outh + 2);  // sums layout of rbo_stats_kernel: rows, evaluations per step, case-3 histogram, failures
-  rbo_gather_sums_kernel<<<1, 64, 0, h->stream>>>(h->sums, need, idx_failed, h->work_counter, sums_device);
+  rbo_gather_sums_kernel<<<1, 64, 0, h->stream>>>(h->sums, L, h->work_counter, sums_device);
   CK(h, cudaGetLastError());
   return RBO_SUCCESS;
 }
 
 int rbo_partial_sums_host(rbo_handle* h, double* sums, int len) {
   if (!h || !sums) return RBO_ERR_ARG;
-  const int need = 1 + 3 * (1 + h->outd + h->outnth) + 2;
-  if (!h->sums || len < need) return fail(h, RBO_ERR_ARG, "rbo_partial_sums_host: need %d doubles (1 + 3 (1 + d + ntheta) + 2)", need);
-  CK(h, cudaSetDevice(h->device));
-  double* tmp = h->sums + h->sums_len;  // the sums buffer is allocated with room for the gathered vector
-  int rc = rbo_partial_sums_device(h, tmp, need);
-  if (rc) return rc;
-  CK(h, cudaMemcpyAsync(sums, tmp, (size_t)need * 8, cudaMemcpyDeviceToHost, h->stream));
+  const LastLaunch& o = h->last;
+  if (!o.valid()) return fail(h, RBO_ERR_STATE, "rbo_partial_sums: no rollout since the handle was created or its last SGA loop");
+  const StatsLayout L(o.d, o.nth, o.h);
+  double* tmp = h->sums + L.len;  // the sums buffer is allocated with room for the gathered vector
+  if (int rc = rbo_partial_sums_device(h, tmp, len)) return rc;
+  CK(h, cudaMemcpyAsync(sums, tmp, (size_t)L.gathered * 8, cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));  // this is the call that waits for the (asynchronous) rbo_rollout_device of this handle
   return RBO_SUCCESS;
 }
 
 int rbo_get_results(rbo_handle* h, double* values, double* grad_x, double* grad_theta, int32_t* best_index, int32_t* grad_case, int32_t* status) {
   if (!h) return RBO_ERR_ARG;
-  if (h->outh < 0 || h->outM <= 0) return fail(h, RBO_ERR_STATE, "rbo_get_results: no rollout has run");
-  if ((grad_x || grad_theta) && h->last_mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_STATE, "rbo_get_results: the last rollout computed no gradients");
+  const LastLaunch& o = h->last;
+  if (!o.valid()) return fail(h, RBO_ERR_STATE, "rbo_get_results: no rollout has run");
+  if ((grad_x || grad_theta) && o.mode != RBO_MODE_VALUE_GRAD) return fail(h, RBO_ERR_STATE, "rbo_get_results: the last rollout computed no gradients");
   CK(h, cudaSetDevice(h->device));
-  const size_t M = h->outM;
+  const size_t M = o.M;
   CK(h, copy_out(values, h->values, M, h->stream));
-  CK(h, copy_out(grad_x, h->grad_x, M * h->outd, h->stream));
-  CK(h, copy_out(grad_theta, h->grad_theta, M * h->outnth, h->stream));
+  CK(h, copy_out(grad_x, h->grad_x, M * o.d, h->stream));
+  CK(h, copy_out(grad_theta, h->grad_theta, M * o.nth, h->stream));
   CK(h, copy_out(best_index, h->best_index, M, h->stream));
   CK(h, copy_out(grad_case, h->grad_case, M, h->stream));
   CK(h, copy_out(status, h->status, M, h->stream));
@@ -1130,7 +1123,7 @@ int rbo_get_results(rbo_handle* h, double* values, double* grad_x, double* grad_
 int rbo_finalize_sums(const double* sums, int d, int ntheta, double* mean, double* std_, double* gx_mean, double* gx_std, double* gth_mean, double* gth_std) {
   if (!sums) return RBO_ERR_ARG;
   const double n = sums[0];
-  const int need = 1 + 3 * (1 + d + ntheta);
+  const int need = StatsLayout(d, ntheta, 0).rows;  // the row block does not depend on the horizon
   // a failed trajectory (where the reference would have thrown) or a kernel watchdog flag on ANY rank poisons the estimate
   if (sums[need] > 0.0 || sums[need + 1] > 0.0) return RBO_ERR_NUMERIC;
   if (!(n > 0)) return RBO_ERR_ARG;
@@ -1149,9 +1142,10 @@ int rbo_finalize_sums(const double* sums, int d, int ntheta, double* mean, doubl
 
 int rbo_get_tape(rbo_handle* h, double* xs, double* ys, double* gys, double* alphas, int32_t* n_evals, int32_t* start_status, int32_t* start_iters) {
   if (!h) return RBO_ERR_ARG;
-  if (h->outh < 0) return fail(h, RBO_ERR_STATE, "rbo_get_tape: no rollout has run");
+  const LastLaunch& o = h->last;
+  if (!o.valid()) return fail(h, RBO_ERR_STATE, "rbo_get_tape: no rollout has run");
   CK(h, cudaSetDevice(h->device));
-  const size_t M = h->outM, hor = h->outh, hh = std::max(h->outh, 1), d = h->outd, S = h->outS;
+  const size_t M = o.M, hor = o.h, hh = std::max(o.h, 1), d = o.d, S = o.S;
   CK(h, copy_out(xs, h->xs, M * (hor + 1) * d, h->stream));
   CK(h, copy_out(ys, h->ys, M * (hor + 1), h->stream));
   CK(h, copy_out(gys, h->gys, M * (hor + 1) * d, h->stream));
@@ -1165,9 +1159,10 @@ int rbo_get_tape(rbo_handle* h, double* xs, double* ys, double* gys, double* alp
 
 extern "C" int rbo_get_tape_ex(rbo_handle* h, double* mu, double* sigma, double* dmu, double* dsigma, double* Halpha) {
   if (!h) return RBO_ERR_ARG;
-  if (!h->tex_valid) return fail(h, RBO_ERR_STATE, "rbo_get_tape_ex: the last rollout did not run with RBO_FLAG_TAPE_EX");
+  const LastLaunch& o = h->last;
+  if (!o.valid() || !o.tape_ex) return fail(h, RBO_ERR_STATE, "rbo_get_tape_ex: the last rollout did not run with RBO_FLAG_TAPE_EX");
   CK(h, cudaSetDevice(h->device));
-  const size_t n = (size_t)h->outM * std::max(h->outh, 0), d = h->outd;
+  const size_t n = (size_t)o.M * o.h, d = o.d;
   CK(h, copy_out(mu, h->t_mu, n, h->stream));
   CK(h, copy_out(sigma, h->t_sigma, n, h->stream));
   CK(h, copy_out(dmu, h->t_dmu, n * d, h->stream));
@@ -1221,8 +1216,7 @@ int rbo_multistart_base_solve(rbo_handle* h, const double* theta, int ntheta, co
   if (!h->have_sur) return fail(h, RBO_ERR_STATE, "rbo_multistart_base_solve: no surrogate");
   double x0[RBO_MAXD] = {0};
   rbo_summary local;
-  int rc = launch_rollout(h, x0, theta, ntheta, lbs, ubs, 0, 0.0, RBO_MODE_VALUE, RBO_FLAG_MYOPIC_INTERNAL, nullptr, nullptr, true, summary ? summary : &local);
-  if (rc) return rc;
+  if (int rc = launch_rollout(h, {x0, theta, ntheta, lbs, ubs, 0, 0.0, RBO_MODE_VALUE, RBO_FLAG_MYOPIC_INTERNAL}, summary ? summary : &local)) return rc;
   double a = 0;
   int st = 0;
   CK(h, cudaMemcpyAsync(xfinal, h->xs, (size_t)h->d * 8, cudaMemcpyDeviceToHost, h->stream));
@@ -1235,8 +1229,6 @@ int rbo_multistart_base_solve(rbo_handle* h, const double* theta, int ntheta, co
 }
 
 int rbo_num_sms(const rbo_handle* h) { return h ? h->num_sms : 0; }
-
-
 
 int rbo_fp64_peak(rbo_handle* h, double* tflops) {
   if (!h || !tflops) return RBO_ERR_ARG;
@@ -1265,14 +1257,11 @@ int rbo_tr_step_batch(rbo_handle* h, int n, int B, const double* H, const double
   CK(h, cudaSetDevice(h->device));
   DevBuf<double> dH, dg, dD, dp;
   DevBuf<int> dh;
-  CK(h, dH.reserve((size_t)B * n * n));
-  CK(h, dg.reserve((size_t)B * n));
-  CK(h, dD.reserve(B));
+  CK(h, copy_in(dH, H, (size_t)B * n * n, h->stream));
+  CK(h, copy_in(dg, g, (size_t)B * n, h->stream));
+  CK(h, copy_in(dD, Delta, B, h->stream));
   CK(h, dp.reserve((size_t)B * n));
   CK(h, dh.reserve(B));
-  CK(h, cudaMemcpyAsync(dH, H, (size_t)B * n * n * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(h, cudaMemcpyAsync(dg, g, (size_t)B * n * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(h, cudaMemcpyAsync(dD, Delta, (size_t)B * 8, cudaMemcpyHostToDevice, h->stream));
   const int wpb = n > 16 ? 2 : 4;  // <= 48 KB of dynamic shared memory
   const size_t smem = (size_t)wpb * (2 * n * n + 4 * n + 32) * 8;
   rbo_tr_step_kernel<<<(B + wpb - 1) / wpb, 32 * wpb, smem, h->stream>>>(dH, dg, dD, n, B, dp, dh);

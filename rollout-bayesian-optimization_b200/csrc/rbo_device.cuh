@@ -22,6 +22,15 @@
 
 namespace rbo {
 
+// DevProblem::work_counter, cleared before every rollout launch; the SGA loop's sticky record keeps the same indices.
+enum WorkCounterIndex : int {
+  WC_SCHED = 0,                  // next entry of the hand-out order
+  WC_STALL = 1, WC_EVAL_CAP = 2,  // flags: a panel pipeline wait never completed; an inner solve exceeded its evaluation bound
+  WC_WAIT_KIND = 4, WC_WAIT_CHUNK, WC_WAIT_WARP, WC_WAIT_CONSUMERS, WC_WAIT_BLOCK,  // the stalled wait
+  WC_STICKY_SEEN = 0, WC_STICKY_HANDLE = 9,  // sticky record: a flag was seen in some iteration; the index of the flagging handle
+  WC_LEN = 16
+};
+
 struct KernelSpec {
   int id;
   double th[4];
@@ -182,7 +191,5 @@ __device__ inline void lu_solve(const double* A, int n, const int* piv, double* 
     b[i] /= A[i * n + i];
   }
 }
-
-__device__ inline double shfl_xor_d(double v, int off) { return __shfl_xor_sync(0xffffffffu, v, off); }
 
 }  // namespace rbo

@@ -75,7 +75,7 @@ struct DevProblem {
   int* start_status;   // [M][h][S]
   int* start_iters;    // [M][h][S]
   double *t_mu, *t_sigma, *t_dmu, *t_dsigma, *t_Halpha;  // extended tape (RBO_FLAG_TAPE_EX): [M][h], [M][h], [M][h][d], [M][h][d], [M][h][d*d]
-  int* work_counter;   // dynamic trajectory scheduler
+  int* work_counter;   // the work counter record: scheduler and watchdog (WorkCounterIndex)
   const int* order;    // [M] trajectories in the order they are handed out (longest first, from the previous launch) or nullptr
   unsigned long long* cta_done;  // [gridDim.x] %globaltimer at the end of each CTA (tail of the persistent grid)
   double* cs_tape;     // [gridDim.x][h+2][NR] coefficient tape of the trajectory each CTA is working on

@@ -595,8 +595,9 @@ RBO_ROW_UNROLL
           "selp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(mb), "r"(parity) : "memory");
       if (ok) return;
     }
-    if (atomicExch(P.work_counter + 1, 1) == 0) {
-      P.work_counter[4] = 2; P.work_counter[5] = (int)q; P.work_counter[6] = warp; P.work_counter[7] = RBO_NCONS; P.work_counter[8] = blockIdx.x;
+    if (atomicExch(P.work_counter + WC_STALL, 1) == 0) {
+      P.work_counter[WC_WAIT_KIND] = 2; P.work_counter[WC_WAIT_CHUNK] = (int)q; P.work_counter[WC_WAIT_WARP] = warp;
+      P.work_counter[WC_WAIT_CONSUMERS] = RBO_NCONS; P.work_counter[WC_WAIT_BLOCK] = blockIdx.x;
     }
   }
   __device__ __forceinline__ void empty_arrive(unsigned q) {
@@ -1087,7 +1088,7 @@ RBO_ROW_UNROLL
     const long long round_cap = (long long)P.S * (P.so.maxit + 2) * (P.so.maxtry + 2);  // no start can use more evaluations than that
     long long rounds_ = 0;
     while (nact > 0) {
-      if (++rounds_ > round_cap) { if (tid == 0) P.work_counter[2] = 1; break; }
+      if (++rounds_ > round_cap) { if (tid == 0) P.work_counter[WC_EVAL_CAP] = 1; break; }
       auto pt = [&](int s) { return (const double*)(sm + pl.sxt + alist[s] * d); };
       auto cb = [&](int s) { return alist[s] * P.CS; };
       PT_MARK(9);
@@ -1310,7 +1311,7 @@ __global__ void __launch_bounds__(RBO_THREADS, 1) RBO_KERNEL_NAME(const __grid_c
     if (tid == 0) {
       // dynamic scheduler; with an order from the previous launch the trajectories are handed out longest-first (LPT), which
       // shortens the tail of the persistent grid -- the per-trajectory results do not depend on the order
-      const int i = atomicAdd(P.work_counter, 1);
+      const int i = atomicAdd(P.work_counter + WC_SCHED, 1);
       si[I_M] = (i < P.M) ? (P.order ? P.order[i] : i) : P.M;
     }
     __syncthreads();

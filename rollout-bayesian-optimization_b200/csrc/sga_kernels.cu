@@ -70,17 +70,17 @@ __global__ void __launch_bounds__(SGA_THREADS) rbo_sga_step_kernel(const __grid_
   __shared__ double s_mean[RBO_MAXD + 1], s_std[RBO_MAXD + 1];
   __shared__ double s_bc;
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  // kernel watchdog: the memset before each rollout launch clears work_counter[1..2]; a flag seen once, on any handle, stops every restart
+  // kernel watchdog: the memset before each rollout launch clears both flags; a flag seen once, on any handle, stops every restart
   int flagged = -1;
   for (int i = 0; i < S.n_watchdog && flagged < 0; ++i)
-    if (S.watchdog[16 * i + 1] != 0 || S.watchdog[16 * i + 2] != 0) flagged = i;
-  if (S.sticky[0] != 0 || flagged >= 0) {
+    if (S.watchdog[WC_LEN * i + WC_STALL] != 0 || S.watchdog[WC_LEN * i + WC_EVAL_CAP] != 0) flagged = i;
+  if (S.sticky[WC_STICKY_SEEN] != 0 || flagged >= 0) {
     if (tid == 0) {
-      if (b == 0 && S.sticky[0] == 0) {
-        const int* wc = S.watchdog + 16 * flagged;
-        for (int i = 1; i <= 8; ++i) S.sticky[i] = wc[i];
-        S.sticky[9] = flagged;
-        S.sticky[0] = 1;
+      if (b == 0 && S.sticky[WC_STICKY_SEEN] == 0) {
+        const int* wc = S.watchdog + WC_LEN * flagged;
+        for (int i = WC_STALL; i <= WC_WAIT_BLOCK; ++i) S.sticky[i] = wc[i];
+        S.sticky[WC_STICKY_HANDLE] = flagged;
+        S.sticky[WC_STICKY_SEEN] = 1;
       }
       S.live[b] = 0;
     }

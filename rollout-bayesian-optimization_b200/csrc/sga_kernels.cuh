@@ -16,7 +16,7 @@ struct SgaProblem {
   const double* values;         // [B * Ms]
   const double* grad_x;         // [B * Ms][d]
   const int* status;            // [B * Ms]
-  const int* watchdog;          // [n_watchdog][16]: each handle's work_counter ([1..8]: the rollout kernel's watchdog flags and details)
+  const int* watchdog;          // [n_watchdog][WC_LEN]: each handle's work counter record (WorkCounterIndex)
   int n_watchdog;
   // optimiser state
   double* x;                    // [B][d] current iterates (the x0_batch the rollout kernel reads)
@@ -29,8 +29,7 @@ struct SgaProblem {
   int* end_status;              // [B] RBO_SGA_*
   int* fail;                    // [B][2] first failing sample, its RBO_TRAJ_* status
   int* nfail;                   // [B] failed trajectories at the last evaluation
-  int* sticky;                  // [16]: [0] a watchdog flag was seen in some iteration, [1..8] the work_counter entries then, [9] the
-                                //       index of the handle whose flag it was
+  int* sticky;                  // [WC_LEN]: WC_STICKY_SEEN, the flagging handle's record from WC_STALL to WC_WAIT_BLOCK, WC_STICKY_HANDLE
 };
 
 __global__ void rbo_sga_worklist_kernel(const int* order, const int* live, int Ms, int M, int* list);

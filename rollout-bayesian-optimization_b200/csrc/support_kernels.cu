@@ -53,16 +53,15 @@ __global__ void rbo_sobol_kernel(const unsigned* __restrict__ dirs, unsigned* __
   }
 }
 
-// Per-handle statistics of the last rollout: sums[0] = n, then [n*mean, M2, n*mean^2] for the value and every gradient
-// row (two-pass: mean first, then centred squares -- rollout.jl:328-337), then the acquisition evaluations per step
-// (max(h,1) entries), then a histogram over t = 0..h of the case-3 trajectories, then the number of failed trajectories.
-// One CTA; M is at most a few 10^5.
+// Per-handle statistics of the last rollout, laid out as StatsLayout says (the rows two-pass: mean first, then centred squares --
+// rollout.jl:328-337). One CTA; M is at most a few 10^5.
 __global__ void rbo_stats_kernel(const double* __restrict__ values, const double* __restrict__ gx, const double* __restrict__ gth,
                                  const int* __restrict__ n_evals, const int* __restrict__ best_index, const int* __restrict__ grad_case,
                                  const int* __restrict__ status, int M, int d, int nth, int h, double* __restrict__ sums) {
   __shared__ double red[32];
   __shared__ double s_mean;
   const int nrows = 1 + d + nth, nw = blockDim.x >> 5;
+  const StatsLayout L(d, nth, h);
   auto block_sum = [&](double acc) -> double {
     for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
     __syncthreads();
@@ -103,23 +102,20 @@ __global__ void rbo_stats_kernel(const double* __restrict__ values, const double
       sums[1 + 3 * row + 2] = nok * mean * mean;
     }
   }
-  const int hh = h > 1 ? h : 1;
-  double* ev = sums + 1 + 3 * nrows;
-  for (int j = 0; j < hh; ++j) {
+  for (int j = 0; j < L.hist - L.evals; ++j) {
     double acc = 0.0;
     if (n_evals && h > 0) for (int i = threadIdx.x; i < M; i += blockDim.x) acc += n_evals[(size_t)i * h + j];
     double tot = block_sum(acc);
-    if (threadIdx.x == 0) ev[j] = tot;
+    if (threadIdx.x == 0) sums[L.evals + j] = tot;
   }
-  double* hist = ev + hh;
-  for (int t = 0; t <= h + 1; ++t) {
+  for (int t = 0; t <= h + 1; ++t) {  // t = h + 1: the failed trajectories
     double acc = 0.0;
     for (int i = threadIdx.x; i < M; i += blockDim.x) {
       if (t <= h) acc += (grad_case && best_index && grad_case[i] == 3 && best_index[i] == t) ? 1.0 : 0.0;
       else acc += (status && status[i] != 0) ? 1.0 : 0.0;
     }
     double tot = block_sum(acc);
-    if (threadIdx.x == 0) hist[t + (t > h ? 1 : 0)] = tot;
+    if (threadIdx.x == 0) sums[t <= h ? L.hist + t : L.failed] = tot;
   }
 }
 
@@ -155,10 +151,10 @@ __global__ void rbo_lpt_order_kernel(const int* __restrict__ n_evals, const int*
   for (int m = threadIdx.x; m < M; m += blockDim.x) order[atomicAdd(&hist[(int)(cost(m) * scale)], 1)] = m;
 }
 
-// out = [sums[0 .. need), number of failed trajectories, kernel watchdog flag]: the vector the multi-GPU all-reduce sums
-__global__ void rbo_gather_sums_kernel(const double* __restrict__ sums, int need, int idx_failed, const int* __restrict__ work_counter, double* __restrict__ out) {
-  for (int i = threadIdx.x; i < need; i += blockDim.x) out[i] = sums[i];
-  if (threadIdx.x == 0) { out[need] = sums[idx_failed]; out[need + 1] = (work_counter[1] || work_counter[2]) ? 1.0 : 0.0; }
+// out = [the row block, number of failed trajectories, kernel watchdog flag]: the vector the multi-GPU all-reduce sums
+__global__ void rbo_gather_sums_kernel(const double* __restrict__ sums, StatsLayout L, const int* __restrict__ work_counter, double* __restrict__ out) {
+  for (int i = threadIdx.x; i < L.rows; i += blockDim.x) out[i] = sums[i];
+  if (threadIdx.x == 0) { out[L.rows] = sums[L.failed]; out[L.rows + 1] = (work_counter[WC_STALL] || work_counter[WC_EVAL_CAP]) ? 1.0 : 0.0; }
 }
 
 // Diagnostic (rbo_tr_step_batch): the device code of the per-start trust-region step on B independent subproblems, one warp each,

@@ -742,11 +742,14 @@ def test_failed_trajectories_poison_the_device_resident_estimate(pkg, orc):
     sur, P, rn, starts, dd, lbs, ubs, x0 = custom_case(pkg, orc, d, N, h, M, S, "Matern12", (0.6,), "EI", (0.01,))
     eng = pkg.RolloutEngine(0)
     try:
-        eng.set_surrogate(pkg.FantasySurrogate(sur, h)); eng.set_normals(rn); eng.set_starts(starts)
-        eng.rollout_device(x0, np.array([0.01]), lbs, ubs, h, float(np.min(sur.y)), 0)
         import torch
         nsum = 1 + 3 * (1 + d + 1) + 2
         sums = torch.zeros(nsum, dtype=torch.float64, device="cuda:0")
+        # before any rollout there are no statistics to gather: RBO_ERR_STATE
+        assert eng.lib.rbo_partial_sums_device(eng.handle.h, C.c_void_p(sums.data_ptr()), nsum) == -3
+        assert eng.lib.rbo_partial_sums_host(eng.handle.h, np.zeros(nsum).ctypes.data_as(C.POINTER(C.c_double)), nsum) == -3
+        eng.set_surrogate(pkg.FantasySurrogate(sur, h)); eng.set_normals(rn); eng.set_starts(starts)
+        eng.rollout_device(x0, np.array([0.01]), lbs, ubs, h, float(np.min(sur.y)), 0)
         eng.handle.check(eng.lib.rbo_partial_sums_device(eng.handle.h, C.c_void_p(sums.data_ptr()), nsum))
         torch.cuda.synchronize()
         host = sums.cpu().numpy()
@@ -828,7 +831,8 @@ def test_two_phase_call_reproduces_the_reference_rng_consumption(pkg, orc):
 
 def test_longest_first_schedule_does_not_change_results(pkg, orc):
     """RBO_TUNE_LPT: the second launch on the same samples hands the trajectories out longest-first (evaluation counts of the previous
-    launch). Scheduling only: per-trajectory results are bitwise those of the natural order; the tail metric is reported."""
+    launch). Scheduling only: per-trajectory results are bitwise those of the natural order; the tail metric is reported. A replay of
+    the path (teacher-forced) neither uses nor records an order, and its summary counts the two kernels that ran."""
     wl, sur, rn, starts, dd = setup(pkg, orc, "C2", M=600, S=6)
     outs = []
     for lpt in (False, True):
@@ -839,10 +843,15 @@ def test_longest_first_schedule_does_not_change_results(pkg, orc):
             for rep in range(2):  # the second launch uses the order computed by the first
                 v, gx, gt = np.zeros(wl.M), np.zeros((wl.d, wl.M), order="F"), np.zeros((1, wl.M), order="F")
                 s = eng.rollout(wl.x0, wl.theta, wl.lbs, wl.ubs, wl.h, float(np.min(sur.y)), v, gx, gt, dual_dirs=dd)
-            outs.append((v, gx, s.tail_ms, s.kernel_ms))
+            assert s.gpu_launches == (3 if lpt else 2)  # rollout, statistics[, longest-first order]
+            vr, gxr, gtr = np.zeros(wl.M), np.zeros((wl.d, wl.M), order="F"), np.zeros((1, wl.M), order="F")
+            sr = eng.rollout(wl.x0, wl.theta, wl.lbs, wl.ubs, wl.h, float(np.min(sur.y)), vr, gxr, gtr, dual_dirs=dd, replay=True)
+            assert sr.gpu_launches == 2
+            outs.append((v, gx, s.tail_ms, s.kernel_ms, vr, gxr))
         finally:
             eng.close()
     assert np.array_equal(outs[0][0], outs[1][0]) and np.array_equal(outs[0][1], outs[1][1])
+    assert np.array_equal(outs[0][4], outs[1][4]) and np.array_equal(outs[0][5], outs[1][5])
     assert outs[0][2] >= 0.0 and outs[1][2] >= 0.0 and outs[1][2] < outs[1][3]
 
 

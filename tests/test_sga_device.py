@@ -202,16 +202,26 @@ def test_failure_is_reported_never_averaged(pkg, orc):
 
 @pytest.mark.gpu
 def test_handle_state_after_the_loop(pkg, orc):
-    """Afterwards rollout / rollout_batch equal a fresh handle bitwise; RBO_FLAG_REPLAY_TAPE is refused (the last launch did not run every
-    restart); the large-n variant agrees with the shared-memory one."""
+    """Afterwards rollout / rollout_batch equal a fresh handle bitwise; RBO_FLAG_REPLAY_TAPE and the partial sums are refused (the last
+    launch did not run every restart, and no statistics ran over it); the large-n variant agrees with the shared-memory one."""
+    import torch
     wl, sur, rn, starts, dd = c2_case(pkg, orc)
     M, d, fmini = wl.M, wl.d, float(np.min(sur.y))
+    nsum = 1 + 3 * (1 + d + 1) + 2
+
+    def partial_sums(e):
+        host, dev = np.zeros(nsum), torch.zeros(nsum, dtype=torch.float64, device="cuda:0")
+        rc = (e.lib.rbo_partial_sums_host(e.handle.h, pkg._lib.dptr(host), nsum), e.lib.rbo_partial_sums_device(e.handle.h, C.c_void_p(dev.data_ptr()), nsum))
+        torch.cuda.synchronize()
+        return rc, host, dev.cpu().numpy()
+
     x0s = random_starts(wl, 3, 5)
     eng = engine(pkg, wl.h, sur, rn, starts)
     fresh = engine(pkg, wl.h, sur, rn, starts)
     big = engine(pkg, wl.h, sur, rn, starts, tuning=dict(large_n=True))
     try:
         r = solve(eng, wl, sur, x0s, dd, max_iterations=6, use_eswavs=False)
+        assert partial_sums(eng)[0] == (-3, -3)  # RBO_ERR_STATE
         with pytest.raises(pkg.RboError, match=r"librbo error -3"):  # RBO_ERR_STATE
             eng.rollout(wl.x0, wl.theta, wl.lbs, wl.ubs, wl.h, fmini, np.zeros(M), np.zeros((d, M), order="F"), np.zeros((1, M), order="F"),
                         dual_dirs=dd, replay=True)
@@ -222,6 +232,8 @@ def test_handle_state_after_the_loop(pkg, orc):
             e.rollout(wl.x0, wl.theta, wl.lbs, wl.ubs, wl.h, fmini, out["v"], out["gx"], out["gt"], dual_dirs=dd, status=out["st"],
                       best_index=out["bi"])
             out.update(e.tape(wl.h))
+            rc, out["sums_host"], out["sums_device"] = partial_sums(e)
+            assert rc == (0, 0)
             e.rollout_batch(r["x_final"], wl.theta, wl.lbs, wl.ubs, wl.h, fmini, out["vb"], out["gxb"], out["gtb"], dual_dirs=dd, status=out["stb"])
             if e is eng:
                 got = out

@@ -175,19 +175,36 @@ def test_several_devices(pkg, orc):
 
 @pytest.mark.gpu
 def test_handle_state_after_the_loop(pkg, orc):
-    """Every handle refuses the per-trajectory read-backs and RBO_FLAG_REPLAY_TAPE; its next rollout equals a fresh handle's."""
+    """Every handle refuses the per-trajectory read-backs, the partial sums and RBO_FLAG_REPLAY_TAPE; its next rollout equals a fresh
+    handle's, and so do the partial sums of a non-leader handle after it."""
+    import torch
     wl, sur, rn, starts, dd = c2_case(pkg, orc, M=40)
     lib = pkg._lib.load()
+    nsum = 1 + 3 * (1 + wl.d + 1) + 2
+    dev = torch.zeros(nsum, dtype=torch.float64, device="cuda:0")
     engs = shard_engines(pkg, wl.h, sur, rn, starts, [(25, 15), (0, 25)])
     try:
         solve_sharded(pkg, engs, wl, sur, random_starts(wl, 3, 5), dd, max_iterations=4, use_eswavs=False)
         for e in engs:
             assert lib.rbo_get_results(e.handle.h, pkg._lib.dptr(np.zeros(e.m_count)), None, None, None, None, None) == -3
+            assert lib.rbo_partial_sums_host(e.handle.h, pkg._lib.dptr(np.zeros(nsum)), nsum) == -3
+            assert lib.rbo_partial_sums_device(e.handle.h, C.c_void_p(dev.data_ptr()), nsum) == -3
             M = e.m_count
             with pytest.raises(pkg.RboError, match=r"librbo error -3"):  # RBO_ERR_STATE
                 e.rollout(wl.x0, wl.theta, wl.lbs, wl.ubs, wl.h, float(np.min(sur.y)), np.zeros(M), np.zeros((wl.d, M), order="F"),
                           np.zeros((1, M), order="F"), dual_dirs=np.asfortranarray(dd[:, :, e.m_begin:e.m_begin + M]), replay=True)
         assert_rollouts_like_fresh(pkg, engs, wl, sur, rn, starts, dd)
+        # the non-leader handle's partial sums after that rollout are a fresh handle's after the same rollout
+        fresh = shard_engines(pkg, wl.h, sur, rn, starts, [(engs[1].m_begin, engs[1].m_count)])
+        try:
+            sums = []
+            for e in (engs[1], fresh[0]):
+                rollout_outputs(e, wl, sur, dd, wl.x0)
+                sums.append(np.zeros(nsum))
+                assert lib.rbo_partial_sums_host(e.handle.h, pkg._lib.dptr(sums[-1]), nsum) == 0
+            assert np.array_equal(sums[0], sums[1]) and sums[0][0] > 0
+        finally:
+            close(fresh)
     finally:
         close(engs)
 
