@@ -136,6 +136,54 @@ int rbo_condition(rbo_handle* h, const double* x, double y);
 /* Reads the resident surrogate back (any pointer may be NULL): N, X (d x N, ldX >= d), y[N], c[N] = K^-1 y. */
 int rbo_get_surrogate(rbo_handle* h, int* N, double* X, int ldX, double* y, double* c);
 
+/* ---- the kernel hyper-parameters, fitted on the device (optimize!, rbs.jl:770-829) ---------------------------------------------
+ * Only the kernel hyper-parameters psi.theta are fitted -- l for the Matern and squared-exponential kernels, (l, p) for Periodic --;
+ * sigma_n2 stays the resident one. K, its Cholesky factor, K^-1 and the gradient are computed on the device in FP64 (hand-written
+ * CUDA, the O(N^3) parts on the FP64 tensor cores); every reduction runs in a fixed order without atomics, so repeated calls on one
+ * handle return bit-identical results. Workspace: about 2 N^2 doubles, kept by the handle (grow-only). */
+
+/* Log marginal likelihood of the resident surrogate's data (X, y of its N observations, rbo_condition included) under kernel
+ * hyper-parameters ktheta of the resident kernel family:
+ *   ll = -y'K^-1 y / 2 - log det K / 2 - N log(2 pi) / 2,   K = [psi(|X_i - X_j|; ktheta)] + sigma_n2 I  (rbf.jl:161-178)
+ *   grad[nktheta] = d ll / d ktheta = tr((a a' - K^-1) dK/dktheta_i) / 2,  a = K^-1 y     (NULL: value only)
+ * The objective of optimize! (rbs.jl:770-829). The resident surrogate is not changed. RBO_ERR_NUMERIC when K is not positive
+ * definite at ktheta; RBO_ERR_ARG when nktheta differs from the family's count (1; Periodic: 2) or a ktheta <= 0; RBO_ERR_STATE
+ * without a surrogate. One synchronisation per call. */
+int rbo_log_marginal_likelihood(rbo_handle* h, const double* ktheta, int nktheta, double* ll, double* grad);
+
+/* set_kernel! (rbs.jl:123-135) on the resident surrogate: K, its Cholesky factor, c = K^-1 y and the packed form the rollout kernel
+ * streams are rebuilt ON THE DEVICE for kernel_id / ktheta from the resident X, y (rbo_condition included), the factor's inverse by
+ * the same double-double kernel as rbo_set_surrogate. Normals, starts and quadrature stay valid (as after rbo_condition).
+ * RBO_ERR_NUMERIC (PosDefException) leaves the handle unchanged; RBO_ERR_ARG for an unknown kernel id or ktheta as above.
+ * Deterministic: handles holding the same surrogate (e.g. the shards of rbo_stochastic_solve_batch_sharded) end with bit-identical
+ * resident surrogates after the same call, so a fit on one handle and rbo_set_kernel with its result on the others keeps them equal. */
+int rbo_set_kernel(rbo_handle* h, int kernel_id, const double* ktheta, int nktheta);
+
+enum { RBO_FIT_GTOL = 0, RBO_FIT_FTOL = 1, RBO_FIT_MAXIT = 2, RBO_FIT_MAXEVALS = 3 };  /* why rbo_fit_kernel stopped */
+typedef struct {
+  int32_t max_iterations; /* accepted quasi-Newton steps (SURVEY 3.4: 30) */
+  int32_t max_evals;      /* likelihood evaluations in all, line-search trials included */
+  double gtol;            /* stop: max |projected gradient of ll in log ktheta| <= gtol * max(1, |ll|) */
+  double ftol;            /* stop: ll gained by the last step <= ftol * max(1, |ll|) */
+} rbo_fit_opts;
+/* 30 iterations, 200 evaluations, gtol 1e-6, ftol 1e-12. */
+void rbo_default_fit_opts(rbo_fit_opts* o);
+
+/* optimize!(s::Surrogate) (rbs.jl:805-829): maximise ll over ktheta of the resident kernel family in the box [lb, ub]
+ * (0 < lb <= ub < inf componentwise, nktheta entries each), starting at the resident ktheta clamped to the box, and end with
+ * rbo_set_kernel at the best point found. The reference's optimize! body and its box are not part of this contract: it specifies
+ * the optimum, not the path. The search runs in t = log ktheta: projected L-BFGS with memory nktheta (pairs with s'y <= 0 on the free
+ * components are skipped), backtracking Armijo (c1 = 1e-4, halving) along the projected path t(alpha) = clamp(t + alpha d); the first
+ * step is scaled to move t by at most 1. A trial at which K is not positive definite counts as a rejected step. A component on a
+ * bound returns that bound exactly. If no trial moving t by more than 1e-10 decreases -ll, the fit ends with RBO_FIT_FTOL.
+ * The host drives the iteration: each evaluation is one rbo_log_marginal_likelihood (one synchronisation).
+ * Outputs (any may be NULL): ktheta_out[nktheta], ll_out, grad_out[nktheta] = d ll / d ktheta at ktheta_out, n_iter (accepted steps),
+ * n_evals (evaluations, the first included), status (RBO_FIT_*). RBO_ERR_NUMERIC if K is not positive definite at the start point;
+ * the handle is then unchanged. RBO_ERR_ARG for NULL options or box, lb > ub, lb <= 0, max_iterations < 0, max_evals < 1, negative
+ * tolerances. */
+int rbo_fit_kernel(rbo_handle* h, const rbo_fit_opts* o, const double* lb, const double* ub, double* ktheta_out, double* ll_out,
+                   double* grad_out, int32_t* n_iter, int32_t* n_evals, int32_t* status);
+
 /* tp.rnstream_sequence (trajectory.jl:47): M_total x (d+1) x hp1, column-major, sample index fastest.
  * This handle keeps samples [m_begin, m_begin + m_count). */
 int rbo_set_normals(rbo_handle* h, const double* rn, int M_total, int hp1, int m_begin, int m_count);

@@ -29,6 +29,10 @@ class SgaOpts(C.Structure):
                 ("eta", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double)]
 
 
+class FitOpts(C.Structure):
+    _fields_ = [("max_iterations", C.c_int32), ("max_evals", C.c_int32), ("gtol", C.c_double), ("ftol", C.c_double)]
+
+
 # every symbol include/rbo.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "rbo_abi_version": (C.c_int, []),
@@ -44,6 +48,10 @@ SYMBOLS = {
                                     _dp, C.c_int, C.c_int, C.c_double]),
     "rbo_condition": (C.c_int, [C.c_void_p, _dp, C.c_double]),
     "rbo_get_surrogate": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), _dp, C.c_int, _dp, _dp]),
+    "rbo_log_marginal_likelihood": (C.c_int, [C.c_void_p, _dp, C.c_int, _dp, _dp]),
+    "rbo_set_kernel": (C.c_int, [C.c_void_p, C.c_int, _dp, C.c_int]),
+    "rbo_default_fit_opts": (None, [C.POINTER(FitOpts)]),
+    "rbo_fit_kernel": (C.c_int, [C.c_void_p, C.POINTER(FitOpts), _dp, _dp, _dp, _dp, _dp, _ip, _ip, _ip]),
     "rbo_set_normals": (C.c_int, [C.c_void_p, _dp, C.c_int, C.c_int, C.c_int, C.c_int]),
     "rbo_generate_normals": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
     "rbo_get_normals": (C.c_int, [C.c_void_p, _dp]),

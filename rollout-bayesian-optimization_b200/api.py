@@ -398,6 +398,7 @@ class RolloutEngine:
         if stream is not None:
             self.handle.check(self.lib.rbo_set_stream(self.handle.h, C.c_void_p(stream)))
         self.d = None
+        self.kernel_id = None  # the resident kernel family: rbo_fit_kernel reads and writes as many entries as it has hyper-parameters
         self.m_count = 0
         self.m_begin, self.M_total = 0, 0  # the shard of the normals: samples [m_begin, m_begin + m_count) of M_total
 
@@ -439,6 +440,7 @@ class RolloutEngine:
         self.handle.check(self.lib.rbo_set_surrogate(self.handle.h, d, N, dptr(X), X.shape[0], dptr(L), L.shape[0], dptr(y), dptr(c),
                                                      fs.σn2, fs.ψ.kernel_id, dptr(kt), len(kt), fs.g.rule_id, fs.g.σtol))
         self.d = d
+        self.kernel_id = fs.ψ.kernel_id
 
     def condition(self, xnew, ynew):
         """condition!(s::Surrogate, x, y) (rbs.jl:214-222) on the device-resident surrogate (rbo_condition)."""
@@ -452,6 +454,43 @@ class RolloutEngine:
         X = np.zeros((self.d, n.value), order="F"); y = np.zeros(n.value); c = np.zeros(n.value)
         self.handle.check(self.lib.rbo_get_surrogate(self.handle.h, C.byref(n), dptr(X), self.d, dptr(y), dptr(c)))
         return X, y, c
+
+    def log_marginal_likelihood(self, ktheta, grad=True):
+        """rbo_log_marginal_likelihood: (ll, d ll / d ktheta) of the resident data under ktheta of the resident kernel family (the gradient
+        is None with grad=False). The resident surrogate is not changed; raises RboError (RBO_ERR_NUMERIC) when K is not positive definite."""
+        kt = np.ascontiguousarray(ktheta, dtype=np.float64).ravel()
+        ll = C.c_double()
+        g = np.zeros(len(kt)) if grad else None
+        self.handle.check(self.lib.rbo_log_marginal_likelihood(self.handle.h, dptr(kt), len(kt), C.byref(ll), dptr(g)))
+        return ll.value, g
+
+    def set_kernel(self, kernel):
+        """set_kernel!(s, kernel) (rbs.jl:123-135) on the resident surrogate (rbo_set_kernel): kernel is a RadialBasisFunction."""
+        kt = np.ascontiguousarray(kernel.θ, dtype=np.float64)
+        self.handle.check(self.lib.rbo_set_kernel(self.handle.h, kernel.kernel_id, dptr(kt), len(kt)))
+        self.kernel_id = kernel.kernel_id
+
+    def fit_kernel(self, lower, upper, max_iterations=None, max_evals=None, gtol=None, ftol=None):
+        """rbo_fit_kernel: maximum-likelihood kernel hyper-parameters in the box [lower, upper] (optimize!, rbs.jl:805-829); the resident
+        surrogate ends at the optimum. Unset options keep rbo_default_fit_opts. Returns a dict: ktheta, ll, grad (d ll / d ktheta there),
+        n_iter, n_evals, status (FIT_GTOL, FIT_FTOL, FIT_MAXIT, FIT_MAXEVALS)."""
+        o = _lib.FitOpts()
+        self.lib.rbo_default_fit_opts(C.byref(o))
+        for k, v in dict(max_iterations=max_iterations, max_evals=max_evals, gtol=gtol, ftol=ftol).items():
+            if v is not None:
+                setattr(o, k, v)
+        lb = np.ascontiguousarray(lower, dtype=np.float64).ravel(); ub = np.ascontiguousarray(upper, dtype=np.float64).ravel()
+        if self.kernel_id is None:
+            raise RboError("fit_kernel: no surrogate (set_surrogate)")
+        n = 2 if self.kernel_id == KERNEL_IDS["Periodic"] else 1
+        if len(lb) != n or len(ub) != n:
+            raise ValueError(f"fit_kernel: the resident kernel has {n} hyper-parameter(s); lower and upper must have {n} entries each")
+        kt, g = np.zeros(len(lb)), np.zeros(len(lb))
+        ll = C.c_double()
+        it, ev, st = C.c_int32(), C.c_int32(), C.c_int32()
+        self.handle.check(self.lib.rbo_fit_kernel(self.handle.h, C.byref(o), dptr(lb), dptr(ub), dptr(kt), C.byref(ll), dptr(g), C.byref(it),
+                                                  C.byref(ev), C.byref(st)))
+        return dict(ktheta=kt, ll=ll.value, grad=g, n_iter=it.value, n_evals=ev.value, status=st.value)
 
     def set_normals(self, rn, m_begin=0, m_count=None):
         rn = np.asfortranarray(rn, dtype=np.float64)
@@ -585,6 +624,24 @@ class RolloutEngine:
         p = np.zeros((B, n)); hit = np.zeros(B, np.int32)
         self.handle.check(self.lib.rbo_tr_step_batch(self.handle.h, n, B, dptr(H), dptr(g), dptr(Delta), dptr(p), iptr(hit)))
         return p, hit.astype(bool)
+
+
+FIT_GTOL, FIT_FTOL, FIT_MAXIT, FIT_MAXEVALS = 0, 1, 2, 3  # why rbo_fit_kernel stopped
+
+
+def optimize(s, lower, upper, device=0, **opts):
+    """optimize!(s::Surrogate) (rbs.jl:805-829) for callers who keep the host Surrogate: the maximum-likelihood fit of ψ.θ in the box
+    [lower, upper] runs on the device (RolloutEngine.fit_kernel; the box comes from the caller), then ψ.θ is set to the optimum and the
+    host mirror's K, L and c are rebuilt there by set_kernel (one host factorisation instead of one per likelihood evaluation). σn2 is not
+    fitted. opts: the options of fit_kernel. Returns fit_kernel's dict."""
+    eng = RolloutEngine(device)
+    try:
+        eng.set_surrogate(s)
+        r = eng.fit_kernel(lower, upper, **opts)
+    finally:
+        eng.close()
+    set_kernel(s, RadialBasisFunction(r["ktheta"], s.ψ.constructor))
+    return r
 
 
 def _mean_std_rows(A):

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "rbo_kernel.cuh"
+#include "likelihood_kernels.cuh"
 #include "sga_kernels.cuh"
 #include "support_kernels.cuh"
 #include "sobol_dirs.h"
@@ -132,6 +133,10 @@ struct rbo_handle {
   // rbo_stochastic_solve_batch_sharded, on the leader: every shard's values and grad_x; status and the watchdog flag table
   DevBuf<double> sga_gather;
   DevBuf<int> sga_igather;
+  // log marginal likelihood / set_kernel workspace (NP = N rounded up to RBO_LK_B): K, then L in place, then K^-1 (NP^2); W = L^-1 (NP^2);
+  // [the diagonal blocks' inverses (NP x RBO_LK_B) | diag L (NP) | u, a (NP each) | per-tile gradient partials | ll, gradient]
+  DevBuf<double> lk_A, lk_W, lk_v;
+  DevBuf<int> lk_stat;
 
   ~rbo_handle() {
     if (ev0) cudaEventDestroy(ev0);
@@ -325,6 +330,26 @@ static int reserve_surrogate(rbo_handle* h, int d, int rows_needed, bool keep) {
   return RBO_SUCCESS;
 }
 
+// The resident form from the lower factor in Ld (N x N, column-major) and the resident y: the explicit inverse L0^-1 on the device in
+// double-double arithmetic (one rounding per stored entry), so that every later "triangular solve" against L0 is a dependency-free
+// panel product on the FP64 tensor cores; u0 = L0^-1 y (kept so that the coefficient re-solve of rbs.jl:422-429 only needs the backward
+// half); with solve_c also c0 = L0^-T u0, as rbo_condition re-solves it; then the packed panels. Stream-ordered.
+static int build_resident_form(rbo_handle* h, bool solve_c) {
+  const int N = h->N, N32 = (N + RBO_BR - 1) / RBO_BR * RBO_BR;
+  CK(h, cudaMemsetAsync(h->Linv, 0, (size_t)N32 * h->ldi * 8, h->stream));
+  {
+    const int wpc = std::max(1, std::min(4, (int)((200 * 1024) / ((size_t)N * 16))));
+    const size_t smem = (size_t)wpc * 2 * N * 8;
+    CK(h, cudaFuncSetAttribute(rbo_trinv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
+    rbo_trinv_kernel<<<(N32 + wpc - 1) / wpc, 32 * wpc, smem, h->stream>>>(h->Ld, N, N32, h->Linv, h->ldi);
+    CK(h, cudaGetLastError());
+  }
+  rbo_matvec_lower_kernel<<<(N + 7) / 8, 256, 0, h->stream>>>(h->Linv, h->ldi, N, h->yb, h->u0);
+  if (solve_c) rbo_matvec_lower_t_kernel<<<(N + 127) / 128, 128, 0, h->stream>>>(h->Linv, h->ldi, N, h->u0, 1.0, h->c0);
+  CK(h, cudaGetLastError());
+  return repack_surrogate(h);
+}
+
 int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, const double* L, int ldL, const double* y, const double* c,
                       double sigma_n2, int kernel_id, const double* ktheta, int nktheta, int rule_id, double sigma_tol) {
   if (!h) return RBO_ERR_ARG;
@@ -357,7 +382,6 @@ int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, con
   double ymin = y[0];
   for (int j = 0; j < N; ++j) ymin = std::min(ymin, y[j]);
   h->ymin_base = ymin;
-  const int N32 = (N + RBO_BR - 1) / RBO_BR * RBO_BR;
   // H2D of what FantasySurrogate(s, h) copies (rbs.jl:345-381): X (d x N), the lower factor, y, c
   CK(h, h->Ld.reserve((size_t)N * N));
   CK(h, cudaMemcpy2DAsync(h->Xpts, (size_t)d * 8, X, (size_t)ldX * 8, (size_t)d * 8, N, cudaMemcpyHostToDevice, h->stream));
@@ -366,20 +390,7 @@ int rbo_set_surrogate(rbo_handle* h, int d, int N, const double* X, int ldX, con
   CK(h, cudaMemsetAsync(h->u0, 0, h->u0.cap * 8, h->stream));
   CK(h, cudaMemcpyAsync(h->yb, y, (size_t)N * 8, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(h->c0, c, (size_t)N * 8, cudaMemcpyHostToDevice, h->stream));
-  // Explicit inverse of the base factor on the device in double-double arithmetic (one rounding per stored entry): every later
-  // "triangular solve" against L0 is then a dependency-free panel product on the FP64 tensor cores.
-  CK(h, cudaMemsetAsync(h->Linv, 0, (size_t)N32 * h->ldi * 8, h->stream));
-  {
-    const int wpc = std::max(1, std::min(4, (int)((200 * 1024) / ((size_t)N * 16))));
-    const size_t smem = (size_t)wpc * 2 * N * 8;
-    CK(h, cudaFuncSetAttribute(rbo_trinv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-    rbo_trinv_kernel<<<(N32 + wpc - 1) / wpc, 32 * wpc, smem, h->stream>>>(h->Ld, N, N32, h->Linv, h->ldi);
-    CK(h, cudaGetLastError());
-  }
-  // u0 = L^-1 y (kept so that the coefficient re-solve of rbs.jl:422-429 only needs the backward half)
-  rbo_matvec_lower_kernel<<<(N + 7) / 8, 256, 0, h->stream>>>(h->Linv, h->ldi, N, h->yb, h->u0);
-  CK(h, cudaGetLastError());
-  rc = repack_surrogate(h);
+  rc = build_resident_form(h, false);
   if (rc) return rc;
   CK(h, cudaStreamSynchronize(h->stream));  // the caller's buffers may change after return
   h->have_sur = true;
@@ -436,6 +447,264 @@ int rbo_get_surrogate(rbo_handle* h, int* N_out, double* X, int ldX, double* y, 
   if (y) CK(h, cudaMemcpyAsync(y, h->yb, (size_t)h->N * 8, cudaMemcpyDeviceToHost, h->stream));
   if (c) CK(h, cudaMemcpyAsync(c, h->c0, (size_t)h->N * 8, cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
+  return RBO_SUCCESS;
+}
+
+// ---- the kernel hyper-parameters on the device: log marginal likelihood, set_kernel!, optimize! (likelihood_kernels.cu) -------------
+// ktheta of kernel family kernel_id as a KernelSpec: the family's count of hyper-parameters (1; Periodic: 2), each positive and finite.
+static int kernel_spec(rbo_handle* h, const char* me, int kernel_id, const double* ktheta, int nktheta, KernelSpec* ks) {
+  if (kernel_id < RBO_KERNEL_MATERN12 || kernel_id > RBO_KERNEL_PERIODIC) return fail(h, RBO_ERR_ARG, "%s: unknown kernel id %d", me, kernel_id);
+  const int want = kernel_id == RBO_KERNEL_PERIODIC ? 2 : 1;
+  if (!ktheta || nktheta != want) return fail(h, RBO_ERR_ARG, "%s: kernel %d takes %d hyper-parameter(s), %d given", me, kernel_id, want, nktheta);
+  ks->id = kernel_id;
+  for (int i = 0; i < 4; ++i) ks->th[i] = i < want ? ktheta[i] : 0.0;
+  for (int i = 0; i < want; ++i)
+    if (!(ktheta[i] > 0.0) || !std::isfinite(ktheta[i])) return fail(h, RBO_ERR_ARG, "%s: ktheta[%d] = %g must be positive and finite", me, i, ktheta[i]);
+  return RBO_SUCCESS;
+}
+
+// The likelihood workspace of the resident N: NP = N rounded up to RBO_LK_B; lk_v = [Dinv | diag L | u | a | partials | out]
+struct LikLayout {
+  int N, NP, nb, ntiles;
+  size_t diagL, u, a, partial, out, len;
+  explicit LikLayout(int N_) : N(N_), NP((N_ + RBO_LK_B - 1) / RBO_LK_B * RBO_LK_B), nb(NP / RBO_LK_B), ntiles(nb * (nb + 1) / 2) {
+    diagL = (size_t)NP * RBO_LK_B; u = diagL + NP; a = u + NP; partial = a + NP; out = partial + 2 * (size_t)ntiles; len = out + 4;
+  }
+};
+
+// Enqueues K at ks (from the resident sites and sigma_n2) and its blocked Cholesky factor into lk_A; a non-positive pivot sets lk_stat.
+static int lik_factor(rbo_handle* h, const KernelSpec& ks, const LikLayout& Y) {
+  const int NP = Y.NP;
+  CK(h, h->lk_A.reserve((size_t)NP * NP));
+  CK(h, h->lk_v.reserve(Y.len));
+  CK(h, h->lk_stat.reserve(1));
+  CK(h, cudaMemsetAsync(h->lk_stat, 0, sizeof(int), h->stream));
+  double k0, a, b;
+  kern_eval(ks, 0.0, k0, a, b);
+  const int blocks = (int)std::min<size_t>(((size_t)NP * NP + 255) / 256, (size_t)h->num_sms * 16);
+  rbo_lik_assemble_kernel<<<blocks, 256, 0, h->stream>>>(h->Xpts, h->d, Y.N, NP, ks, k0 + h->sigma_n2, h->lk_A);
+  CK(h, cudaFuncSetAttribute(rbo_lik_potrf_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RBO_LK_DIAG_SMEM));
+  for (int kb = 0; kb < Y.nb; ++kb) {
+    rbo_lik_potrf_diag_kernel<<<1, RBO_LK_THREADS, RBO_LK_DIAG_SMEM, h->stream>>>(h->lk_A, NP, kb, h->lk_v, h->lk_v + Y.diagL, h->lk_stat);
+    const int m = Y.nb - kb - 1;
+    if (m > 0) {
+      rbo_lik_panel_kernel<<<m, RBO_LK_THREADS, 0, h->stream>>>(h->lk_A, NP, kb, h->lk_v);
+      rbo_lik_update_kernel<<<m * (m + 1) / 2, RBO_LK_THREADS, 0, h->stream>>>(h->lk_A, NP, kb);
+    }
+  }
+  CK(h, cudaGetLastError());
+  return RBO_SUCCESS;
+}
+
+static int not_pd(rbo_handle* h, const char* me) {
+  return fail(h, RBO_ERR_NUMERIC, "%s: PosDefException -- K is not positive definite at these kernel hyper-parameters (set_kernel!, rbs.jl:123-135)", me);
+}
+
+// ll and (grad != NULL) d ll / d ktheta[nk] at ks over the resident data; one synchronisation. The resident surrogate is not touched.
+// L^-1 here is the plain-FP64 blocked inverse on the tensor cores: a fit needs it at every evaluation, and the double-double inverse
+// of the resident form (rbo_trinv_kernel, scalar, O(N^3)) would dominate the fit.
+static int lik_eval(rbo_handle* h, const char* me, const KernelSpec& ks, int nk, double* ll, double* grad) {
+  const LikLayout Y(h->N);
+  const int NP = Y.NP, N = Y.N;
+  if (int rc = lik_factor(h, ks, Y)) return rc;
+  CK(h, h->lk_W.reserve((size_t)NP * NP));
+  double* v = h->lk_v;
+  for (int i = 0; i < Y.nb; ++i) rbo_lik_trinv_row_kernel<<<i + 1, RBO_LK_THREADS, 0, h->stream>>>(h->lk_A, NP, i, v, h->lk_W);
+  // a = K^-1 y = W'(W y)
+  rbo_matvec_lower_kernel<<<(N + 7) / 8, 256, 0, h->stream>>>(h->lk_W, NP, N, h->yb, v + Y.u);
+  rbo_matvec_lower_t_kernel<<<(N + 127) / 128, 128, 0, h->stream>>>(h->lk_W, NP, N, v + Y.u, 1.0, v + Y.a);
+  if (grad) {
+    rbo_lik_lauum_kernel<<<Y.ntiles, RBO_LK_THREADS, 0, h->stream>>>(h->lk_W, NP, h->lk_A);  // K^-1 over the factor
+    rbo_lik_grad_kernel<<<Y.ntiles, RBO_LK_THREADS, 0, h->stream>>>(h->Xpts, h->d, N, NP, ks, v + Y.a, h->lk_A, v + Y.partial);
+  }
+  rbo_lik_final_kernel<<<1, 1024, 0, h->stream>>>(h->yb, v + Y.a, v + Y.diagL, N, v + Y.partial, grad ? Y.ntiles : 0, nk, v + Y.out);
+  CK(h, cudaGetLastError());
+  double res[3];
+  int st = 0;
+  CK(h, cudaMemcpyAsync(res, v + Y.out, (size_t)(1 + nk) * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaMemcpyAsync(&st, h->lk_stat, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  if (st) return not_pd(h, me);
+  *ll = res[0];
+  if (grad) for (int i = 0; i < nk; ++i) grad[i] = res[1 + i];
+  return RBO_SUCCESS;
+}
+
+// set_kernel! on the resident surrogate: factor into the workspace, and only once K is known to be positive definite replace Ld and
+// rebuild the resident form from it exactly as rbo_set_surrogate builds it from a caller's factor.
+static int set_kernel_resident(rbo_handle* h, const char* me, const KernelSpec& ks) {
+  const LikLayout Y(h->N);
+  const int N = Y.N;
+  if (int rc = lik_factor(h, ks, Y)) return rc;
+  int st = 0;
+  CK(h, cudaMemcpyAsync(&st, h->lk_stat, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  if (st) return not_pd(h, me);
+  CK(h, h->Ld.reserve((size_t)N * N));
+  rbo_lik_to_colmajor_kernel<<<(int)std::min<size_t>(((size_t)N * N + 255) / 256, (size_t)h->num_sms * 16), 256, 0, h->stream>>>(h->lk_A, Y.NP, N, h->Ld);
+  CK(h, cudaGetLastError());
+  h->kern = ks;
+  double a;
+  kern_eval(h->kern, 0.0, h->k0, a, h->d2k0);
+  if (int rc = build_resident_form(h, true)) return rc;
+  CK(h, cudaStreamSynchronize(h->stream));
+  return RBO_SUCCESS;
+}
+
+int rbo_log_marginal_likelihood(rbo_handle* h, const double* ktheta, int nktheta, double* ll, double* grad) {
+  const char* me = "rbo_log_marginal_likelihood";
+  if (!h) return RBO_ERR_ARG;
+  if (!ll) return fail(h, RBO_ERR_ARG, "%s: ll is NULL", me);
+  if (!h->have_sur) return fail(h, RBO_ERR_STATE, "%s: no surrogate (rbo_set_surrogate)", me);
+  KernelSpec ks;
+  if (int rc = kernel_spec(h, me, h->kern.id, ktheta, nktheta, &ks)) return rc;
+  CK(h, cudaSetDevice(h->device));
+  return lik_eval(h, me, ks, nktheta, ll, grad);
+}
+
+int rbo_set_kernel(rbo_handle* h, int kernel_id, const double* ktheta, int nktheta) {
+  const char* me = "rbo_set_kernel";
+  if (!h) return RBO_ERR_ARG;
+  if (!h->have_sur) return fail(h, RBO_ERR_STATE, "%s: no surrogate (rbo_set_surrogate)", me);
+  KernelSpec ks;
+  if (int rc = kernel_spec(h, me, kernel_id, ktheta, nktheta, &ks)) return rc;
+  CK(h, cudaSetDevice(h->device));
+  return set_kernel_resident(h, me, ks);
+}
+
+void rbo_default_fit_opts(rbo_fit_opts* o) {
+  if (!o) return;
+  o->max_iterations = 30;  // SURVEY 3.4: Fminbox(LBFGS), 30 iterations
+  o->max_evals = 200;
+  o->gtol = 1e-6;
+  o->ftol = 1e-12;
+}
+
+int rbo_fit_kernel(rbo_handle* h, const rbo_fit_opts* o, const double* lb, const double* ub, double* ktheta_out, double* ll_out, double* grad_out,
+                   int32_t* n_iter, int32_t* n_evals, int32_t* status) {
+  const char* me = "rbo_fit_kernel";
+  if (!h) return RBO_ERR_ARG;
+  if (!o || !lb || !ub) return fail(h, RBO_ERR_ARG, "%s: o, lb and ub are required", me);
+  if (!h->have_sur) return fail(h, RBO_ERR_STATE, "%s: no surrogate (rbo_set_surrogate)", me);
+  if (o->max_iterations < 0 || o->max_evals < 1 || !(o->gtol >= 0.0) || !(o->ftol >= 0.0)) return fail(h, RBO_ERR_ARG, "%s: invalid options", me);
+  const int n = h->kern.id == RBO_KERNEL_PERIODIC ? 2 : 1;
+  for (int i = 0; i < n; ++i)
+    if (!(lb[i] > 0.0) || !(lb[i] <= ub[i]) || !std::isfinite(ub[i]))
+      return fail(h, RBO_ERR_ARG, "%s: box [%g, %g] of ktheta[%d] is not 0 < lb <= ub < inf", me, lb[i], ub[i], i);
+  CK(h, cudaSetDevice(h->device));
+  // Projected L-BFGS on f(t) = -ll(exp(t)), t = log ktheta in [log lb, log ub]. A component on a bound maps to that bound exactly.
+  double tlo[2], thi[2], t[2], g[2], f, gll[2];
+  KernelSpec ks = h->kern;
+  auto to_theta = [&](const double* tt, KernelSpec& k) {
+    k = h->kern;
+    for (int i = 0; i < n; ++i) k.th[i] = tt[i] <= tlo[i] ? lb[i] : tt[i] >= thi[i] ? ub[i] : std::min(std::max(std::exp(tt[i]), lb[i]), ub[i]);
+  };
+  int evals = 0, iters = 0;
+  // f and its gradient in t at tt (fo, go, the gradient of ll in ktheta into gl); RBO_ERR_NUMERIC when K is not positive definite there
+  auto eval = [&](const double* tt, double& fo, double* go, double* gl, KernelSpec& k) -> int {
+    to_theta(tt, k);
+    ++evals;
+    double ll;
+    const int rc = lik_eval(h, me, k, n, &ll, gl);
+    if (rc) return rc;
+    fo = -ll;
+    for (int i = 0; i < n; ++i) go[i] = -gl[i] * k.th[i];
+    return RBO_SUCCESS;
+  };
+  auto proj_grad = [&](const double* tt, const double* gg, double* pg) {
+    double m = 0.0;
+    for (int i = 0; i < n; ++i) {
+      pg[i] = ((tt[i] <= tlo[i] && gg[i] > 0.0) || (tt[i] >= thi[i] && gg[i] < 0.0)) ? 0.0 : gg[i];
+      m = std::max(m, std::fabs(pg[i]));
+    }
+    return m;
+  };
+  for (int i = 0; i < n; ++i) {
+    tlo[i] = std::log(lb[i]);
+    thi[i] = std::log(ub[i]);
+    const double th0 = std::min(std::max(h->kern.th[i], lb[i]), ub[i]);
+    t[i] = th0 == lb[i] ? tlo[i] : th0 == ub[i] ? thi[i] : std::min(std::max(std::log(th0), tlo[i]), thi[i]);
+  }
+  if (int rc = eval(t, f, g, gll, ks)) return rc;  // not PD at the start: nothing has changed
+  const std::string err_before = h->err;  // a rejected trial records its PosDefException; a fit that succeeds does not report it
+  double S[2][2], Yv[2][2];  // the last n accepted steps and gradient changes, oldest first
+  int npairs = 0, st = -1;
+  double pg[2];
+  if (proj_grad(t, g, pg) <= o->gtol * std::max(1.0, std::fabs(f))) st = RBO_FIT_GTOL;
+  else if (o->max_iterations == 0) st = RBO_FIT_MAXIT;
+  while (st < 0) {
+    // direction: two-loop recursion over the pairs on the free components (pg != 0); the others stay on their bound
+    double q[2], d[2], al[2], rho[2];
+    bool freev[2];
+    for (int i = 0; i < n; ++i) { freev[i] = pg[i] != 0.0; q[i] = pg[i]; }
+    auto dotf = [&](const double* a, const double* b) { double s = 0.0; for (int i = 0; i < n; ++i) if (freev[i]) s += a[i] * b[i]; return s; };
+    double gamma = 1.0;  // initial Hessian scale s'y / y'y of the newest usable pair
+    bool use[2] = {false, false}, scaled = false;
+    for (int k = npairs - 1; k >= 0; --k) {
+      const double sy = dotf(S[k], Yv[k]);
+      if (!(sy > 0.0)) continue;
+      use[k] = true;
+      rho[k] = 1.0 / sy;
+      al[k] = rho[k] * dotf(S[k], q);
+      for (int i = 0; i < n; ++i) if (freev[i]) q[i] -= al[k] * Yv[k][i];
+      if (!scaled) { gamma = sy / dotf(Yv[k], Yv[k]); scaled = true; }
+    }
+    for (int i = 0; i < n; ++i) q[i] *= gamma;
+    for (int k = 0; k < npairs; ++k) {
+      if (!use[k]) continue;
+      const double be = rho[k] * dotf(Yv[k], q);
+      for (int i = 0; i < n; ++i) if (freev[i]) q[i] += S[k][i] * (al[k] - be);
+    }
+    double dmax = 0.0, slope = 0.0;
+    for (int i = 0; i < n; ++i) { d[i] = freev[i] ? -q[i] : 0.0; slope += d[i] * pg[i]; }
+    if (!(slope < 0.0)) for (int i = 0; i < n; ++i) d[i] = -pg[i];  // not a descent direction: steepest descent
+    for (int i = 0; i < n; ++i) dmax = std::max(dmax, std::fabs(d[i]));
+    // backtracking Armijo on the projected path; a trial at which K is not positive definite is a rejected step
+    double alpha = npairs == 0 ? std::min(1.0, 1.0 / dmax) : 1.0, tn[2], fn = 0.0, gn[2], gln[2];
+    KernelSpec kn;
+    bool accepted = false;
+    while (!accepted) {
+      bool moved = false;
+      double dec = 0.0;
+      for (int i = 0; i < n; ++i) {
+        tn[i] = std::min(std::max(t[i] + alpha * d[i], tlo[i]), thi[i]);
+        moved |= std::fabs(tn[i] - t[i]) > 1e-10;  // below this the trials differ from t in rounding only
+        dec += g[i] * (tn[i] - t[i]);
+      }
+      if (!moved) break;
+      if (evals >= o->max_evals) { st = RBO_FIT_MAXEVALS; break; }
+      const int rc = eval(tn, fn, gn, gln, kn);
+      if (rc && rc != RBO_ERR_NUMERIC) return rc;
+      if (rc == RBO_SUCCESS && fn <= f + 1e-4 * dec) accepted = true;
+      else alpha *= 0.5;
+    }
+    if (st >= 0) break;
+    if (!accepted) { st = RBO_FIT_FTOL; break; }  // no step along the projected path decreases f: nothing left to gain
+    if (npairs == n) {
+      for (int k = 1; k < n; ++k) for (int i = 0; i < n; ++i) { S[k - 1][i] = S[k][i]; Yv[k - 1][i] = Yv[k][i]; }
+      --npairs;
+    }
+    for (int i = 0; i < n; ++i) { S[npairs][i] = tn[i] - t[i]; Yv[npairs][i] = gn[i] - g[i]; }
+    ++npairs;
+    const double gain = f - fn;
+    for (int i = 0; i < n; ++i) { t[i] = tn[i]; g[i] = gn[i]; gll[i] = gln[i]; }
+    f = fn;
+    ks = kn;
+    ++iters;
+    if (proj_grad(t, g, pg) <= o->gtol * std::max(1.0, std::fabs(f))) st = RBO_FIT_GTOL;
+    else if (gain <= o->ftol * std::max(1.0, std::fabs(f))) st = RBO_FIT_FTOL;
+    else if (iters >= o->max_iterations) st = RBO_FIT_MAXIT;
+  }
+  if (int rc = set_kernel_resident(h, me, ks)) return rc;
+  h->err = err_before;
+  for (int i = 0; i < n; ++i) {
+    if (ktheta_out) ktheta_out[i] = ks.th[i];
+    if (grad_out) grad_out[i] = gll[i];
+  }
+  if (ll_out) *ll_out = -f;
+  if (n_iter) *n_iter = iters;
+  if (n_evals) *n_evals = evals;
+  if (status) *status = st;
   return RBO_SUCCESS;
 }
 

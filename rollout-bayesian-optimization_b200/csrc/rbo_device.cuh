@@ -80,6 +80,42 @@ __host__ __device__ inline void kern_eval(const KernelSpec& k, double rho, doubl
   }
 }
 
+// Derivatives of psi(rho) with respect to the kernel hyper-parameters: dth[0] = d psi / d l (every family), dth[1] = d psi / d p
+// (Periodic only). The objective of the maximum-likelihood fit (rbs.jl:770-829) needs them; psi(0) = 1 does not depend on them.
+__host__ __device__ inline void kern_dtheta(const KernelSpec& k, double rho, double* dth) {
+  dth[1] = 0.0;
+  switch (k.id) {
+    case RBO_KERNEL_MATERN52: {
+      const double l = k.th[0], s = sqrt(5.0) / l * rho;
+      dth[0] = s * s * (1.0 + s) / (3.0 * l) * exp(-s);
+      break;
+    }
+    case RBO_KERNEL_MATERN32: {
+      const double l = k.th[0], s = sqrt(3.0) / l * rho;
+      dth[0] = s * s / l * exp(-s);
+      break;
+    }
+    case RBO_KERNEL_MATERN12: {
+      const double l = k.th[0];
+      dth[0] = rho / (l * l) * exp(-rho / l);
+      break;
+    }
+    case RBO_KERNEL_SE: {
+      const double l = k.th[0], l2 = l * l;
+      dth[0] = rho * rho / (l2 * l) * exp(-rho * rho / (2.0 * l2));
+      break;
+    }
+    default: {  // RBO_KERNEL_PERIODIC
+      const double pi = 3.141592653589793;
+      const double l = k.th[0], p = k.th[1], u = pi * rho / p, sn = sin(u);
+      const double psi = exp(-2.0 * sn * sn / (l * l));
+      dth[0] = 4.0 * sn * sn / (l * l * l) * psi;
+      dth[1] = 2.0 * u * sin(2.0 * u) / (l * l * p) * psi;
+      break;
+    }
+  }
+}
+
 // Radial quantities at distance rho: psi, b = psi'/rho, a = (psi'' - psi'/rho)/rho^2, so that
 // grad k = b r (rbf.jl:127-134, 0 at rho = 0) and Hk = a r r' + b I (rbf.jl:141-150, psi''(0) I at rho = 0).
 __host__ __device__ inline void kern_radial(const KernelSpec& k, double rho2, double& psi, double& a, double& b, double& gb) {

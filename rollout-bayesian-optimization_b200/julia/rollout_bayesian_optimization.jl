@@ -16,7 +16,10 @@
 #      stochastic_solve_batch runs the whole ascent from a batch of restarts on the device in one call.
 #
 # Resident inputs: the handle remembers a fingerprint of the surrogate / normals / starts it holds and re-uploads only what changed
-# (a BO iteration changes the surrogate; an ascent iteration changes only x0). rbo_condition! appends an observation on the device.
+# (a BO iteration changes the surrogate; an ascent iteration changes only x0). rbo_condition!(s, x, y) appends an observation on the
+# host and on the device, rbo_optimize! fits the kernel hyper-parameters on the device and refits the host copy once; both keep the host
+# surrogate valid and record the fingerprint of the result, so a BO iteration rbo_condition! -> rbo_optimize! -> stochastic_solve_batch
+# uploads no surrogate and runs no likelihood evaluation on the host.
 #
 # rand(dim) of solve_dual_y (rollout.jl:133, SURVEY.md hard part 2): reproduced EXACTLY by a two-phase call -- values and best
 # indices first, then rand(d) is drawn on the host only for the case-3 samples, j = t, t-1, .., 1, in sample order (the reference's
@@ -102,10 +105,13 @@ end
 const _RBO_RESIDENT = Dict{Symbol, UInt}()   # fingerprints of what the handle currently holds
 _rbo_fp(xs...) = hash(xs)
 
+# what the handle holds of a (fantasy) surrogate with N observations: data, kernel and its hyper-parameters, rule, noise
+_rbo_surrogate_fp(s, N) = _rbo_fp(N, size(s.X, 1), view(s.X, :, 1:N), view(s.y, 1:N), Vector{Float64}(s.ψ.θ), s.ψ.constructor, s.g.name, s.σn2)
+
 """Uploads the base part of the fantasy surrogate unless the handle already holds it (same data, kernel, rule)."""
 function _rbo_sync_surrogate!(h::RboHandle, fs)
     N = get_known_observations(fs)
-    fp = _rbo_fp(N, size(fs.X, 1), view(fs.X, :, 1:N), view(fs.y, 1:N), Vector{Float64}(fs.ψ.θ), fs.ψ.constructor, fs.g.name, fs.σn2)
+    fp = _rbo_surrogate_fp(fs, N)
     get(_RBO_RESIDENT, :surrogate, UInt(0)) == fp && return
     _rbo_set_surrogate!(h, fs.X, fs.L.data, fs.y, fs.cs[1], N, fs.ψ, fs.g, fs.σn2)
     _RBO_RESIDENT[:surrogate] = fp
@@ -125,13 +131,73 @@ function _rbo_sync_starts!(h::RboHandle, starts::Matrix{Float64})
     _RBO_RESIDENT[:starts] = fp
 end
 
-"""condition!(s::Surrogate, x, y) (rbs.jl:214-222) mirrored on the device-resident surrogate: call it right after the host-side
-`condition!` of a BO iteration and the next simulate call uploads nothing (the fingerprint is refreshed by the caller's next sync)."""
+"""condition!(s::Surrogate, x, y) (rbs.jl:214-222) mirrored on the device-resident surrogate, for a caller that has already run the
+host-side `condition!(s, x, y)`: the device appends the same observation and the row of its factor in place. It cannot see s, so it
+forgets the fingerprint: the next sync hashes the host copy (X, y, θ) again and uploads it if the handle does not hold it.
+`rbo_condition!(s, x, y)` does both sides and records the fingerprint instead."""
 function rbo_condition!(x::Vector{Float64}, y::Float64)
     h = _rbo_handle()
     _rbo_check(h, ccall((:rbo_condition, librbo), Cint, (Ptr{Cvoid}, Ptr{Float64}, Float64), h.ptr, x, y))
-    delete!(_RBO_RESIDENT, :surrogate)   # the next sync compares against the host copy again (cheap: a hash of X, y)
+    delete!(_RBO_RESIDENT, :surrogate)
     return nothing
+end
+
+"""condition!(s, x, y) (rbs.jl:214-222) on the host surrogate AND on the device-resident one, in one call: the host's condition! (a
+rank-1 extension of K and L and the coefficient re-solve, O(N^2)) keeps s a valid surrogate for every path that uploads from it, the
+device appends the same observation and the row of its factor in place, and the fingerprint of the result is recorded so that the
+next simulate call or rbo_optimize! uploads nothing. Do not call the host's condition! as well: the observation would be appended
+twice. s must be the surrogate the default handle holds (its last sync)."""
+function rbo_condition!(s::Surrogate, x::Vector{Float64}, y::Float64)
+    h = _rbo_handle()
+    _rbo_sync_surrogate!(h, FantasySurrogate(s, 0))   # uploads only if the handle does not hold s already (fingerprint)
+    condition!(s, x, y)                                # throws before the device is touched if the host factor is not PD
+    delete!(_RBO_RESIDENT, :surrogate)
+    _rbo_check(h, ccall((:rbo_condition, librbo), Cint, (Ptr{Cvoid}, Ptr{Float64}, Float64), h.ptr, x, y))
+    _RBO_RESIDENT[:surrogate] = _rbo_surrogate_fp(s, get_observed(s))
+    return s
+end
+
+"""set_kernel!(s, kernel) (rbs.jl:123-135) on the host surrogate and on the default handle's resident surrogate (rbo_set_kernel: K,
+its factor and c rebuilt on the device from the resident data). The host's set_kernel! keeps s valid for every path that uploads from
+it; the fingerprint of the result is recorded. PosDefException (RBO_ERR_NUMERIC) on the device leaves the handle and s unchanged."""
+function rbo_set_kernel!(s::Surrogate, kernel)
+    h = _rbo_handle()
+    _rbo_sync_surrogate!(h, FantasySurrogate(s, 0))
+    θk = Vector{Float64}(kernel.θ)
+    _rbo_check(h, ccall((:rbo_set_kernel, librbo), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}, Cint), h.ptr, _RBO_KERNEL_ID[kernel.constructor],
+                        θk, length(θk)))
+    delete!(_RBO_RESIDENT, :surrogate)
+    set_kernel!(s, kernel)
+    _RBO_RESIDENT[:surrogate] = _rbo_surrogate_fp(s, get_observed(s))
+    return s
+end
+
+struct RboFitOpts
+    max_iterations::Int32; max_evals::Int32; gtol::Float64; ftol::Float64
+end
+
+"""The maximum-likelihood fit of the kernel hyper-parameters s.ψ.θ in the box [lower, upper] on the device (rbo_fit_kernel: projected
+L-BFGS in log θ, include/rbo.h), for optimize!(s::Surrogate) (rbs.jl:805-829) -- whose body and box this checkout cannot read, so the
+box comes from the caller and the reference's optimize! is left as it is. Every likelihood evaluation of the fit runs on the device,
+and the default handle's surrogate ends at the optimum. The host surrogate is then refitted once with set_kernel!(s, ψ(θ*)) -- one
+host factorisation instead of one per evaluation --, so s stays valid for every path that uploads from it (the multi-GPU calls
+included), and the fingerprint is recorded so that the default handle uploads nothing. σn² is not fitted. Returns (θ*, ll*, status)."""
+function rbo_optimize!(s::Surrogate, lower::AbstractVector, upper::AbstractVector; max_iterations::Integer = 30, max_evals::Integer = 200,
+                       gtol::Real = 1e-6, ftol::Real = 1e-12)
+    n = length(s.ψ.θ)
+    length(lower) == n && length(upper) == n || throw(ArgumentError("rbo_optimize!: the kernel has $n hyper-parameter(s); the box must have $n entries"))
+    h = _rbo_handle()
+    _rbo_sync_surrogate!(h, FantasySurrogate(s, 0))   # uploads only if the handle does not hold s already (fingerprint)
+    θ, ll, g = zeros(n), Ref{Float64}(0.0), zeros(n)
+    it, ev, st = Ref{Int32}(0), Ref{Int32}(0), Ref{Int32}(0)
+    o = Ref(RboFitOpts(max_iterations, max_evals, gtol, ftol))
+    _rbo_check(h, ccall((:rbo_fit_kernel, librbo), Cint,
+        (Ptr{Cvoid}, Ref{RboFitOpts}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Float64}, Ptr{Float64}, Ref{Int32}, Ref{Int32}, Ref{Int32}),
+        h.ptr, o, Vector{Float64}(lower), Vector{Float64}(upper), θ, ll, g, it, ev, st))
+    delete!(_RBO_RESIDENT, :surrogate)   # the device holds θ* now; s does until set_kernel! below has run
+    set_kernel!(s, s.ψ.constructor(θ))
+    _RBO_RESIDENT[:surrogate] = _rbo_surrogate_fp(s, get_observed(s))
+    return θ, ll[], st[]
 end
 
 function _rbo_rollout!(h, tp, θ, fmini, mode::Int, flags::Int, dual, resolutions, gx, gθ, best_index, status, summary)
